@@ -2,12 +2,15 @@
 """Benchmark of the PhylOligo hot path on B200: profile a synthetic multi-FASTA and
 compute its all-by-all JSD matrix (BASELINE.json: contig-pairs/sec, JSD k=4, strand both).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--scale S]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--scale S] [--dump-outputs DIR]
 
 One "step" = one full pass over the workload: composition profiling of every
 contig (k=4, both strands) + the JSD distance matrix.  Default workload is
 BASELINE.json configs[1] (C2: 100 000 contigs x 20 kb); ``--scale`` shrinks the
-contig count for quick checks (the JSON line then says so).
+contig count for quick checks (the JSON line then says so).  The input is drawn
+from a fixed seed, so two builds run with the same arguments see the same bytes;
+``--dump-outputs DIR`` writes what the last timed step computed (see dump_outputs)
+so that their results can be compared.
 
 `value`: unique contig pairs N(N+1)/2 resolved per second with the FASTA text
 already resident in HBM and the matrix left in HBM.  `e2e`: the same pass from
@@ -35,6 +38,8 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the benchmark leaves the source tree as it found it (it may be read-only): no bytecode caches
+sys.dont_write_bytecode = True
 
 METRIC = "contig-pairs/sec (JSD, k=4)"
 UNIT = "pairs/s"
@@ -42,6 +47,7 @@ PATTERN = "1111"
 STRAND = "both"
 DIM = 256
 JSD_FLOPS_PER_PAIR = 10 * DIM  # SURVEY.md 8(d) convention: 10 flop per dimension per pair
+DUMP_RECORDS = 2048  # --dump-outputs: 2048 x 2048 float32 distances + 2048 x 256 float32 profiles, 18 MB
 
 
 def parse_args():
@@ -58,7 +64,37 @@ def parse_args():
     ap.add_argument("--no-cli", action="store_true", help="skip the e2e_cli leg (dispatcher functions into a real memmap file)")
     ap.add_argument("--ring-sink", action="store_true",
                     help="end to end: copy whole row panels into a 2-slot pinned ring instead of a host matrix")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the profiles and distances of the last one as DIR/<name>.npy "
+                         "(one process only; a fixed sample of %d records when there are more)" % DUMP_RECORDS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    return args
+
+
+def dump_outputs(out_dir, freq, matrix):
+    """Write what a caller of the timed path receives, for comparing two builds output for output:
+    profiles.npy  float32 (m, 256)  k=4 frequency profiles of the sampled records
+    distances.npy float32 (m, m)    their JSD matrix (rows and columns of the sampled records)
+    records.npy   float64 (m,)      which records: all of them when there are at most DUMP_RECORDS, else a
+                                    seeded sample of DUMP_RECORDS - 2 plus the first and the last"""
+    import torch
+
+    n = int(matrix.shape[0])
+    if n <= DUMP_RECORDS:
+        idx = np.arange(n)
+    else:
+        idx = np.union1d(np.random.default_rng(0).choice(n, DUMP_RECORDS - 2, replace=False), [0, n - 1])
+    d_idx = torch.from_numpy(idx).to(matrix.device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"profiles": freq[d_idx].cpu().numpy(),
+              "distances": matrix[d_idx[:, None], d_idx[None, :]].cpu().numpy(),
+              "records": idx.astype(np.float64)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def workload_name(n, mean_len):
@@ -548,6 +584,8 @@ def run_ours(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (no CPU fallback)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single process: under torchrun every rank holds only its rows of the matrix")
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
     if world > 1:
@@ -837,6 +875,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = ms_total / args.steps
     value = pairs_unique / (ms_per_step * 1e-3)
+    if args.dump_outputs:  # the buffers still hold the last timed step's results
+        dump_outputs(args.dump_outputs, freq_pad[:n_contigs], matrix)
 
     # ---- end to end (host buffers in, host buffers out) ----
     for _ in range(max(1, min(2, args.warmup))):
@@ -1025,6 +1065,8 @@ def run_ours(args):
 def main():
     args = parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the results of this project's path (--impl ours)")
         run_reference(args)
     else:
         run_ours(args)

@@ -5,9 +5,8 @@ sklearn.externals.joblib are absent), but the hot-path function bodies are pure
 stdlib + numpy.  This module parses the reference source files where they lie
 under /root/reference, picks the named ``FunctionDef`` nodes and ``exec``s only
 those into a namespace that provides ``re, np, Counter, product, sys``.  Nothing
-is copied into the repository; the GPU box never has /root/reference, so this is
-used only by ``tests/golden/make_golden.py`` (to generate the committed golden
-vectors) and by CPU tests that skip when the reference is not mounted.
+is copied into the repository; this is used only by ``tests/golden/make_golden.py``
+to generate the committed golden vectors, which the tests compare against.
 """
 from __future__ import annotations
 

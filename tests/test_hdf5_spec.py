@@ -1,33 +1,23 @@
 """The HDF5 files of --large h5py, checked by an independent byte-level walker of the published
 format (tests/hdf5_spec_check.py) that is itself pinned to a file written by the real libhdf5."""
-import glob
 import os
 import sys
 
 import numpy as np
 import pytest
 
-sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, HERE)
 import hdf5_spec_check as spec  # noqa: E402
 
 from phyloligo_b200 import io_formats  # noqa: E402
 
 
-def _libhdf5_fixture():
-    try:
-        import scipy.io
-    except ImportError:
-        return None
-    hits = glob.glob(os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat"))
-    return hits[0] if hits else None
-
-
 def test_walker_reads_a_file_written_by_libhdf5():
     """MATLAB 7.3 files are HDF5 files behind a 512-byte user block; this one was written by libhdf5 in
-    2008 and holds the variable testdouble = 0 : pi/4 : 2 pi (scipy's own test vector for it)."""
-    path = _libhdf5_fixture()
-    if path is None:
-        pytest.skip("scipy's MATLAB 7.3 test fixture is not installed")
+    2008 and holds the variable testdouble = 0 : pi/4 : 2 pi.  It is scipy's own test vector for that
+    format (scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat, BSD licence), stored unchanged."""
+    path = os.path.join(HERE, "golden", "testhdf5_7.4_GLNX86.mat")
     f = spec.H5File(path)
     assert f.base == 512 and f.eof == os.path.getsize(path)
     root = f.root_group()

@@ -2,8 +2,7 @@
 
 The golden vectors were produced by tests/golden/make_golden.py, which executes
 the reference's function bodies (bin/phyloligo.py:601-661, core/phylodist.py:12-68)
-AST-extracted from /root/reference.  When the reference is mounted the same
-comparison is also made live.
+AST-extracted from the reference's sources.
 """
 import math
 
@@ -14,7 +13,6 @@ import scipy.stats as sst
 
 from conftest import golden_case_arrays
 from oracle import phylo_oracle as po
-from oracle import ref_extract
 from phyloligo_b200 import synth
 
 
@@ -69,28 +67,6 @@ def test_distance_oracle_matches_reference_golden(distance_golden):
         # vectorised oracle agrees with the pair functions
         assert np.allclose(po.pairwise_np(X, "JSD"), distance_golden[name + "_JSD"], rtol=1e-12, atol=1e-15)
         assert np.allclose(po.pairwise_np(X, "Eucl"), distance_golden[name + "_Eucl"], rtol=1e-12, atol=1e-15)
-
-
-@pytest.mark.skipif(not ref_extract.available(), reason="reference checkout not mounted")
-def test_oracle_against_live_reference_bodies():
-    ref = ref_extract.load()
-    rng = np.random.default_rng(5)
-    seqs = synth.make_sequences(6, 800, seed=3)
-    for s in seqs:
-        s = s.decode()
-        for pat in ("1111", "111010011", "1101"):
-            for strand in ("plus", "minus", "both"):
-                prepared = po.select_strand(s, strand).upper()
-                words, total = ref["cut_sequence_and_count_pattern"](prepared, pat)
-                freq = ref["count2freq"](words, total, pat.count("1"))
-                assert np.array_equal(np.asarray(freq, dtype=np.float64), po.frequency_np(s, pat, strand))
-    X = rng.random((6, 64))
-    X[X < 0.3] = 0
-    X /= X.sum(axis=1, keepdims=True)
-    for a in range(6):
-        for b in range(6):
-            assert ref["JSD"](X[a].copy(), X[b].copy()) == po.JSD(X[a], X[b])
-            assert ref["Eucl"](X[a].copy(), X[b].copy()) == po.Eucl(X[a], X[b])
 
 
 def test_reverse_complement_iupac():

@@ -32,23 +32,6 @@ def test_oracle_reproduces_the_reference_class(golden):
         assert sum("is empty" in str(w.message) for w in caught) == int(golden[name + "_empty_warnings"]), name
 
 
-def test_golden_matches_the_reference_when_mounted(golden):
-    """Regenerate the goldens from /root/reference (absent on the GPU box: skipped there)."""
-    src = os.path.join(os.environ.get("PHYLOLIGO_REFERENCE", "/root/reference"), "phylopackage", "bin", "phyloselect.py")
-    if not os.path.isfile(src):
-        pytest.skip("reference checkout not mounted")
-    import sys
-    sys.path.insert(0, GOLDEN)
-    import make_select_golden as mk
-    KMedoids = mk.load_kmedoids()
-    for name, D, kw in mk.matrices():
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            km = KMedoids(distance_metric="precomputed", **kw).fit(D)
-        assert np.array_equal(np.asarray(km.labels_), golden[name + "_labels"]), name
-        assert km.n_iter_ == int(golden[name + "_n_iter"])
-
-
 def test_knn_oracle_is_sklearns_graph():
     rng = np.random.default_rng(3)
     P = rng.random((40, 5))
