@@ -344,6 +344,43 @@ int po_cluster_argmin(const double* d_cost, const int* d_labels, int64_t n, int 
 int po_matrix_knn(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int64_t self0, int k, int* d_idx,
                   float* d_dist, po_stream_t stream);
 
+/*
+ * HDBSCAN on the resident matrix: what find_clusters (:403-428) gets from
+ * hdbscan.HDBSCAN(min_cluster_size, min_samples, metric="precomputed"), every other argument at its default.
+ * MST edges compare by the triple (mutual reachability, min(i, j), max(i, j)); the MST is then unique.
+ *   po_hdbscan_check         refuses (PO_ERR_ARG) a matrix that is not square, not bitwise symmetric or holds a
+ *                            NaN or an infinite entry; the message names the first offending entry in row-major
+ *                            order.  d_work: 8 bytes.  Synchronises `stream`.
+ *   po_matrix_kth            d_out[i] = the k-th smallest (1-based) entry of row i, every column counted (the
+ *                            diagonal too), bit for bit in the matrix's dtype: the core distances, k =
+ *                            min_samples + 1 (contrib's np.partition(D, min_samples, axis=0)[min_samples] in
+ *                            mutual_reachability)
+ *   po_hdbscan_mst_workspace bytes of d_work the two entries below need for n points
+ *   po_hdbscan_mst_init      n singleton components in d_work
+ *   po_hdbscan_mst_round     one Boruvka round over mr(i, j) = max(core_i, core_j, D[i, j]), computed on the fly
+ *                            and never stored (replaces contrib's mutual_reachability and mst_linkage_core): one
+ *                            pass over the matrix finds every row's lightest edge to another component, then a
+ *                            per-component reduction, hooking and pointer jumping.  Appends the new edges to
+ *                            d_u, d_v (int64) and d_w (the matrix's dtype), n - 1 entries each over all rounds,
+ *                            in no particular order; *h_components = components left (1 when done).  Reads two
+ *                            counters to the host (synchronises `stream`).
+ *   po_hdbscan_tree          host: sorts the n - 1 MST edges in place by the tie rule (u < v), then contrib's
+ *                            label (single-linkage rows sl_*: left, right, distance, size), condense_tree
+ *                            (ct_*: parent, child, lambda_val, child_size; up to 2 n rows, *ct_rows written),
+ *                            compute_stability, get_clusters (excess of mass, allow_single_cluster=False) and
+ *                            get_probabilities: labels (-1 = noise; clusters numbered in ascending condensed-tree
+ *                            id) and probabilities.  O(N log N).
+ */
+int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, void* d_work, po_stream_t stream);
+int po_matrix_kth(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int k, void* d_out, po_stream_t stream);
+int64_t po_hdbscan_mst_workspace(int64_t n);
+int po_hdbscan_mst_init(int64_t n, void* d_work, po_stream_t stream);
+int po_hdbscan_mst_round(const void* d_D, int64_t ld, int dtype, int64_t n, const void* d_core, void* d_work, int64_t* d_u,
+                         int64_t* d_v, void* d_w, int64_t* h_components, po_stream_t stream);
+int po_hdbscan_tree(int64_t n, int64_t min_cluster_size, int64_t* u, int64_t* v, double* w, int64_t* sl_left, int64_t* sl_right,
+                    double* sl_dist, int64_t* sl_size, int64_t* ct_parent, int64_t* ct_child, double* ct_lambda, int64_t* ct_size,
+                    int64_t* ct_rows, int64_t* labels, double* probabilities);
+
 /* Number of kernels this library has launched since load (for bench.py's gpu_launches). */
 int64_t po_launch_count(void);
 

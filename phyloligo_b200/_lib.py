@@ -30,7 +30,9 @@ EXPORTED = [
     "po_host_prefault", "po_host_premap", "po_host_register", "po_host_unregister", "po_host_copy2d", "po_host_pwrite2d",
     "po_host_pread", "po_host_transpose_f32",
     "po_host_mirror_open", "po_host_mirror_submit", "po_host_mirror_wait", "po_host_mirror_close",
-    "po_matrix_rowsums", "po_matrix_argmin_rows", "po_cluster_argmin", "po_matrix_knn", "po_launch_count", "po_timing_enable", "po_timing_reset", "po_timing_read", "po_microbench",
+    "po_matrix_rowsums", "po_matrix_argmin_rows", "po_cluster_argmin", "po_matrix_knn",
+    "po_hdbscan_check", "po_matrix_kth", "po_hdbscan_mst_workspace", "po_hdbscan_mst_init", "po_hdbscan_mst_round", "po_hdbscan_tree",
+    "po_launch_count", "po_timing_enable", "po_timing_reset", "po_timing_read", "po_microbench",
 ]
 
 
@@ -124,6 +126,18 @@ def load():
     lib.po_cluster_argmin.restype = i32
     lib.po_matrix_knn.argtypes = [vp, i64, i32, i64, i64, i64, i32, vp, vp, vp]
     lib.po_matrix_knn.restype = i32
+    lib.po_hdbscan_check.argtypes = [vp, i64, i32, i64, i64, vp, vp]
+    lib.po_hdbscan_check.restype = i32
+    lib.po_matrix_kth.argtypes = [vp, i64, i32, i64, i64, i32, vp, vp]
+    lib.po_matrix_kth.restype = i32
+    lib.po_hdbscan_mst_workspace.argtypes = [i64]
+    lib.po_hdbscan_mst_workspace.restype = i64
+    lib.po_hdbscan_mst_init.argtypes = [i64, vp, vp]
+    lib.po_hdbscan_mst_init.restype = i32
+    lib.po_hdbscan_mst_round.argtypes = [vp, i64, i32, i64, vp, vp, vp, vp, vp, C.POINTER(i64), vp]
+    lib.po_hdbscan_mst_round.restype = i32
+    lib.po_hdbscan_tree.argtypes = [i64, i64] + [vp] * 14
+    lib.po_hdbscan_tree.restype = i32
     lib.po_launch_count.restype = i64
     lib.po_timing_enable.argtypes = [i32]
     lib.po_timing_enable.restype = i32

@@ -12,8 +12,10 @@
 //                                                                                              + po_cluster_argmin
 //   TSNE(metric="precomputed") / HDBSCAN(metric="precomputed") :381-428: the k nearest
 //   neighbours of every row (sklearn kneighbors_graph on a precomputed matrix)                -> po_matrix_knn
+//   HDBSCAN's core distances (hdbscan's mutual_reachability: np.partition(D, min_samples,
+//   axis=0)[min_samples], an exact entry of the matrix)                                       -> po_matrix_kth
 //
-// All four are single passes over rows of the matrix: HBM bound, 4 bytes per entry read once.
+// The first four are single passes over rows of the matrix: HBM bound, 4 bytes per entry read once.
 #include <float.h>
 #include "po_common.cuh"
 
@@ -145,6 +147,58 @@ constexpr int KNN_SAMPLE = 8192;  // entries of the row sampled for the fast pat
 __device__ __forceinline__ unsigned fkey(float v) {
     const unsigned b = __float_as_uint(v);
     return (b >> 31) ? ~b : (b | 0x80000000u);
+}
+
+// Radix select over order-preserving keys K (32 bits for float entries, 64 for double), 8 bits per pass from
+// the top, each pass a shared-memory histogram of the still undecided prefix class: the key of the
+// need-th smallest (1-based) key_of(j) over the columns j < ncols, j != self, and in *nties how many
+// entries equal to it belong to the `need` smallest.  Called by every thread of the CTA.
+template <typename K, typename KeyOf>
+__device__ __forceinline__ K radix_select(KeyOf key_of, int64_t ncols, int64_t self, unsigned need, unsigned* hist, unsigned* nties) {
+    __shared__ K r_prefix, r_mask;
+    __shared__ unsigned r_need;
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        r_prefix = 0;
+        r_mask = 0;
+        r_need = need;  // rank (1-based) of the wanted entry inside the current prefix class
+    }
+    __syncthreads();
+    for (int pass = 0; pass < (int)sizeof(K); ++pass) {
+        const int shift = 8 * ((int)sizeof(K) - 1 - pass);
+        hist[tid] = 0u;
+        __syncthreads();
+        const K prefix = r_prefix, mask = r_mask;
+        for (int64_t j0 = 0; j0 < ncols; j0 += KNN_THREADS) {
+            const int64_t j = j0 + tid;
+            unsigned bin = 0xFFFFFFFFu;
+            if (j < ncols && j != self) {
+                const K key = key_of(j);
+                if ((key & mask) == prefix) bin = (unsigned)(key >> shift) & 255u;
+            }
+            // distances share their leading bits: aggregate equal bins inside the warp, one atomic per distinct bin
+            const unsigned active = __ballot_sync(0xFFFFFFFFu, bin != 0xFFFFFFFFu);
+            if (bin != 0xFFFFFFFFu) {
+                const unsigned peers = __match_any_sync(active, bin);
+                if ((tid & 31) == __ffs(peers) - 1) atomicAdd(&hist[bin], (unsigned)__popc(peers));
+            }
+        }
+        __syncthreads();
+        if (tid == 0) {
+            unsigned need_ = r_need, acc = 0u;
+            int b = 0;
+            for (; b < 255; ++b) {
+                if (acc + hist[b] >= need_) break;
+                acc += hist[b];
+            }
+            r_need = need_ - acc;
+            r_prefix = prefix | ((K)b << shift);
+            r_mask = mask | ((K)255u << shift);
+        }
+        __syncthreads();
+    }
+    *nties = r_need;
+    return r_prefix;
 }
 
 template <typename T>
@@ -304,47 +358,8 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
         __syncthreads();
     }
     // ---------------- exact path ----------------
-    if (tid == 0) {
-        s_prefix = 0u;
-        s_mask = 0u;
-        s_need = (unsigned)k;  // rank (1-based) of the wanted entry inside the current prefix class
-    }
-    __syncthreads();
-    for (int pass = 0; pass < 4; ++pass) {
-        const int shift = 24 - 8 * pass;
-        hist[tid] = 0u;
-        __syncthreads();
-        const unsigned prefix = s_prefix, mask = s_mask;
-        for (int64_t j0 = 0; j0 < ncols; j0 += KNN_THREADS) {
-            const int64_t j = j0 + tid;
-            unsigned bin = 0xFFFFFFFFu;
-            if (j < ncols && j != self) {
-                const unsigned key = key_of(j);
-                if ((key & mask) == prefix) bin = (key >> shift) & 255u;
-            }
-            // distances share their leading bits: aggregate equal bins inside the warp, one atomic per distinct bin
-            const unsigned active = __ballot_sync(0xFFFFFFFFu, bin != 0xFFFFFFFFu);
-            if (bin != 0xFFFFFFFFu) {
-                const unsigned peers = __match_any_sync(active, bin);
-                if ((tid & 31) == __ffs(peers) - 1) atomicAdd(&hist[bin], (unsigned)__popc(peers));
-            }
-        }
-        __syncthreads();
-        if (tid == 0) {
-            unsigned need = s_need, acc = 0u;
-            int b = 0;
-            for (; b < 255; ++b) {
-                if (acc + hist[b] >= need) break;
-                acc += hist[b];
-            }
-            s_need = need - acc;
-            s_prefix = prefix | ((unsigned)b << shift);
-            s_mask = mask | (255u << shift);
-        }
-        __syncthreads();
-    }
-    const unsigned kth = s_prefix;   // key of the k-th smallest entry
-    const unsigned nties = s_need;   // how many entries equal to it belong to the k smallest
+    unsigned nties;  // how many entries equal to the k-th smallest belong to the k smallest
+    const unsigned kth = radix_select<unsigned>(key_of, ncols, self, (unsigned)k, hist, &nties);  // key of the k-th smallest
     if (tid == 0) {
         s_below = 0u;
         s_ties = 0u;
@@ -403,6 +418,27 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
         out_idx[i * k + q] = (it == ~0ull) ? -1 : col;
         out_dist[i * k + q] = (it == ~0ull) ? __int_as_float(0x7FC00000) : (float)row[col];
     }
+}
+
+
+// The k-th smallest entry (1-based, every column counted, the diagonal too) of every row, returned bit for
+// bit in the matrix's dtype: the exact radix select of knn_kernel over the full-width key of the entry
+// (4 passes for float, 8 for double), so that no two float64 entries that round to one float32 are
+// confused.  NaN entries sort last.  One CTA per row.
+__device__ __forceinline__ unsigned okey(float v) { return (v != v) ? 0xFFFFFFFFu : fkey(v); }
+__device__ __forceinline__ unsigned long long okey(double v) { return (v != v) ? ~0ull : dkey(v); }
+__device__ __forceinline__ float from_okey(unsigned k) { return __uint_as_float((k >> 31) ? (k & 0x7FFFFFFFu) : ~k); }
+__device__ __forceinline__ double from_okey(unsigned long long k) {
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7FFFFFFFFFFFFFFFull) : ~k));
+}
+
+template <typename T>
+__global__ void __launch_bounds__(KNN_THREADS) kth_kernel(const void* __restrict__ D, int64_t ld, int64_t ncols, int k, T* __restrict__ out) {
+    __shared__ unsigned hist[256];
+    const T* row = reinterpret_cast<const T*>(D) + (int64_t)blockIdx.x * ld;
+    unsigned nties;
+    const auto key = radix_select<decltype(okey(T()))>([&](int64_t j) { return okey(row[j]); }, ncols, (int64_t)-1, (unsigned)k, hist, &nties);
+    if (threadIdx.x == 0) out[blockIdx.x] = from_okey(key);
 }
 
 }  // namespace po
@@ -487,6 +523,26 @@ int po_matrix_knn(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_
         knn_kernel<double><<<(unsigned)n_rows, KNN_THREADS, smem, (cudaStream_t)stream>>>(d_D, ld, n_cols, self0, k, kpad, d_idx, d_dist);
     count_launch(2);
     PO_LAUNCH_CHECK("knn_kernel");
+    return PO_OK;
+}
+
+int po_matrix_kth(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int k, void* d_out, po_stream_t stream) {
+    if (!d_D || !d_out || n_rows < 0 || n_cols < 1 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64) || k < 1 ||
+        n_rows > 0x7FFFFFFFll) {
+        set_error("po_matrix_kth: bad arguments");
+        return PO_ERR_ARG;
+    }
+    if (k > n_cols) {
+        set_error("po_matrix_kth: k = %d outside [1, columns = %lld]", k, (long long)n_cols);
+        return PO_ERR_UNSUPPORTED;
+    }
+    if (n_rows == 0) return PO_OK;
+    if (dtype == PO_F32)
+        kth_kernel<float><<<(unsigned)n_rows, KNN_THREADS, 0, (cudaStream_t)stream>>>(d_D, ld, n_cols, k, (float*)d_out);
+    else
+        kth_kernel<double><<<(unsigned)n_rows, KNN_THREADS, 0, (cudaStream_t)stream>>>(d_D, ld, n_cols, k, (double*)d_out);
+    count_launch(2);
+    PO_LAUNCH_CHECK("kth_kernel");
     return PO_OK;
 }
 

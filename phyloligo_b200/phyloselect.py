@@ -1,17 +1,19 @@
 #!/usr/bin/env python3
-"""The front half of phyloselect.py on B200 (SURVEY.md 8f rank 4): K-medoids on the contig distance
-matrix and the nearest-neighbour graph its t-SNE / HDBSCAN consumers start from, computed on the
-device while the matrix is resident -- straight after the distance stage if wanted, without the
-round trip through a 40 GB file and 800 GB of host RAM the reference's documentation asks for.
+"""The front half of phyloselect.py on B200 (SURVEY.md 8f rank 4): K-medoids and HDBSCAN on the contig
+distance matrix, and the nearest-neighbour graph its t-SNE consumer starts from, computed on the device
+while the matrix is resident -- straight after the distance stage if wanted, without the round trip
+through a 40 GB file and 800 GB of host RAM the reference's documentation asks for.
 
 Mirrors reference phylopackage/bin/phyloselect.py: ``KMedoids`` (:37-309; same constructor
 arguments and fitted attributes), ``clusterize`` (:573-590), ``find_clusters`` (:403-428), the
 matrix readers of ``main`` (:597-622), ``write_fastafile`` (:547-571) and the
-``data_cluster_indexes.dat`` writer (:742-751).  Plotting, t-SNE itself, the interactive loop and
-HDBSCAN (third-party, not installed) are out of scope: ``knn_graph`` hands those consumers the
+``data_cluster_indexes.dat`` writer (:742-751).  ``HDBSCAN`` computes what the reference gets from
+the third-party hdbscan.HDBSCAN(metric="precomputed") with its default arguments (core distances,
+mutual-reachability MST, condensed tree, excess-of-mass selection), with MST ties broken by vertex
+index.  Plotting, t-SNE itself and the interactive loop are out of scope: ``knn_graph`` hands t-SNE the
 sparse precomputed neighbour graph scikit-learn's TSNE accepts in place of the dense matrix.
 
-There is no CPU fallback: the sums, assignments and selections run in libphyloligo_b200.so.
+There is no CPU fallback: the sums, assignments, selections and the MST run in libphyloligo_b200.so.
 """
 from __future__ import annotations
 
@@ -190,6 +192,136 @@ class KMedoids:
         return self
 
 
+def check_matrix(D):
+    """Refuse (PhyloligoError) a device matrix that is not square, not bitwise symmetric or holds a NaN or an
+    infinite entry; the message names the first offending entry (po_hdbscan_check)."""
+    lib = _lib.load()
+    work = torch.empty(1, dtype=torch.int64, device=D.device)
+    rc = lib.po_hdbscan_check(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), _ptr(work), _stream())
+    _lib.check(rc, "po_hdbscan_check")
+
+
+def kth_smallest(D, k):
+    """The k-th smallest entry (1-based, the diagonal counted) of every row of the device matrix D, bit for bit
+    in D's dtype (po_matrix_kth)."""
+    lib = _lib.load()
+    out = torch.empty(int(D.shape[0]), dtype=D.dtype, device=D.device)
+    rc = lib.po_matrix_kth(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), int(k), _ptr(out), _stream())
+    _lib.check(rc, "po_matrix_kth")
+    return out
+
+
+def mutual_reachability_mst(D, core, on_round=None):
+    """The minimum spanning tree of mr(i, j) = max(core[i], core[j], D[i, j]) by Boruvka rounds on the device
+    (po_hdbscan_mst_round), edges compared by (mr, min(i, j), max(i, j)).  Returns device tensors
+    (u int64, v int64, w in D's dtype), n - 1 edges in no particular order.  `on_round(components)` is
+    called after every round."""
+    lib = _lib.load()
+    n = int(D.shape[0])
+    dev = D.device
+    work = torch.empty(int(lib.po_hdbscan_mst_workspace(n)), dtype=torch.uint8, device=dev)
+    u = torch.empty(max(n - 1, 1), dtype=torch.int64, device=dev)
+    v = torch.empty_like(u)
+    w = torch.empty(max(n - 1, 1), dtype=D.dtype, device=dev)
+    _lib.check(lib.po_hdbscan_mst_init(n, _ptr(work), _stream()), "po_hdbscan_mst_init")
+    comps = C.c_int64(n)
+    while comps.value > 1:
+        rc = lib.po_hdbscan_mst_round(_ptr(D), int(D.stride(0)), _dt(D), n, _ptr(core), _ptr(work), _ptr(u), _ptr(v), _ptr(w),
+                                      C.byref(comps), _stream())
+        _lib.check(rc, "po_hdbscan_mst_round")
+        if on_round is not None:
+            on_round(comps.value)
+    return u[:n - 1], v[:n - 1], w[:n - 1]
+
+
+CONDENSED_DTYPE = np.dtype([("parent", np.int64), ("child", np.int64), ("lambda_val", np.float64), ("child_size", np.int64)])
+
+
+def hdbscan_tree(u, v, w, n, min_cluster_size):
+    """Host stage (po_hdbscan_tree) from the n - 1 MST edges, in any order and orientation.  Returns (labels
+    int64, probabilities float64, condensed tree, single-linkage tree n - 1 x 4, MST n - 1 x 3 of (i, j, w)
+    with i < j in tie-rule order).  The inputs are not modified."""
+    lib = _lib.load()
+    u = np.array(u, dtype=np.int64)  # copies: the library sorts them in place
+    v = np.array(v, dtype=np.int64)
+    w = np.array(w, dtype=np.float64)
+    m = n - 1
+    if not (u.shape == v.shape == w.shape == (m,)):
+        raise PhyloligoError("hdbscan_tree: %d points need %d edges" % (n, m))
+    sl = [np.empty(m, np.int64), np.empty(m, np.int64), np.empty(m, np.float64), np.empty(m, np.int64)]
+    cols = [np.empty(2 * n, np.int64), np.empty(2 * n, np.int64), np.empty(2 * n, np.float64), np.empty(2 * n, np.int64)]
+    rows = np.zeros(1, np.int64)
+    labels = np.empty(n, np.int64)
+    probs = np.empty(n, np.float64)
+    args = [u, v, w] + sl + cols + [rows, labels, probs]
+    rc = lib.po_hdbscan_tree(n, int(min_cluster_size), *[C.c_void_p(a.ctypes.data) for a in args])
+    _lib.check(rc, "po_hdbscan_tree")
+    r = int(rows[0])
+    ct = np.empty(r, dtype=CONDENSED_DTYPE)
+    for name, col in zip(CONDENSED_DTYPE.names, cols):
+        ct[name] = col[:r]
+    slt = np.column_stack([sl[0].astype(np.float64), sl[1].astype(np.float64), sl[2], sl[3].astype(np.float64)])
+    return labels, probs, ct, slt, np.column_stack([u.astype(np.float64), v.astype(np.float64), w])
+
+
+class HDBSCAN:
+    """HDBSCAN on the device.  Same parameters, defaults and fitted attributes as the hdbscan.HDBSCAN the
+    reference calls (bin/phyloselect.py:403-428): ``labels_`` (-1 = noise), ``probabilities_``,
+    ``minimum_spanning_tree_`` (n - 1 x 3 ndarray of (i, j, distance), i < j, sorted by the tie rule),
+    ``condensed_tree_`` (structured ndarray: parent, child, lambda_val, child_size) and
+    ``single_linkage_tree_`` (n - 1 x 4, scipy's linkage layout).  ``metric`` is "precomputed" (X is the
+    N x N matrix: ndarray, memmap or a device tensor, which is used in place) or one of the package's metrics
+    (X is the N x D profile matrix and the distances never leave the device).  Arguments of hdbscan.HDBSCAN
+    other than min_cluster_size, min_samples and metric are accepted at their default values only.  MST
+    edges of equal weight are ordered by (min(i, j), max(i, j)), which makes the result deterministic."""
+
+    # hdbscan.HDBSCAN's other arguments and the only value accepted for each
+    DEFAULTS = {"cluster_selection_epsilon": 0.0, "max_cluster_size": 0, "alpha": 1.0, "p": None, "algorithm": "best",
+                "leaf_size": 40, "memory": None, "approx_min_span_tree": True, "gen_min_span_tree": False,
+                "core_dist_n_jobs": 4, "cluster_selection_method": "eom", "allow_single_cluster": False,
+                "prediction_data": False, "match_reference_implementation": False}
+
+    def __init__(self, min_cluster_size=5, min_samples=None, metric="precomputed", **kwargs):
+        for key, value in kwargs.items():
+            if key not in self.DEFAULTS:
+                raise ValueError("HDBSCAN has no argument {!r}".format(key))
+            if value != self.DEFAULTS[key]:
+                raise ValueError("{}={!r} is not supported; only the default {!r}".format(key, value, self.DEFAULTS[key]))
+        if not isinstance(min_cluster_size, (int, np.integer)) or isinstance(min_cluster_size, bool) or (
+                min_samples is not None and (not isinstance(min_samples, (int, np.integer)) or isinstance(min_samples, bool))):
+            raise ValueError("Min samples and min cluster size must be integers!")
+        if min_cluster_size <= 0 or (min_samples is not None and min_samples <= 0):
+            raise ValueError("Min samples and Min cluster size must be positive integers (min_cluster_size={}, min_samples={})"
+                             .format(min_cluster_size, min_samples))
+        if min_cluster_size == 1:
+            raise ValueError("Min cluster size must be greater than one (min_cluster_size=1)")
+        if metric != "precomputed" and metric not in _lib.METRICS:
+            raise ValueError("metric needs to be 'precomputed' or one of {}. Instead, '{}' was given.".format(sorted(_lib.METRICS), metric))
+        self.min_cluster_size = int(min_cluster_size)
+        self.min_samples = None if min_samples is None else int(min_samples)
+        self.metric = metric
+
+    def fit(self, X, y=None):
+        if self.metric == "precomputed":
+            D = as_device_matrix(X)
+        else:
+            Xd = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(X)))
+            D = engine.distance_matrix_device(Xd.to(engine.require_cuda()), self.metric, torch.float32, symmetric=True)
+        n = int(D.shape[0])
+        if n < 2:
+            raise ValueError("HDBSCAN needs at least 2 samples, got {}".format(n))
+        check_matrix(D)
+        ms = min(self.min_cluster_size if self.min_samples is None else self.min_samples, n - 1)
+        core = kth_smallest(D, ms + 1)
+        u, v, w = mutual_reachability_mst(D, core)
+        (self.labels_, self.probabilities_, self.condensed_tree_, self.single_linkage_tree_,
+         self.minimum_spanning_tree_) = hdbscan_tree(u.cpu().numpy(), v.cpu().numpy(), w.cpu().numpy(), n, self.min_cluster_size)
+        return self
+
+    def fit_predict(self, X, y=None):
+        return self.fit(X).labels_
+
+
 # ---------------------------------------------------------------------------
 # the script's functions
 # ---------------------------------------------------------------------------
@@ -217,16 +349,7 @@ def find_clusters(data, method, kwargs):
     if method == "kmedoids":
         return KMedoids(**kwargs).fit(data).labels_
     if method == "hdbscan":
-        try:
-            import hdbscan
-        except ImportError:
-            print("Error, method hdbscan needs the hdbscan package, which is not installed; "
-                  "knn_graph() provides its neighbour graph", file=sys.stderr)
-            sys.exit(1)
-        host = data.cpu().numpy() if isinstance(data, torch.Tensor) else np.asarray(data)
-        clusterer = hdbscan.HDBSCAN(**kwargs)
-        clusterer.fit(host.astype(np.float64))
-        return clusterer.labels_
+        return HDBSCAN(**kwargs).fit(data).labels_
     print("Error, unknown method {}".format(method), file=sys.stderr)
     sys.exit(1)
 
@@ -283,7 +406,8 @@ def get_cmd(argv=None):
     parser = argparse.ArgumentParser(description="Cluster contigs from their oligonucleotide-profile distances on B200 GPUs")
     parser.add_argument("-i", action="store", dest="distmat", help="The input matrix file")
     parser.add_argument("-m", action="store", dest="method", required=True, choices=["hdbscan", "kmedoids"],
-                        help="Method to use to compute cluster on the distance matrix")
+                        help="Method to use to compute cluster on the distance matrix: HDBSCAN (--minclustersize, "
+                             "--minsamples; noise goes to data_fasta_unclust.fa) or K-medoids (-k)")
     parser.add_argument("--minclustersize", action="store", dest="min_cluster_size", type=int,
                         help="Set the minimal cluster size of an HDBSCAN cluster")
     parser.add_argument("--minsamples", action="store", dest="min_samples", type=int,
