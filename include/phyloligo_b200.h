@@ -381,6 +381,42 @@ int po_hdbscan_tree(int64_t n, int64_t min_cluster_size, int64_t* u, int64_t* v,
                     double* sl_dist, int64_t* sl_size, int64_t* ct_parent, int64_t* ct_child, double* ct_lambda, int64_t* ct_size,
                     int64_t* ct_rows, int64_t* labels, double* probabilities);
 
+/*
+ * t-SNE on the resident matrix: what sklearn.manifold.TSNE(metric="precomputed", method="barnes_hut", angle=0.0)
+ * computes for the reference's -t projection (:381-398).  With angle 0 scikit-learn's Barnes-Hut gradient is the
+ * exact gradient of the sparse-P objective; these entries evaluate it exactly.  Sums run in a fixed order.
+ *   po_tsne_check            refuses (PO_ERR_ARG) a matrix holding a NaN, an infinite or a negative entry
+ *                            (check_array / check_non_negative); the message names the first in row-major order.
+ *                            d_work: 8 bytes.  Synchronises `stream`.
+ *   po_tsne_conditional      _binary_search_perplexity over the k neighbours d_idx [n x k] (po_matrix_knn) of
+ *                            every row: squared distances D[i, idx]^2 in the matrix's dtype, then float32; the
+ *                            search in float64 (tolerance 1e-5 on the entropy, at most 100 steps).  d_P float64
+ *                            [n x k], each row summing to 1 (0 where every exp underflows)
+ *   po_tsne_sum              *d_out = sum of d_x[0 .. n) in float64 in a fixed order (one CTA)
+ *   po_tsne_workspace        bytes of d_work the two entries below need for n points
+ *   po_tsne_repulsion        the exact all-pairs pass over the positions d_Y (float32 [n x 2]): per row
+ *                            sum_j q_ij^2 (y_i - y_j) and Z = sum_{i != j} q_ij, q_ij = 1 / (1 + |y_i - y_j|^2),
+ *                            kept in d_work for the step
+ *   po_tsne_attraction_step  per row the CSR walk sum_j p_ij q_ij (y_i - y_j), p_ij = float32((P_ij * mul) / div),
+ *                            and the gradient 4 (attraction - repulsion / Z) of the positions the last
+ *                            po_tsne_repulsion saw.  d_grad (optional, float32 [n x 2]) receives it.  With d_Y_next
+ *                            one _gradient_descent step: gains (+0.2 / x0.8, at least 0.01, float32), update =
+ *                            momentum update - learning_rate grad gains (float64 when update64, else float32 as
+ *                            scikit-learn's arithmetic with a float32 learning rate), d_Y_next = d_Y + update.
+ *                            With h_kl_gradnorm2 the KL divergence sum p_ij log(max(p_ij, tiny) / max(q_ij / Z,
+ *                            tiny)) and |grad gains|^2 are reduced and copied to h_kl_gradnorm2[0..1]
+ *                            (synchronises `stream`).
+ */
+int po_tsne_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, void* d_work, po_stream_t stream);
+int po_tsne_conditional(const void* d_D, int64_t ld, int dtype, int64_t n, const int* d_idx, int k, double perplexity, double* d_P,
+                        po_stream_t stream);
+int po_tsne_sum(const double* d_x, int64_t n, double* d_out, po_stream_t stream);
+int64_t po_tsne_workspace(int64_t n);
+int po_tsne_repulsion(const float* d_Y, int64_t n, void* d_work, po_stream_t stream);
+int po_tsne_attraction_step(const int64_t* d_indptr, const int* d_indices, const double* d_P, int64_t n, double mul, double div,
+                            const float* d_Y, void* d_work, float* d_Y_next, double* d_update, float* d_gains, float* d_grad,
+                            double momentum, double learning_rate, int update64, double* h_kl_gradnorm2, po_stream_t stream);
+
 /* Number of kernels this library has launched since load (for bench.py's gpu_launches). */
 int64_t po_launch_count(void);
 
@@ -392,7 +428,7 @@ int po_timing_reset(void);
 int po_timing_read(int family, double* total_ms, int64_t* launches);
 
 /* Pipe-peak microbenchmark for roofline denominators that MEASURED_PEAKS.json lacks.
- * kind 0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s (best of 4 timed runs). */
+ * kind 0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s (best of 4 timed runs). */
 int po_microbench(int kind, double* result);
 
 #ifdef __cplusplus

@@ -32,6 +32,7 @@ EXPORTED = [
     "po_host_mirror_open", "po_host_mirror_submit", "po_host_mirror_wait", "po_host_mirror_close",
     "po_matrix_rowsums", "po_matrix_argmin_rows", "po_cluster_argmin", "po_matrix_knn",
     "po_hdbscan_check", "po_matrix_kth", "po_hdbscan_mst_workspace", "po_hdbscan_mst_init", "po_hdbscan_mst_round", "po_hdbscan_tree",
+    "po_tsne_check", "po_tsne_conditional", "po_tsne_sum", "po_tsne_workspace", "po_tsne_repulsion", "po_tsne_attraction_step",
     "po_launch_count", "po_timing_enable", "po_timing_reset", "po_timing_read", "po_microbench",
 ]
 
@@ -138,6 +139,19 @@ def load():
     lib.po_hdbscan_mst_round.restype = i32
     lib.po_hdbscan_tree.argtypes = [i64, i64] + [vp] * 14
     lib.po_hdbscan_tree.restype = i32
+    lib.po_tsne_check.argtypes = [vp, i64, i32, i64, i64, vp, vp]
+    lib.po_tsne_check.restype = i32
+    lib.po_tsne_conditional.argtypes = [vp, i64, i32, i64, vp, i32, C.c_double, vp, vp]
+    lib.po_tsne_conditional.restype = i32
+    lib.po_tsne_sum.argtypes = [vp, i64, vp, vp]
+    lib.po_tsne_sum.restype = i32
+    lib.po_tsne_workspace.argtypes = [i64]
+    lib.po_tsne_workspace.restype = i64
+    lib.po_tsne_repulsion.argtypes = [vp, i64, vp, vp]
+    lib.po_tsne_repulsion.restype = i32
+    lib.po_tsne_attraction_step.argtypes = [vp, vp, vp, i64, C.c_double, C.c_double, vp, vp, vp, vp, vp, vp, C.c_double,
+                                            C.c_double, i32, C.POINTER(C.c_double), vp]
+    lib.po_tsne_attraction_step.restype = i32
     lib.po_launch_count.restype = i64
     lib.po_timing_enable.argtypes = [i32]
     lib.po_timing_enable.restype = i32
@@ -184,7 +198,7 @@ def timing_read(family: int):
 
 
 def microbench(kind: int) -> float:
-    """0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s."""
+    """0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s."""
     out = C.c_double()
     check(load().po_microbench(kind, C.byref(out)), "po_microbench")
     return out.value

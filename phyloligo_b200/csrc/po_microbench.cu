@@ -3,6 +3,7 @@
 //   kind 0: dependent-chain-free FFMA throughput, TFLOP/s (2 flop per FFMA)
 //   kind 1: MUFU.LG2 throughput, 1e12 op/s
 //   kind 2: POPC throughput, 1e12 op/s
+//   kind 3: MUFU.RCP throughput (rcp.approx.ftz.f32, the t-SNE repulsion's reciprocal), 1e12 op/s
 #include "po_common.cuh"
 
 namespace po {
@@ -25,6 +26,10 @@ __global__ void __launch_bounds__(256) pipe_peak_kernel(float* sink, int iters) 
                 if (KIND == 0) a[i] = fmaf(a[i], m, c);
                 if (KIND == 1) asm volatile("lg2.approx.f32 %0, %0;" : "+f"(a[i]));
                 if (KIND == 2) u[i] = __popc(u[i]) + u[i];
+                if (KIND == 3) {  // the add keeps ptxas from folding rcp(rcp(x)) = x; the FP32 pipe has 8x the MUFU rate
+                    asm volatile("rcp.approx.ftz.f32 %0, %0;" : "+f"(a[i]));
+                    a[i] += c;
+                }
             }
         }
     }
@@ -38,7 +43,7 @@ __global__ void __launch_bounds__(256) pipe_peak_kernel(float* sink, int iters) 
 
 extern "C" int po_microbench(int kind, double* result) {
     using namespace po;
-    if (kind < 0 || kind > 2 || !result) {
+    if (kind < 0 || kind > 3 || !result) {
         set_error("po_microbench: bad arguments");
         return PO_ERR_ARG;
     }
@@ -58,6 +63,7 @@ extern "C" int po_microbench(int kind, double* result) {
         if (kind == 0) pipe_peak_kernel<0><<<blocks, 256>>>(sink, iters);
         if (kind == 1) pipe_peak_kernel<1><<<blocks, 256>>>(sink, iters);
         if (kind == 2) pipe_peak_kernel<2><<<blocks, 256>>>(sink, iters);
+        if (kind == 3) pipe_peak_kernel<3><<<blocks, 256>>>(sink, iters);
         cudaEventRecord(e1, 0);
         PO_CUDA_CHECK(cudaEventSynchronize(e1));
         float ms = 0.f;

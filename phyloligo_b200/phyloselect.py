@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
-"""The front half of phyloselect.py on B200 (SURVEY.md 8f rank 4): K-medoids and HDBSCAN on the contig
-distance matrix, and the nearest-neighbour graph its t-SNE consumer starts from, computed on the device
-while the matrix is resident -- straight after the distance stage if wanted, without the round trip
-through a 40 GB file and 800 GB of host RAM the reference's documentation asks for.
+"""The front half of phyloselect.py on B200 (SURVEY.md 8f rank 4): K-medoids, HDBSCAN and the t-SNE projection
+of the contig distance matrix, computed on the device while the matrix is resident -- straight after the
+distance stage if wanted, without the round trip through a 40 GB file and 800 GB of host RAM the reference's documentation asks for.
 
 Mirrors reference phylopackage/bin/phyloselect.py: ``KMedoids`` (:37-309; same constructor
 arguments and fitted attributes), ``clusterize`` (:573-590), ``find_clusters`` (:403-428), the
@@ -10,10 +9,12 @@ matrix readers of ``main`` (:597-622), ``write_fastafile`` (:547-571) and the
 ``data_cluster_indexes.dat`` writer (:742-751).  ``HDBSCAN`` computes what the reference gets from
 the third-party hdbscan.HDBSCAN(metric="precomputed") with its default arguments (core distances,
 mutual-reachability MST, condensed tree, excess-of-mass selection), with MST ties broken by vertex
-index.  Plotting, t-SNE itself and the interactive loop are out of scope: ``knn_graph`` hands t-SNE the
-sparse precomputed neighbour graph scikit-learn's TSNE accepts in place of the dense matrix.
+index.  ``TSNE`` computes what the reference gets from sklearn.manifold.TSNE(metric="precomputed") (:381-398)
+with angle=0.0, i.e. the exact gradient; ``--tsne-out`` writes its embedding.  Plotting and the interactive loop
+are out of scope.
 
-There is no CPU fallback: the sums, assignments, selections and the MST run in libphyloligo_b200.so.
+There is no CPU fallback: the sums, assignments, selections, the MST and the t-SNE gradient run in
+libphyloligo_b200.so.
 """
 from __future__ import annotations
 
@@ -322,6 +323,252 @@ class HDBSCAN:
         return self.fit(X).labels_
 
 
+TSNE_MAX_K = 1024  # po_matrix_knn's largest k
+
+
+def check_tsne_matrix(D):
+    """Refuse (PhyloligoError) a device matrix holding a NaN, an infinite or a negative entry, as scikit-learn's
+    TSNE(metric="precomputed") does; the message names the first one in row-major order (po_tsne_check)."""
+    lib = _lib.load()
+    work = torch.empty(1, dtype=torch.int64, device=D.device)
+    rc = lib.po_tsne_check(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), _ptr(work), _stream())
+    _lib.check(rc, "po_tsne_check")
+
+
+def _fixed_sum(x):
+    """float64 sum of a device vector in a fixed order (po_tsne_sum), as a 1-element device tensor."""
+    out = torch.empty(1, dtype=torch.float64, device=x.device)
+    _lib.check(_lib.load().po_tsne_sum(_ptr(x), int(x.numel()), _ptr(out), _stream()), "po_tsne_sum")
+    return out
+
+
+def tsne_affinities(D, perplexity, as_sparse=False):
+    """The joint probabilities P of scikit-learn's TSNE(metric="precomputed", method="barnes_hut") from the device
+    matrix D: the k = min(n - 1, int(3 perplexity + 1)) nearest neighbours of every row (po_matrix_knn), their
+    squared distances, the per-row perplexity search (po_tsne_conditional), then P = (C + C^T) / sum(C + C^T) with
+    the pairs whose sum is 0 dropped, as scipy's sparse addition drops them.  Returns the symmetric CSR as device
+    tensors (indptr int64 [n + 1], indices int32, data float64), columns ascending in every row, or with
+    `as_sparse` the scipy CSR matrix.  The transpose and the merge of the two halves are torch sort and gather
+    plumbing; each merged value is one addition of two terms, and the total is a fixed-order sum, so the result
+    is deterministic."""
+    lib = _lib.load()
+    D = D if isinstance(D, torch.Tensor) and D.is_cuda else as_device_matrix(D)
+    n = int(D.shape[0])
+    k = min(n - 1, int(3.0 * perplexity + 1))
+    if k > TSNE_MAX_K:
+        raise ValueError("perplexity {} needs {} neighbours per point; at most {} are supported (perplexity <= 341)"
+                         .format(perplexity, k, TSNE_MAX_K))
+    idx, _ = knn_graph(D, k)
+    cond = torch.empty((n, k), dtype=torch.float64, device=D.device)
+    rc = lib.po_tsne_conditional(_ptr(D), int(D.stride(0)), _dt(D), n, _ptr(idx), k, float(perplexity), _ptr(cond), _stream())
+    _lib.check(rc, "po_tsne_conditional")
+    rows = torch.arange(n, dtype=torch.int64, device=D.device).repeat_interleave(k)
+    cols = idx.reshape(-1).to(torch.int64)
+    keys, order = torch.sort(torch.cat([rows * n + cols, cols * n + rows]), stable=True)
+    vals = torch.cat([cond.reshape(-1), cond.reshape(-1)])[order]
+    m = int(keys.numel())
+    first = torch.ones(m, dtype=torch.bool, device=D.device)
+    first[1:] = keys[1:] != keys[:-1]
+    starts = torch.nonzero(first).flatten()
+    nxt = torch.clamp(starts + 1, max=m - 1)
+    paired = (starts + 1 < m) & (keys[nxt] == keys[starts])
+    merged = vals[starts] + torch.where(paired, vals[nxt], torch.zeros_like(vals[nxt]))  # C_ij + C_ji (at most two terms)
+    keep = merged != 0
+    ukeys, data = keys[starts][keep], merged[keep]
+    indices = (ukeys % n).to(torch.int32)
+    indptr = torch.zeros(n + 1, dtype=torch.int64, device=D.device)
+    indptr[1:] = torch.cumsum(torch.bincount(ukeys // n, minlength=n), 0)
+    total = max(float(_fixed_sum(data).item()), float(np.finfo(np.float64).eps))
+    data = data / total
+    if not as_sparse:
+        return indptr, indices, data
+    from scipy.sparse import csr_matrix
+    return csr_matrix((data.cpu().numpy(), indices.cpu().numpy(), indptr.cpu().numpy()), shape=(n, n))
+
+
+def _device_csr(P, device):
+    if isinstance(P, tuple):
+        return tuple(t.to(device) for t in P)
+    P = P.tocsr()
+    return (torch.from_numpy(np.asarray(P.indptr, dtype=np.int64)).to(device),
+            torch.from_numpy(np.asarray(P.indices, dtype=np.int32)).to(device),
+            torch.from_numpy(np.asarray(P.data, dtype=np.float64)).to(device))
+
+
+class _Descent:
+    """Device state of one t-SNE optimisation: two position buffers, update, gains and the workspace."""
+
+    def __init__(self, P, Y0):
+        self.lib = _lib.load()
+        dev = P[0].device
+        self.P = P
+        self.n = int(Y0.shape[0])
+        self.Y = torch.as_tensor(np.ascontiguousarray(Y0, dtype=np.float32)).to(dev)
+        self.Y_next = torch.empty_like(self.Y)
+        self.update = torch.zeros((self.n, 2), dtype=torch.float64, device=dev)
+        self.gains = torch.ones((self.n, 2), dtype=torch.float32, device=dev)
+        self.work = torch.empty(int(self.lib.po_tsne_workspace(self.n)), dtype=torch.uint8, device=dev)
+        self.out = (C.c_double * 2)()
+
+    def gradient(self, mul, div, Y_next=None, grad=None, momentum=0.0, lr=0.0, update64=True, compute_error=False):
+        lib = self.lib
+        _lib.check(lib.po_tsne_repulsion(_ptr(self.Y), self.n, _ptr(self.work), _stream()), "po_tsne_repulsion")
+        indptr, indices, data = self.P
+        rc = lib.po_tsne_attraction_step(_ptr(indptr), _ptr(indices), _ptr(data), self.n, float(mul), float(div), _ptr(self.Y),
+                                         _ptr(self.work), _ptr(Y_next), _ptr(self.update), _ptr(self.gains), _ptr(grad),
+                                         float(momentum), float(lr), int(update64), self.out if compute_error else None, _stream())
+        _lib.check(rc, "po_tsne_attraction_step")
+        return self.out[0], self.out[1]
+
+    def descend(self, it, max_iter, momentum, lr, update64, mul, div, n_iter_without_progress, min_grad_norm, n_iter_check=50):
+        """scikit-learn's _gradient_descent: returns (error, last iteration index)."""
+        self.update.zero_()
+        self.gains.fill_(1.0)
+        error = best_error = np.finfo(float).max
+        best_iter = i = it
+        for i in range(it, max_iter):
+            check = (i + 1) % n_iter_check == 0
+            compute_error = check or i == max_iter - 1
+            kl, gn2 = self.gradient(mul, div, Y_next=self.Y_next, momentum=momentum, lr=lr, update64=update64,
+                                    compute_error=compute_error)
+            self.Y, self.Y_next = self.Y_next, self.Y
+            if compute_error:
+                error = kl
+            if check:
+                if error < best_error:
+                    best_error, best_iter = error, i
+                elif i - best_iter > n_iter_without_progress:
+                    break
+                if np.sqrt(gn2) <= min_grad_norm:
+                    break
+        return error, i
+
+
+def tsne_gradient(P, Y, exaggeration=1.0):
+    """(grad float32 [n, 2], KL) of the t-SNE objective at the positions Y for the joint probabilities P (the
+    device CSR of tsne_affinities or a scipy CSR): what scikit-learn's _kl_divergence_bh(angle=0.0) returns with
+    P * exaggeration, the repulsion summed exactly over all pairs on the device."""
+    dev = engine.require_cuda()
+    P = _device_csr(P, dev)
+    Y = Y.cpu().numpy() if isinstance(Y, torch.Tensor) else np.asarray(Y)
+    st = _Descent(P, Y)
+    grad = torch.empty((st.n, 2), dtype=torch.float32, device=dev)
+    kl, _ = st.gradient(exaggeration, 1.0, grad=grad, compute_error=True)
+    return grad.cpu().numpy(), kl
+
+
+def _random_state(seed):
+    """sklearn.utils.check_random_state"""
+    if seed is None or seed is np.random:
+        return np.random.mtrand._rand
+    if isinstance(seed, (int, np.integer)):
+        return np.random.RandomState(seed)
+    if isinstance(seed, np.random.RandomState):
+        return seed
+    raise ValueError("%r cannot be used to seed a numpy.random.RandomState instance" % (seed,))
+
+
+class TSNE:
+    """t-SNE on the device: what sklearn.manifold.TSNE(metric="precomputed", method="barnes_hut", angle=0.0)
+    computes (scikit-learn 1.9), which with angle 0 is the exact gradient of the sparse-P objective.  Same
+    constructor arguments and defaults; ``method``, ``angle``, ``verbose``, ``metric_params`` and ``n_jobs`` are
+    accepted at "barnes_hut", 0.0, 0, None and None only.  ``metric`` is "precomputed" (X is the N x N matrix:
+    ndarray, memmap or a device tensor, used in place and not modified) or one of the package's metrics (X is the
+    N x D profile matrix and the distances never leave the device).  ``init`` is "random" (scikit-learn's draw on
+    the host, bit for bit) or an (N, 2) array, used as float32.  Fitted attributes: ``embedding_`` (float32),
+    ``kl_divergence_``, ``n_iter_``, ``learning_rate_``."""
+
+    _EXPLORATION_MAX_ITER = 250
+    _N_ITER_CHECK = 50
+    # scikit-learn's arguments this implementation takes at one value only
+    FIXED = {"method": "barnes_hut", "angle": 0.0, "verbose": 0, "metric_params": None, "n_jobs": None}
+
+    def __init__(self, n_components=2, *, perplexity=30.0, early_exaggeration=12.0, learning_rate="auto", max_iter=1000,
+                 n_iter_without_progress=300, min_grad_norm=1e-7, metric="precomputed", metric_params=None, init="random",
+                 verbose=0, random_state=None, method="barnes_hut", angle=0.0, n_jobs=None):
+        given = {"method": method, "angle": angle, "verbose": verbose, "metric_params": metric_params, "n_jobs": n_jobs}
+        for key, value in given.items():
+            if value is not self.FIXED[key] and value != self.FIXED[key]:
+                raise ValueError("{}={!r} is not supported; only {!r} (the exact gradient)".format(key, value, self.FIXED[key]))
+        if n_components != 2:
+            raise ValueError("n_components={!r} is not supported; only 2".format(n_components))
+        if not perplexity > 0:
+            raise ValueError("perplexity must be positive, got {!r}".format(perplexity))
+        if not early_exaggeration >= 1:
+            raise ValueError("early_exaggeration must be at least 1, got {!r}".format(early_exaggeration))
+        if not (isinstance(learning_rate, str) and learning_rate == "auto") and not (
+                isinstance(learning_rate, (int, float, np.integer, np.floating)) and learning_rate > 0):
+            raise ValueError("learning_rate must be 'auto' or positive, got {!r}".format(learning_rate))
+        if not isinstance(max_iter, (int, np.integer)) or max_iter < self._EXPLORATION_MAX_ITER:
+            raise ValueError("max_iter must be an integer of at least 250, got {!r}".format(max_iter))
+        if isinstance(init, str) and init == "pca":
+            raise ValueError('The parameter init="pca" cannot be used with metric="precomputed".' if metric == "precomputed"
+                             else 'init="pca" is not supported; use "random" or an array')
+        if not (isinstance(init, str) and init == "random") and not isinstance(init, np.ndarray):
+            raise ValueError("init must be 'random' or an (n_samples, 2) array, got {!r}".format(init))
+        if metric != "precomputed" and metric not in _lib.METRICS:
+            raise ValueError("metric needs to be 'precomputed' or one of {}. Instead, '{}' was given.".format(sorted(_lib.METRICS), metric))
+        self.n_components = n_components
+        self.perplexity = perplexity
+        self.early_exaggeration = early_exaggeration
+        self.learning_rate = learning_rate
+        self.max_iter = max_iter
+        self.n_iter_without_progress = n_iter_without_progress
+        self.min_grad_norm = min_grad_norm
+        self.metric = metric
+        self.metric_params = metric_params
+        self.init = init
+        self.verbose = verbose
+        self.random_state = random_state
+        self.method = method
+        self.angle = angle
+        self.n_jobs = n_jobs
+
+    def _matrix(self, X):
+        if self.metric == "precomputed":
+            return as_device_matrix(X)
+        Xd = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(X)))
+        return engine.distance_matrix_device(Xd.to(engine.require_cuda()), self.metric, torch.float32, symmetric=True)
+
+    def fit_transform(self, X, y=None):
+        D = self._matrix(X)
+        n = int(D.shape[0])
+        if n < 2:
+            raise ValueError("TSNE needs at least 2 samples, got {}".format(n))
+        if self.perplexity >= n:
+            raise ValueError("perplexity ({}) must be less than n_samples ({})".format(self.perplexity, n))
+        if self.learning_rate == "auto":
+            self.learning_rate_ = np.maximum(n / self.early_exaggeration / 4, 50)
+        else:
+            self.learning_rate_ = self.learning_rate
+        check_tsne_matrix(D)
+        if isinstance(self.init, np.ndarray):
+            if self.init.shape != (n, 2):
+                raise ValueError("init has shape {}; ({}, 2) is expected".format(self.init.shape, n))
+            Y0 = self.init
+        else:
+            Y0 = 1e-4 * _random_state(self.random_state).standard_normal(size=(n, self.n_components)).astype(np.float32)
+        P = tsne_affinities(D, self.perplexity)
+        st = _Descent(P, Y0)
+        # scikit-learn's update is float64 when the learning rate is a float64 scalar ("auto": np.maximum), float32
+        # for a Python float
+        update64 = (self.learning_rate_ * np.ones(1, np.float32)).dtype == np.float64
+        ee, lr = float(self.early_exaggeration), float(self.learning_rate_)
+        kl, it = st.descend(0, self._EXPLORATION_MAX_ITER, 0.5, lr, update64, ee, 1.0, self._EXPLORATION_MAX_ITER,
+                            self.min_grad_norm, self._N_ITER_CHECK)
+        if it < self._EXPLORATION_MAX_ITER or self.max_iter - self._EXPLORATION_MAX_ITER > 0:
+            kl, it = st.descend(it + 1, self.max_iter, 0.8, lr, update64, ee, ee, self.n_iter_without_progress, self.min_grad_norm,
+                                self._N_ITER_CHECK)
+        self.n_iter_ = it
+        self.kl_divergence_ = kl
+        self.embedding_ = st.Y.cpu().numpy()
+        return self.embedding_
+
+    def fit(self, X, y=None):
+        self.fit_transform(X)
+        return self
+
+
 # ---------------------------------------------------------------------------
 # the script's functions
 # ---------------------------------------------------------------------------
@@ -418,11 +665,15 @@ def get_cmd(argv=None):
     parser.add_argument("--large", action="store", choices=["memmap", "h5py"], dest="large", default=False,
                         help="Format of a matrix written with phyloligo.py --large")
     parser.add_argument("-o", action="store", dest="outputdir", required=True)
-    parser.add_argument("-t", action="store_true", dest="performtsne", default=False, help="(not built: plotting is out of scope)")
+    parser.add_argument("-t", action="store_true", dest="performtsne", default=False,
+                        help="(not built: plotting is out of scope; --tsne-out writes the embedding)")
     parser.add_argument("--interactive", action="store_true", dest="interactive", default=False,
                         help="(not built: plotting is out of scope)")
     parser.add_argument("--noX", action="store_true", dest="noX", help="accepted for compatibility")
-    parser.add_argument("-p", action="store", dest="perplexity", default=100, type=int, help="accepted for compatibility")
+    parser.add_argument("-p", action="store", dest="perplexity", default=100, type=int, help="t-SNE perplexity (--tsne-out)")
+    parser.add_argument("--tsne-out", action="store", dest="tsne_out",
+                        help="write the 2-D t-SNE embedding of the matrix (perplexity -p, random_state 0) to this file: one "
+                             "tab-separated %%.18e row per contig")
     parser.add_argument("-q", "--infreq", action="store", dest="in_freq_file", help="accepted for compatibility")
     # without a matrix file: profile the assembly and keep the matrix on the device
     parser.add_argument("--assembly", action="store", dest="assembly",
@@ -433,7 +684,7 @@ def get_cmd(argv=None):
     params = parser.parse_args(argv)
     if params.performtsne or params.interactive:
         print("Error, t-SNE projection and the interactive mode draw pictures: not part of the GPU front half "
-              "(use knn_graph() to feed sklearn.manifold.TSNE(metric='precomputed'))", file=sys.stderr)
+              "(--tsne-out FILE writes the 2-D t-SNE embedding computed on the device)", file=sys.stderr)
         sys.exit(1)
     if not params.distmat and not params.assembly:
         print("Error, give a matrix (-i) or an assembly (--assembly)", file=sys.stderr)
@@ -467,6 +718,9 @@ def main(argv=None):
     if params.fastafile:
         print("Write fasta per classes in {}/data_fasta_*.fa".format(params.outputdir))
         write_fastafile(labels_pred, params.fastafile, params.outputdir)
+    if params.tsne_out:
+        print("Store t-SNE embedding in {}".format(params.tsne_out))
+        np.savetxt(params.tsne_out, TSNE(perplexity=params.perplexity, random_state=0).fit(matrix).embedding_, delimiter="\t")
     return 0
 
 
