@@ -417,18 +417,44 @@ int po_tsne_attraction_step(const int64_t* d_indptr, const int* d_indices, const
                             const float* d_Y, void* d_work, float* d_Y_next, double* d_update, float* d_gains, float* d_grad,
                             double momentum, double learning_rate, int update64, double* h_kl_gradnorm2, po_stream_t stream);
 
+/*
+ * Hierarchical clustering of the resident matrix: the tree phyloselect.R builds with hclust (:22-35), computed
+ * as scipy.cluster.hierarchy.linkage(squareform(D, checks=False), method) computes it, bit for bit.
+ * method: 0 single, 1 complete, 2 average, 3 weighted, 4 ward.
+ *   po_linkage_workspace     bytes of d_work po_linkage_run needs for n points
+ *   po_linkage_run           one persistent cooperative launch (one CTA per SM at most, steps separated by
+ *                            grid.sync()).  single: scipy's mst_single_linkage (Prim from vertex 0) on d_D in
+ *                            place, n - 1 steps.  Otherwise scipy's nn_chain on d_W, a float64 n x n working copy
+ *                            of d_D (row stride n) that this call fills: every scan takes the minimum of the tip's
+ *                            row (smallest index on ties; the chain's previous entry when it holds the minimum),
+ *                            every merge applies the Lance-Williams update to row y and column y in float64 without
+ *                            FMA contraction.  At most 3 (n - 1) scans: past that bound the launch stops and the
+ *                            call fails.  Writes the n - 1 raw merges (d_zx, d_zy, d_zh: x, y, height) in merge
+ *                            order and *h_phases = the number of grid barriers.  d_D is read only; it must be
+ *                            finite and symmetric (po_hdbscan_check).  Synchronises `stream`.
+ *   po_linkage_tree          host: the stable sort of the raw merges by height (NaN last; numpy's mergesort
+ *                            argsort) and scipy's label (union-find, new clusters n, n + 1, ...) into Z, the
+ *                            row-major (n - 1) x 4 float64 linkage matrix
+ */
+int64_t po_linkage_workspace(int64_t n);
+int po_linkage_run(const void* d_D, int64_t ld, int dtype, int64_t n, int method, double* d_W, void* d_work, int64_t* d_zx,
+                   int64_t* d_zy, double* d_zh, int64_t* h_phases, po_stream_t stream);
+int po_linkage_tree(int64_t n, const int64_t* zx, const int64_t* zy, const double* zh, double* Z);
+
 /* Number of kernels this library has launched since load (for bench.py's gpu_launches). */
 int64_t po_launch_count(void);
 
 /* Average device time (ms) of the launches of one kernel family since the last
  * po_timing_reset(): CUDA events recorded on the launching stream around each
- * launch while timing is enabled.  family: 0 = profiling, 1 = distance tile. */
+ * launch while timing is enabled.  family: 0 = profiling, 1 = distance tile, 2 = the linkage kernels'
+ * cooperative launch (po_linkage_run). */
 int po_timing_enable(int on);
 int po_timing_reset(void);
 int po_timing_read(int family, double* total_ms, int64_t* launches);
 
 /* Pipe-peak microbenchmark for roofline denominators that MEASURED_PEAKS.json lacks.
- * kind 0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s (best of 4 timed runs). */
+ * kind 0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s (best of 4 timed runs),
+ * 4: microseconds per grid.sync() of the linkage kernels' grid (least of 4 timed runs). */
 int po_microbench(int kind, double* result);
 
 #ifdef __cplusplus

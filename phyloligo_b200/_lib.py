@@ -33,6 +33,7 @@ EXPORTED = [
     "po_matrix_rowsums", "po_matrix_argmin_rows", "po_cluster_argmin", "po_matrix_knn",
     "po_hdbscan_check", "po_matrix_kth", "po_hdbscan_mst_workspace", "po_hdbscan_mst_init", "po_hdbscan_mst_round", "po_hdbscan_tree",
     "po_tsne_check", "po_tsne_conditional", "po_tsne_sum", "po_tsne_workspace", "po_tsne_repulsion", "po_tsne_attraction_step",
+    "po_linkage_workspace", "po_linkage_run", "po_linkage_tree",
     "po_launch_count", "po_timing_enable", "po_timing_reset", "po_timing_read", "po_microbench",
 ]
 
@@ -152,6 +153,12 @@ def load():
     lib.po_tsne_attraction_step.argtypes = [vp, vp, vp, i64, C.c_double, C.c_double, vp, vp, vp, vp, vp, vp, C.c_double,
                                             C.c_double, i32, C.POINTER(C.c_double), vp]
     lib.po_tsne_attraction_step.restype = i32
+    lib.po_linkage_workspace.argtypes = [i64]
+    lib.po_linkage_workspace.restype = i64
+    lib.po_linkage_run.argtypes = [vp, i64, i32, i64, i32, vp, vp, vp, vp, vp, C.POINTER(i64), vp]
+    lib.po_linkage_run.restype = i32
+    lib.po_linkage_tree.argtypes = [i64, vp, vp, vp, vp]
+    lib.po_linkage_tree.restype = i32
     lib.po_launch_count.restype = i64
     lib.po_timing_enable.argtypes = [i32]
     lib.po_timing_enable.restype = i32
@@ -198,7 +205,8 @@ def timing_read(family: int):
 
 
 def microbench(kind: int) -> float:
-    """0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s."""
+    """0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s,
+    4: microseconds per grid barrier of the linkage kernels' grid."""
     out = C.c_double()
     check(load().po_microbench(kind, C.byref(out)), "po_microbench")
     return out.value

@@ -95,4 +95,7 @@ int launch_jsd(const void* d_P, int64_t n, int64_t dim, int64_t row0, int64_t ro
                void* d_out, int64_t ld_out, int64_t out_row0, int64_t out_col0, void* d_mir, int64_t ld_mir,
                int64_t mir_row0, int64_t mir_col0, int out_dtype, unsigned flags, cudaStream_t stream);
 
+// microseconds per grid.sync() of the linkage kernels' grid (po_linkage.cu; po_microbench kind 4)
+int barrier_latency_us(double* result);
+
 }  // namespace po

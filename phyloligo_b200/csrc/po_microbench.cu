@@ -4,6 +4,7 @@
 //   kind 1: MUFU.LG2 throughput, 1e12 op/s
 //   kind 2: POPC throughput, 1e12 op/s
 //   kind 3: MUFU.RCP throughput (rcp.approx.ftz.f32, the t-SNE repulsion's reciprocal), 1e12 op/s
+//   kind 4: grid-barrier latency, microseconds per grid.sync() of the linkage kernels' grid (po_linkage.cu)
 #include "po_common.cuh"
 
 namespace po {
@@ -43,10 +44,11 @@ __global__ void __launch_bounds__(256) pipe_peak_kernel(float* sink, int iters) 
 
 extern "C" int po_microbench(int kind, double* result) {
     using namespace po;
-    if (kind < 0 || kind > 3 || !result) {
+    if (kind < 0 || kind > 4 || !result) {
         set_error("po_microbench: bad arguments");
         return PO_ERR_ARG;
     }
+    if (kind == 4) return barrier_latency_us(result);
     int dev = 0, sms = 0;
     PO_CUDA_CHECK(cudaGetDevice(&dev));
     PO_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """The front half of phyloselect.py on B200 (SURVEY.md 8f rank 4): K-medoids, HDBSCAN and the t-SNE projection
-of the contig distance matrix, computed on the device while the matrix is resident -- straight after the
+of the contig distance matrix, and phyloselect.R's hierarchical tree, computed on the device while the matrix is resident -- straight after the
 distance stage if wanted, without the round trip through a 40 GB file and 800 GB of host RAM the reference's documentation asks for.
 
 Mirrors reference phylopackage/bin/phyloselect.py: ``KMedoids`` (:37-309; same constructor
@@ -10,11 +10,12 @@ matrix readers of ``main`` (:597-622), ``write_fastafile`` (:547-571) and the
 the third-party hdbscan.HDBSCAN(metric="precomputed") with its default arguments (core distances,
 mutual-reachability MST, condensed tree, excess-of-mass selection), with MST ties broken by vertex
 index.  ``TSNE`` computes what the reference gets from sklearn.manifold.TSNE(metric="precomputed") (:381-398)
-with angle=0.0, i.e. the exact gradient; ``--tsne-out`` writes its embedding.  Plotting and the interactive loop
-are out of scope.
+with angle=0.0, i.e. the exact gradient; ``--tsne-out`` writes its embedding.  ``linkage`` / ``HClust`` build the
+tree bin/phyloselect.R:22-35 builds with hclust, as scipy.cluster.hierarchy.linkage computes it; ``-m hclust`` cuts
+it and ``--tree-out`` writes it in Newick format.  Plotting and the interactive loop are out of scope.
 
-There is no CPU fallback: the sums, assignments, selections, the MST and the t-SNE gradient run in
-libphyloligo_b200.so.
+There is no CPU fallback: the sums, assignments, selections, the MST, the t-SNE gradient and the linkage loop run
+in libphyloligo_b200.so.
 """
 from __future__ import annotations
 
@@ -569,6 +570,158 @@ class TSNE:
         return self
 
 
+LINKAGE_METHODS = {"single": 0, "complete": 1, "average": 2, "weighted": 3, "ward": 4}
+
+
+def _check_linkage_method(method):
+    if method in ("centroid", "median"):
+        raise ValueError("method={!r} is not supported: scipy builds it with a different algorithm (the Lance-Williams "
+                         "update is not reducible there); use one of {}".format(method, list(LINKAGE_METHODS)))
+    if method not in LINKAGE_METHODS:
+        raise ValueError("method must be one of {}, got {!r}".format(list(LINKAGE_METHODS), method))
+
+
+def linkage_bytes(n, method):
+    """Device bytes linkage(D, method) allocates for n rows besides D: the float64 n x n working copy (not for
+    "single", which reads D in place), the workspace and the raw merges."""
+    _check_linkage_method(method)
+    return int(_lib.load().po_linkage_workspace(n)) + 24 * (n - 1) + (0 if method == "single" else 8 * n * n)
+
+
+def check_linkage_fits(n, method, free_bytes):
+    """Refuse (PhyloligoError) a linkage of n rows whose device memory (linkage_bytes) exceeds free_bytes."""
+    need = linkage_bytes(n, method)
+    if need > free_bytes:
+        raise PhyloligoError("linkage(method={!r}) of {} rows needs {} bytes of device memory ({}), {} are free".format(
+            method, n, need, "the float64 working copy of the matrix and the workspace" if method != "single" else "the workspace",
+            free_bytes))
+
+
+def linkage_raw(D, method="average"):
+    """The n - 1 merges of scipy's nn_chain (Prim for "single") on the device matrix D, in merge order, before the
+    sort and relabelling: device tensors (x int64, y int64, height float64) and the number of grid barriers the
+    launch took (po_linkage_run).  D is checked (check_matrix) and not modified."""
+    _check_linkage_method(method)
+    lib = _lib.load()
+    n = int(D.shape[0])
+    if n < 2:
+        raise ValueError("linkage needs at least 2 observations, got {}".format(n))
+    check_matrix(D)
+    dev = D.device
+    free, _ = torch.cuda.mem_get_info(dev)
+    free += torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+    check_linkage_fits(n, method, free)
+    W = None if method == "single" else torch.empty((n, n), dtype=torch.float64, device=dev)
+    work = torch.empty(int(lib.po_linkage_workspace(n)), dtype=torch.uint8, device=dev)
+    zx = torch.empty(n - 1, dtype=torch.int64, device=dev)
+    zy = torch.empty_like(zx)
+    zh = torch.empty(n - 1, dtype=torch.float64, device=dev)
+    phases = C.c_int64()
+    rc = lib.po_linkage_run(_ptr(D), int(D.stride(0)), _dt(D), n, LINKAGE_METHODS[method], _ptr(W), _ptr(work), _ptr(zx), _ptr(zy),
+                            _ptr(zh), C.byref(phases), _stream())
+    _lib.check(rc, "po_linkage_run")
+    return zx, zy, zh, phases.value
+
+
+def linkage_tree(x, y, h):
+    """Host stage (po_linkage_tree): the stable sort of the raw merges by height and scipy's label, giving the
+    (n - 1, 4) linkage matrix."""
+    x = np.ascontiguousarray(x, dtype=np.int64)
+    y = np.ascontiguousarray(y, dtype=np.int64)
+    h = np.ascontiguousarray(h, dtype=np.float64)
+    n = len(x) + 1
+    Z = np.empty((n - 1, 4), dtype=np.float64)
+    rc = _lib.load().po_linkage_tree(n, *[C.c_void_p(a.ctypes.data) for a in (x, y, h, Z)])
+    _lib.check(rc, "po_linkage_tree")
+    return Z
+
+
+def linkage(D, method="average"):
+    """Hierarchical clustering on the device: the (n - 1, 4) float64 array that
+    scipy.cluster.hierarchy.linkage(squareform(D, checks=False), method) returns, bit for bit, for method "single",
+    "complete", "average", "weighted" or "ward".  D is an ndarray, a memmap or a device tensor (used in place and
+    not modified); it must be square, bitwise symmetric and finite.  All but "single" use a float64 working copy of
+    D on the device (8 n^2 bytes); a matrix whose copy does not fit is refused before anything is allocated."""
+    _check_linkage_method(method)
+    D = as_device_matrix(D)
+    x, y, h, _ = linkage_raw(D, method)
+    return linkage_tree(x.cpu().numpy(), y.cpu().numpy(), h.cpu().numpy())
+
+
+class HClust:
+    """The tree phyloselect.R builds with hclust, cut into flat clusters.  ``linkage_`` is Z (see linkage) and
+    ``labels_`` = scipy.cluster.hierarchy.fcluster(Z, n_clusters, "maxclust") - 1, numbered from 0 as KMedoids'
+    labels are (fewer than n_clusters clusters when heights tie, as scipy gives).  ``metric`` is "precomputed" (X
+    is the N x N matrix: ndarray, memmap or a device tensor, used in place) or one of the package's metrics (X is
+    the N x D profile matrix and the distances never leave the device)."""
+
+    def __init__(self, n_clusters=8, linkage="average", metric="precomputed"):
+        if not isinstance(n_clusters, (int, np.integer)) or isinstance(n_clusters, bool) or n_clusters < 1:
+            raise ValueError("n_clusters must be a positive integer, got {!r}".format(n_clusters))
+        _check_linkage_method(linkage)
+        if metric != "precomputed" and metric not in _lib.METRICS:
+            raise ValueError("metric needs to be 'precomputed' or one of {}. Instead, '{}' was given.".format(sorted(_lib.METRICS), metric))
+        self.n_clusters = int(n_clusters)
+        self.linkage = linkage
+        self.metric = metric
+
+    def fit(self, X, y=None):
+        from scipy.cluster.hierarchy import fcluster
+        if self.metric == "precomputed":
+            D = X
+        else:
+            Xd = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(X)))
+            D = engine.distance_matrix_device(Xd.to(engine.require_cuda()), self.metric, torch.float32, symmetric=True)
+        self.linkage_ = linkage(D, self.linkage)
+        self.labels_ = fcluster(self.linkage_, self.n_clusters, "maxclust").astype(np.int64) - 1
+        return self
+
+    def fit_predict(self, X, y=None):
+        return self.fit(X).labels_
+
+
+def newick_name(name):
+    """A Newick leaf label: single-quoted, with every ' doubled, when it is empty or holds a blank or one of
+    ( ) [ ] ' : ; ,"""
+    s = str(name)
+    if s == "" or any(c in "()[]':;," or c.isspace() for c in s):
+        return "'" + s.replace("'", "''") + "'"
+    return s
+
+
+def write_newick(Z, names, path):
+    """Write the linkage matrix Z as a rooted Newick tree with leaves names[0 .. n).  Node depth is height / 2
+    (the ultrametric convention of ape's as.phylo(hclust)), so a leaf-to-leaf path is as long as the height of the
+    two leaves' merge.  Children are written in Z's order (column 0, then column 1).  The walk is iterative:
+    single-linkage trees can be n deep."""
+    Z = np.asarray(Z, dtype=np.float64)
+    n = Z.shape[0] + 1
+    if Z.ndim != 2 or Z.shape[1] != 4 or len(names) != n:
+        raise ValueError("a ({}, 4) linkage matrix and {} names are expected, got {} and {} names".format(n - 1, n, Z.shape, len(names)))
+    depth = Z[:, 2] / 2.0
+
+    def length(child, parent_depth):
+        return repr(float(parent_depth - (depth[child - n] if child >= n else 0.0)))
+
+    out = []
+    stack = [(2 * n - 2, "")]
+    while stack:
+        item = stack.pop()
+        if isinstance(item, str):
+            out.append(item)
+            continue
+        node, tail = item
+        if node < n:
+            out.append(newick_name(names[node]) + tail)
+            continue
+        k = node - n
+        a, b = int(Z[k, 0]), int(Z[k, 1])
+        out.append("(")
+        stack += [")" + tail, (b, ":" + length(b, depth[k])), ",", (a, ":" + length(a, depth[k]))]
+    with open(path, "w") as fh:
+        fh.write("".join(out) + ";\n")
+
+
 # ---------------------------------------------------------------------------
 # the script's functions
 # ---------------------------------------------------------------------------
@@ -591,19 +744,31 @@ def read_matrix(path, large=False):
     return read_distmat(path)
 
 
-def find_clusters(data, method, kwargs):
-    """reference :403-428"""
+def find_clusters(data, method, kwargs, return_model=False):
+    """reference :403-428; with `return_model` the fitted estimator (its ``labels_`` are what is returned
+    otherwise; HClust's also holds the tree, ``linkage_``)"""
     if method == "kmedoids":
-        return KMedoids(**kwargs).fit(data).labels_
-    if method == "hdbscan":
-        return HDBSCAN(**kwargs).fit(data).labels_
-    print("Error, unknown method {}".format(method), file=sys.stderr)
-    sys.exit(1)
+        model = KMedoids(**kwargs)
+    elif method == "hdbscan":
+        model = HDBSCAN(**kwargs)
+    elif method == "hclust":
+        model = HClust(**kwargs)
+    else:
+        print("Error, unknown method {}".format(method), file=sys.stderr)
+        sys.exit(1)
+    model.fit(data)
+    return model if return_model else model.labels_
 
 
-def clusterize(data, method, min_cluster_size=None, min_samples=None, nbk=None):
+def clusterize(data, method, min_cluster_size=None, min_samples=None, nbk=None, linkage_method=None, return_model=False):
     """reference :573-590"""
     kwargs = dict()
+    if method == "hclust":
+        if nbk is not None:
+            kwargs["n_clusters"] = nbk
+        if linkage_method is not None:
+            kwargs["linkage"] = linkage_method
+        kwargs["metric"] = "precomputed"
     if method == "hdbscan":
         if min_cluster_size is not None:
             kwargs["min_cluster_size"] = min_cluster_size
@@ -614,7 +779,7 @@ def clusterize(data, method, min_cluster_size=None, min_samples=None, nbk=None):
         if nbk is not None:
             kwargs["n_clusters"] = nbk
         kwargs["distance_metric"] = "precomputed"
-    return find_clusters(data, method, kwargs)
+    return find_clusters(data, method, kwargs, return_model=return_model)
 
 
 def write_cluster_indexes(labels_pred, pathout):
@@ -649,17 +814,36 @@ def write_fastafile(labels_pred, fastafile, outputdir):
                     outf.write(seq[p:p + 60] + b"\n")
 
 
+def fasta_record_ids(fastafile):
+    """The id of every record of a FASTA file: its title up to the first blank."""
+    text = np.fromfile(fastafile, dtype=np.uint8)
+    begin, end = engine.fasta_index(text)
+    raw = text.tobytes()
+    ids = []
+    for s, b in zip(engine.fasta_header_starts(raw, begin, end), begin):
+        title = raw[int(s):int(b)].strip()
+        title = title[1:] if title.startswith(b">") else title
+        ids.append((title.split(None, 1) or [b""])[0].decode("utf-8", "replace"))
+    return ids
+
+
 def get_cmd(argv=None):
     parser = argparse.ArgumentParser(description="Cluster contigs from their oligonucleotide-profile distances on B200 GPUs")
     parser.add_argument("-i", action="store", dest="distmat", help="The input matrix file")
-    parser.add_argument("-m", action="store", dest="method", required=True, choices=["hdbscan", "kmedoids"],
+    parser.add_argument("-m", action="store", dest="method", required=True, choices=["hdbscan", "kmedoids", "hclust"],
                         help="Method to use to compute cluster on the distance matrix: HDBSCAN (--minclustersize, "
-                             "--minsamples; noise goes to data_fasta_unclust.fa) or K-medoids (-k)")
+                             "--minsamples; noise goes to data_fasta_unclust.fa), K-medoids (-k) or the hierarchical "
+                             "tree cut into -k clusters (--linkage)")
     parser.add_argument("--minclustersize", action="store", dest="min_cluster_size", type=int,
                         help="Set the minimal cluster size of an HDBSCAN cluster")
     parser.add_argument("--minsamples", action="store", dest="min_samples", type=int,
                         help="Set the minimal sample size of an HDBSCAN cluster")
     parser.add_argument("-k", action="store", dest="nbk", type=int, help="Number of cluster")
+    parser.add_argument("--linkage", action="store", dest="linkage", default="average", choices=list(LINKAGE_METHODS),
+                        help="linkage of -m hclust and --tree-out (scipy.cluster.hierarchy.linkage's method)")
+    parser.add_argument("--tree-out", action="store", dest="tree_out",
+                        help="write the hierarchical tree of the matrix (--linkage) to this file in Newick format; leaves "
+                             "are the FASTA record ids with -f or --assembly, row indices otherwise")
     parser.add_argument("-f", action="store", dest="fastafile",
                         help="Path of the original fasta file used for the computation of the distance matrix")
     parser.add_argument("--large", action="store", choices=["memmap", "h5py"], dest="large", default=False,
@@ -710,8 +894,10 @@ def main(argv=None):
         print("Read matrix")
         matrix = read_matrix(params.distmat, params.large)
     print("Clusterize")
-    labels_pred = clusterize(matrix, params.method, min_cluster_size=params.min_cluster_size, min_samples=params.min_samples,
-                             nbk=params.nbk)
+    model = clusterize(matrix, params.method, min_cluster_size=params.min_cluster_size, min_samples=params.min_samples,
+                       nbk=params.nbk, linkage_method=params.linkage, return_model=True)
+    labels_pred = model.labels_
+    Z = getattr(model, "linkage_", None)  # -m hclust: the tree --tree-out writes
     pathout = os.path.join(params.outputdir, "data_cluster_indexes.dat")
     print("Store cluster indexes in {}".format(pathout))
     write_cluster_indexes(labels_pred, pathout)
@@ -721,6 +907,14 @@ def main(argv=None):
     if params.tsne_out:
         print("Store t-SNE embedding in {}".format(params.tsne_out))
         np.savetxt(params.tsne_out, TSNE(perplexity=params.perplexity, random_state=0).fit(matrix).embedding_, delimiter="\t")
+    if params.tree_out:
+        print("Store the {} linkage tree in {}".format(params.linkage, params.tree_out))
+        if Z is None:
+            Z = linkage(matrix, params.linkage)
+        names = fasta_record_ids(params.fastafile) if params.fastafile else [str(i) for i in range(Z.shape[0] + 1)]
+        if len(names) != Z.shape[0] + 1:
+            raise PhyloligoError("{} holds {} records, the matrix {} rows".format(params.fastafile, len(names), Z.shape[0] + 1))
+        write_newick(Z, names, params.tree_out)
     return 0
 
 
