@@ -134,7 +134,7 @@ int po_profile_batch(const uint8_t* d_text, const int64_t* d_begin, const int64_
  *   JSD       : float32 with exact zeros biased to 1e-30, dim rounded up to a multiple of 32
  *               and n to a multiple of 64, stored as bulk-copy blocks: [n/64][dim/32] blocks
  *               of [32 dims][64 profiles], then [n/32][dim/32] blocks of
- *               [32 dims][32 profiles][2] (every value twice, for packed f32x2 math)
+ *               [32 dims][32 profiles]
  * po_prepared_row_bytes is the per-profile figure of the row-major layouts (Eucl, BC, KT, and
  * the CUDA-core SC layout); the blocked layouts (JSD, EuclGram, tensor-core SC) are padded to
  * whole groups of profiles -- use po_prepared_bytes.
@@ -454,7 +454,8 @@ int po_timing_read(int family, double* total_ms, int64_t* launches);
 
 /* Pipe-peak microbenchmark for roofline denominators that MEASURED_PEAKS.json lacks.
  * kind 0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s (best of 4 timed runs),
- * 4: microseconds per grid.sync() of the linkage kernels' grid (least of 4 timed runs). */
+ * 4: microseconds per grid.sync() of the linkage kernels' grid (least of 4 timed runs),
+ * 5..12: warp-instructions per SM per clock of packed-f32x2 operand forms (csrc/po_microbench.cu; best of 4). */
 int po_microbench(int kind, double* result);
 
 #ifdef __cplusplus

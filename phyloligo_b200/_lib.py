@@ -206,7 +206,8 @@ def timing_read(family: int):
 
 def microbench(kind: int) -> float:
     """0: FP32 FFMA TFLOP/s, 1: MUFU.LG2 1e12 op/s, 2: POPC 1e12 op/s, 3: MUFU.RCP 1e12 op/s,
-    4: microseconds per grid barrier of the linkage kernels' grid."""
+    4: microseconds per grid barrier of the linkage kernels' grid, 5..12: warp-instructions per SM per clock of
+    the packed-f32x2 operand forms listed in csrc/po_microbench.cu."""
     out = C.c_double()
     check(load().po_microbench(kind, C.byref(out)), "po_microbench")
     return out.value

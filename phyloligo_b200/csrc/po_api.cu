@@ -203,7 +203,7 @@ int64_t po_prepared_row_bytes(int metric, int64_t dim) {
         set_error("po_prepared_row_bytes: bad metric/dim");
         return PO_ERR_ARG;
     }
-    return prepared_row_elems(metric, dim) * 4 * (metric == PO_JSD ? 3 : 1);
+    return prepared_row_elems(metric, dim) * 4 * (metric == PO_JSD ? 2 : 1);
 }
 
 int64_t po_prepared_bytes(int metric, int64_t n, int64_t dim) {

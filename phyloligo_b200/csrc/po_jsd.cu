@@ -17,13 +17,17 @@
 //
 // Layout.  po_prepare_profiles(JSD) writes the operands "blocked": for every group of
 // 64 profiles and every chunk of 32 dimensions one 8 KB block [32 dims][64 profiles]
-// (the column operand, B), and for every group of 32 profiles one 8 KB block
-// [32 dims][32 profiles][2] with each value stored twice (the row operand, A).  A CTA
-// computes a 32 x 64 tile; per chunk it needs exactly one A block and one B block, each
-// a single contiguous cp.async.bulk into a 3-stage shared-memory ring.  Thread (ty, tx)
-// owns rows 4ty..4ty+3 and columns 4tx..4tx+3: per dimension it reads {a,a} pairs and
-// {b_j, b_j+1} pairs with three 128-bit shared loads and evaluates 16 terms as 8 packed
-// f32x2 operations per step of the recipe (add, sub, mul, mul, Horner FMAs, mul, FMA).
+// (the column operand, B), and for every group of 32 profiles one 4 KB block
+// [32 dims][32 profiles] (the row operand, A).  A CTA computes a 32 x 64 tile; per chunk
+// it needs exactly one A block and one B block, each a single contiguous cp.async.bulk
+// into a 3-stage shared-memory ring.  Thread (ty, tx) owns rows 4ty..4ty+3 and columns
+// 4tx..4tx+3: per dimension it reads its four row values and its {b_j, b_j+1} pairs with
+// two 128-bit shared loads and evaluates 16 terms as 8 packed f32x2 operations per step
+// of the recipe (add, sub, mul, mul, Horner FMAs, mul, FMA).  The row value enters the
+// add and the subtract as pk2(a, a) of one register, which ptxas emits as the scalar
+// broadcast operand (R.F32) of FADD2: three 32-bit register reads instead of four.  The
+// FP32 pipe of this loop is fed by register-file reads (DESIGN.md section 4.3), so the
+// operand that is the same in both halves is stored and read once.
 //
 // Two-phase evaluation.  Phase 1 adds the series value q*G(u) for every term and tracks
 // the largest u it met.  If some lane of the warp met u > 1/2 in this dimension, phase 2
@@ -75,9 +79,11 @@ constexpr int JDK = 32;            // dimensions per chunk
 #endif
 constexpr int JSTAGES = JSD_STAGES;
 constexpr int JUNROLL = JSD_UNROLL;
-constexpr int JBLOCK_FLOATS = 2048;  // one operand block: 8 KB
-constexpr int JSTAGE_BYTES = 2 * JBLOCK_FLOATS * 4;
+constexpr int JA_FLOATS = JDK * JT_M;  // one row-operand block: 4 KB
+constexpr int JB_FLOATS = JDK * JT_N;  // one column-operand block: 8 KB
+constexpr int JSTAGE_BYTES = (JA_FLOATS + JB_FLOATS) * 4;
 constexpr int JTHREADS = 128;
+constexpr int JT_TOTALS_BYTES = 16 * JTHREADS * 8;  // every thread's 16 float64 totals
 constexpr int JRASTER = 128;        // tile columns per rasterisation chunk
 
 // ---- packed f32x2 helpers (sm_100 FADD2 / FMUL2 / FFMA2) ----
@@ -188,7 +194,7 @@ __device__ __forceinline__ void bulk_g2s(unsigned dst, const void* src, unsigned
 
 struct JsdParams {
     const float* B;   // column-operand blocks  [n/64 groups][nchunks][32][64]
-    const float* A;   // row-operand blocks     [n/32 groups][nchunks][32][32][2]
+    const float* A;   // row-operand blocks     [n/32 groups][nchunks][32][32]
     const float* gmin;  // [n/64 groups][nchunks * 32] smallest / largest value of the group per (permuted) dimension
     const float* gmax;
     int nchunks;
@@ -205,18 +211,23 @@ struct JsdParams {
 
 // One chunk (32 dimensions) of a thread's 4 x 4 pairs, as 8 packed term pairs per dimension.
 // V = 0: degree-4 fit, u <= 1/4 guaranteed; V = 1: degree-6 fit, u < 1/2 guaranteed; V = 2: two phases.
+// V = 2 tracks u only in the dimensions whose bit is set in p2dims: in the others the value ranges of the
+// warp's rows and of the column group bound u below 1/2, so phase 2 cannot run there and the loop computes
+// exactly what V = 1 computes.
 template <int V>
-__device__ __forceinline__ void jsd_chunk(const ulonglong2* __restrict__ sA, const ulonglong2* __restrict__ sB, u64 (&c2)[4][2]) {
+__device__ __forceinline__ void jsd_chunk(const float4* __restrict__ sA, const ulonglong2* __restrict__ sB, u64 (&c2)[4][2],
+                                          unsigned p2dims) {
     const u64 g6 = pk2(JG6, JG6), g5 = pk2(JG5, JG5), g4 = pk2(JG4, JG4);
     const u64 g3 = pk2(JG3, JG3), g2 = pk2(JG2, JG2), g1 = pk2(JG1, JG1), g0 = pk2(JG0, JG0);
     const u64 h4 = pk2(JH4, JH4), h3 = pk2(JH3, JH3), h2 = pk2(JH2, JH2), h1 = pk2(JH1, JH1), h0 = pk2(JH0, JH0);
 #pragma unroll JUNROLL
     for (int d = 0; d < JDK; ++d) {
-        const ulonglong2 A01 = sA[d * 16], A23 = sA[d * 16 + 1], Bv = sB[d * 16];
-        const u64 a2[4] = {A01.x, A01.y, A23.x, A23.y};
+        const float4 Av = sA[d * (JT_M / 4)];
+        const ulonglong2 Bv = sB[d * (JT_N / 4)];
+        const float a[4] = {Av.x, Av.y, Av.z, Av.w};
+        const u64 a2[4] = {pk2(a[0], a[0]), pk2(a[1], a[1]), pk2(a[2], a[2]), pk2(a[3], a[3])};
         const u64 b2[2] = {Bv.x, Bv.y};
         u64 dd[4][2], xx[4][2], uu[4][2];
-        float umax = 0.f;
 #pragma unroll
         for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -227,11 +238,6 @@ __device__ __forceinline__ void jsd_chunk(const ulonglong2* __restrict__ sA, con
                 upk2(sm, s0, s1);
                 xx[i][j] = mul2(dd[i][j], pk2(rcp_approx(s0), rcp_approx(s1)));
                 uu[i][j] = mul2(xx[i][j], xx[i][j]);
-                if (V == 2) {
-                    float u0, u1;
-                    upk2(uu[i][j], u0, u1);
-                    umax = fmaxf(umax, fmaxf(u0, u1));
-                }
             }
         u64 G[4][2];
 #define JSD_HORNER_FIRST(ga, gb)                  \
@@ -260,7 +266,16 @@ __device__ __forceinline__ void jsd_chunk(const ulonglong2* __restrict__ sA, con
 #pragma unroll
             for (int j = 0; j < 2; ++j) c2[i][j] = fma2(mul2(dd[i][j], xx[i][j]), G[i][j], c2[i][j]);
 
-        if (V == 2) {
+        if (V == 2 && ((p2dims >> d) & 1u)) {
+            float umax = 0.f;
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    float u0, u1;
+                    upk2(uu[i][j], u0, u1);
+                    umax = fmaxf(umax, fmaxf(u0, u1));
+                }
             // largest u of the warp's 512 terms in this dimension (u >= 0: bit order = value order)
             const unsigned umax_w = __reduce_max_sync(0xFFFFFFFFu, __float_as_uint(umax));
             if (umax_w > JSD_P2_BITS) {
@@ -268,11 +283,7 @@ __device__ __forceinline__ void jsd_chunk(const ulonglong2* __restrict__ sA, con
                 // value s * fB(min(a,b)/s) and add (that - series value) where u > 1/2, 0 elsewhere.
                 // Typically a few of the 8 pairs are concerned (one outlier profile of the tile); sparse
                 // profiles flag all of them.
-                float a[4], b[4], dummy;
-                upk2(a2[0], a[0], dummy);
-                upk2(a2[1], a[1], dummy);
-                upk2(a2[2], a[2], dummy);
-                upk2(a2[3], a[3], dummy);
+                float b[4];
                 upk2(b2[0], b[0], b[1]);
                 upk2(b2[1], b[2], b[3]);
                 const u64 e4 = pk2(2.100300184e-01f, 2.100300184e-01f), e3 = pk2(3.274813073e-01f, 3.274813073e-01f);
@@ -328,8 +339,8 @@ __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdP
     const int tid = threadIdx.x;
     const int tx = tid & 15, ty = tid >> 4;
     const int nchunks = p.nchunks;
-    const float* gA = p.A + (size_t)(row_base / JT_M) * nchunks * JBLOCK_FLOATS;
-    const float* gB = p.B + (size_t)(col_base / JT_N) * nchunks * JBLOCK_FLOATS;
+    const float* gA = p.A + (size_t)(row_base / JT_M) * nchunks * JA_FLOATS;
+    const float* gB = p.B + (size_t)(col_base / JT_N) * nchunks * JB_FLOATS;
     const unsigned smem0 = smem_u32(jsmem);
     const unsigned bar0 = smem_u32(bars);
 
@@ -347,51 +358,64 @@ __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdP
         const unsigned bar = bar0 + 8 * s;
         const unsigned dst = smem0 + s * JSTAGE_BYTES;
         mbar_expect_tx(bar, JSTAGE_BYTES);
-        bulk_g2s(dst, gA + (size_t)chunk * JBLOCK_FLOATS, JBLOCK_FLOATS * 4, bar);
-        bulk_g2s(dst + JBLOCK_FLOATS * 4, gB + (size_t)chunk * JBLOCK_FLOATS, JBLOCK_FLOATS * 4, bar);
+        bulk_g2s(dst, gA + (size_t)chunk * JA_FLOATS, JA_FLOATS * 4, bar);
+        bulk_g2s(dst + JA_FLOATS * 4, gB + (size_t)chunk * JB_FLOATS, JB_FLOATS * 4, bar);
     };
     if (tid == 0) {
         for (int c = 0; c < JSTAGES && c < nchunks; ++c) issue(c);
     }
 
-    // variant of a chunk from the value ranges of the two 64-profile groups: one dimension per lane
+    // variant of a chunk from the value ranges of the two 64-profile groups: one dimension per lane.
+    // Bit 2 of a lane's code flags the dimensions in which this warp may meet u > 1/2: the range of the
+    // warp's own 8 rows (read from the A block in global memory) against the column group's range.  Where
+    // it is clear, phase 2 cannot run, so V2 skips tracking u there; the results do not change.
+    const float* rW = gA + (tid & 31) * JT_M + 8 * (tid >> 5);
     const float* rI_min = p.gmin + (size_t)(row_base / 64) * nchunks * JDK + (tid & 31);
     const float* rI_max = p.gmax + (size_t)(row_base / 64) * nchunks * JDK + (tid & 31);
     const float* rJ_min = p.gmin + (size_t)(col_base / 64) * nchunks * JDK + (tid & 31);
     const float* rJ_max = p.gmax + (size_t)(col_base / 64) * nchunks * JDK + (tid & 31);
     auto lane_code = [&](int ch) -> unsigned {
 #ifdef JSD_FORCE_VARIANT
-        return JSD_FORCE_VARIANT;
+        return JSD_FORCE_VARIANT | 4u;  // every dimension flagged
 #else
         const float ilo = rI_min[ch * JDK], ihi = rI_max[ch * JDK], jlo = rJ_min[ch * JDK], jhi = rJ_max[ch * JDK];
+        const float4 w0 = *reinterpret_cast<const float4*>(rW + (size_t)ch * JA_FLOATS);
+        const float4 w1 = *reinterpret_cast<const float4*>(rW + (size_t)ch * JA_FLOATS + 4);
+        const float wlo = fminf(fminf(fminf(w0.x, w0.y), fminf(w0.z, w0.w)), fminf(fminf(w1.x, w1.y), fminf(w1.z, w1.w)));
+        const float whi = fmaxf(fmaxf(fmaxf(w0.x, w0.y), fmaxf(w0.z, w0.w)), fmaxf(fmaxf(w1.x, w1.y), fmaxf(w1.z, w1.w)));
+        const unsigned flag = (whi <= JSD_RATIO_V1 * jlo && jhi <= JSD_RATIO_V1 * wlo) ? 0u : 4u;
         // a in [ilo, ihi], b in [jlo, jhi]: max(a/b, b/a) <= max(ihi/jlo, jhi/ilo)
-        if (ihi <= JSD_RATIO_V0 * jlo && jhi <= JSD_RATIO_V0 * ilo) return 0u;
-        if (ihi <= JSD_RATIO_V1 * jlo && jhi <= JSD_RATIO_V1 * ilo) return 1u;
-        return 2u;
+        if (ihi <= JSD_RATIO_V0 * jlo && jhi <= JSD_RATIO_V0 * ilo) return flag;
+        if (ihi <= JSD_RATIO_V1 * jlo && jhi <= JSD_RATIO_V1 * ilo) return flag | 1u;
+        return flag | 2u;
 #endif
     };
     unsigned code_next = lane_code(0);
 
+    // The float64 totals are touched once per chunk: they live in shared memory behind the ring
+    // ([16][JTHREADS], conflict-free), which leaves the registers to the chunk loops and keeps them
+    // free of spills at JSD_CTAS CTAs per SM.
+    double* t = reinterpret_cast<double*>(jsmem + JSTAGES * JSTAGE_BYTES) + tid;
     u64 c2[4][2];
-    double t[4][4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         c2[i][0] = 0ull;
         c2[i][1] = 0ull;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) t[i][j] = 0.0;
+        for (int j = 0; j < 4; ++j) t[(4 * i + j) * JTHREADS] = 0.0;
     }
 
     for (int ch = 0; ch < nchunks; ++ch) {
         const int s = ch % JSTAGES;
-        const unsigned variant = __reduce_max_sync(0xFFFFFFFFu, code_next);
+        const unsigned variant = __reduce_max_sync(0xFFFFFFFFu, code_next & 3u);
+        const unsigned p2dims = __ballot_sync(0xFFFFFFFFu, (code_next & 4u) != 0u);  // lane = dimension of the chunk
         if (ch + 1 < nchunks) code_next = lane_code(ch + 1);  // in flight during this chunk's loop
         mbar_wait(bar0 + 8 * s, (unsigned)((ch / JSTAGES) & 1));
-        const ulonglong2* sA = reinterpret_cast<const ulonglong2*>(jsmem + s * JSTAGE_BYTES) + 2 * ty;
-        const ulonglong2* sB = reinterpret_cast<const ulonglong2*>(jsmem + s * JSTAGE_BYTES + JBLOCK_FLOATS * 4) + tx;
-        if (variant == 0u) jsd_chunk<0>(sA, sB, c2);
-        else if (variant == 1u) jsd_chunk<1>(sA, sB, c2);
-        else jsd_chunk<2>(sA, sB, c2);
+        const float4* sA = reinterpret_cast<const float4*>(jsmem + s * JSTAGE_BYTES) + ty;
+        const ulonglong2* sB = reinterpret_cast<const ulonglong2*>(jsmem + s * JSTAGE_BYTES + JA_FLOATS * 4) + tx;
+        if (variant == 0u) jsd_chunk<0>(sA, sB, c2, 0u);
+        else if (variant == 1u) jsd_chunk<1>(sA, sB, c2, 0u);
+        else jsd_chunk<2>(sA, sB, c2, p2dims);
         // fold the chunk's float32 partial sums (32 non-negative terms each) into float64
 #pragma unroll
         for (int i = 0; i < 4; ++i)
@@ -399,8 +423,8 @@ __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdP
             for (int j = 0; j < 2; ++j) {
                 float c0, c1;
                 upk2(c2[i][j], c0, c1);
-                t[i][2 * j] += (double)c0;
-                t[i][2 * j + 1] += (double)c1;
+                t[(4 * i + 2 * j) * JTHREADS] += (double)c0;
+                t[(4 * i + 2 * j + 1) * JTHREADS] += (double)c1;
                 c2[i][j] = 0ull;
             }
         // Stage s is refilled by whichever warp finishes reading it last: no block-wide barrier in the
@@ -412,7 +436,7 @@ __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdP
             if (atomicAdd(&done_warps[s], 1u) % (JTHREADS / 32) == JTHREADS / 32 - 1) issue(ch + JSTAGES);
         }
     }
-    __syncthreads();  // the epilogue reuses the ring as the tile buffer
+    __syncthreads();  // the epilogue reuses the ring as the tile buffer (the totals lie behind it)
 
     // ---- epilogue: stage the tile in shared memory, then coalesced stores (and the mirror) ----
     constexpr int TP = JT_N + 1;
@@ -420,7 +444,7 @@ __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdP
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) tile[(4 * ty + i) * TP + 4 * tx + j] = (OUT_T)(0.25 * t[i][j]);
+        for (int j = 0; j < 4; ++j) tile[(4 * ty + i) * TP + 4 * tx + j] = (OUT_T)(0.25 * t[(4 * i + j) * JTHREADS]);
     __syncthreads();
     OUT_T* out = reinterpret_cast<OUT_T*>(p.out);
     const int r_lo = (int)max((int64_t)0, p.row0 - row_base), r_hi = (int)min((int64_t)JT_M, p.row1 - row_base);
@@ -448,7 +472,7 @@ int launch_jsd(const void* d_P, int64_t n, int64_t dim, int64_t row0, int64_t ro
     JsdParams p;
     p.B = reinterpret_cast<const float*>(d_P);
     p.A = p.B + npad * ldp;
-    p.gmin = p.A + 2 * npad * ldp;
+    p.gmin = p.A + npad * ldp;
     p.gmax = p.gmin + (npad / 64) * ldp;
     p.nchunks = (int)(ldp / JDK);
     p.n = n;
@@ -465,7 +489,7 @@ int launch_jsd(const void* d_P, int64_t n, int64_t dim, int64_t row0, int64_t ro
     }
     p.tiles_r = tr;
     p.tiles_c = tc;
-    const size_t smem = (size_t)JSTAGES * JSTAGE_BYTES;
+    const size_t smem = (size_t)JSTAGES * JSTAGE_BYTES + JT_TOTALS_BYTES;
     dim3 grid((unsigned)(tr * tc), 1, 1);
     LaunchTimer tm(1, stream);
     // the opt-in is per device: set it on every launch (a process may drive several GPUs)

@@ -7,7 +7,7 @@
 //                change a term by < 1e-27 relative.  Stored "blocked" for the bulk
 //                copies of po_jsd.cu: [n/64][dim/32] blocks of [32 dims][64 profiles]
 //                (column operand) followed by [n/32][dim/32] blocks of
-//                [32 dims][32 profiles][2] with every value twice (row operand).
+//                [32 dims][32 profiles] (row operand).
 //   BC         : the same copy; aux = sum of the row (the sum|a+b| denominator of
 //                scipy's braycurtis splits into row sums for non-negative profiles;
 //                a negative entry poisons aux with NaN so the result is loudly NaN).
@@ -45,10 +45,10 @@ int64_t prepared_row_elems(int metric, int64_t dim) {
 int64_t prepared_bytes(int metric, int64_t n, int64_t dim) {
     const int64_t ldp = prepared_row_elems(metric, dim);
     if (metric == PO_JSD) {
-        // blocked B + doubled A (rows padded to 64), the per-group value ranges, the dimension permutation
+        // blocked B + blocked A (rows padded to 64), the per-group value ranges, the dimension permutation
         // and the scratch of its computation (per-slice column minima / maxima, spreads)
         const int64_t npad = (n + 63) / 64 * 64;
-        return 3 * npad * ldp * 4 + 2 * (npad / 64) * ldp * 4 + ldp * 4 + (2 * JSD_MINMAX_SLICES + 1) * ldp * 4;
+        return 2 * npad * ldp * 4 + 2 * (npad / 64) * ldp * 4 + ldp * 4 + (2 * JSD_MINMAX_SLICES + 1) * ldp * 4;
     }
     if (eucl_use_gram(metric, dim)) return gram_prepared_bytes(n, dim);
     if (sc_use_gram(metric, dim)) return sc_gram_prepared_bytes(n, dim);
@@ -170,13 +170,10 @@ __global__ void __launch_bounds__(256) prepare_jsd_kernel(const void* __restrict
     __syncthreads();
     float* blkB = PB + ((size_t)grp * nchunks + kc) * 2048;
     for (int q = threadIdx.x; q < 2048; q += 256) blkB[q] = tile[q & 63][q >> 6];  // [d][c]
-    // two row-operand blocks (profiles 0..31 and 32..63 of the group): [d][r][2]
+    // two row-operand blocks (profiles 0..31 and 32..63 of the group): [d][r]
     for (int h = 0; h < 2; ++h) {
-        float2* blkA = reinterpret_cast<float2*>(PA + ((size_t)(grp * 2 + h) * nchunks + kc) * 2048);
-        for (int q = threadIdx.x; q < 1024; q += 256) {
-            const float v = tile[h * 32 + (q & 31)][q >> 5];
-            blkA[q] = make_float2(v, v);
-        }
+        float* blkA = PA + ((size_t)(grp * 2 + h) * nchunks + kc) * 1024;
+        for (int q = threadIdx.x; q < 1024; q += 256) blkA[q] = tile[h * 32 + (q & 31)][q >> 5];
     }
     if (w == 0) {
         float lo = __int_as_float(0x7F800000), hi = 0.f;
@@ -297,7 +294,7 @@ static int launch_prepare_t(int metric, const void* d_X, int64_t n, int64_t dim,
             const int64_t npad = (n + 63) / 64 * 64;
             float* PB = (float*)d_P;
             float* PA = PB + npad * ldp;
-            float* gmin = PA + 2 * npad * ldp;
+            float* gmin = PA + npad * ldp;
             float* gmax = gmin + (npad / 64) * ldp;
             int* perm = reinterpret_cast<int*>(gmax + (npad / 64) * ldp);
             float* pmin = reinterpret_cast<float*>(perm + ldp);
