@@ -441,13 +441,37 @@ int po_linkage_run(const void* d_D, int64_t ld, int dtype, int64_t n, int method
                    int64_t* d_zy, double* d_zh, int64_t* h_phases, po_stream_t stream);
 int po_linkage_tree(int64_t n, const int64_t* zx, const int64_t* zy, const double* zh, double* Z);
 
+/*
+ * Neighbour-joining trees of the resident matrix: the NJ and BIONJ trees phyloselect.R builds with ape's nj / bionj
+ * (:22-35), bit for bit in the order of float64 operations DESIGN.md section 4.11 fixes (agreement with ape itself
+ * is not pinned).
+ * method: 0 NJ, 1 BIONJ.
+ *   po_nj_capacity     C, the slots per side of the working state for n points (n plus a front headroom, rounded up
+ *                      to 32)
+ *   po_nj_workspace    bytes of d_work po_nj_run needs for n points
+ *   po_nj_stage_bytes  bytes of d_stage po_nj_run needs for n points (the compaction's staging rows, <= 256 MB)
+ *   po_nj_run          n - 3 joins, each four launches on `stream` (row sums, Q scan, decision, update) with no host
+ *                      synchronisation in between, then the three root edges.  d_W is the float64 C x C working state
+ *                      (8 C^2 bytes) that this call fills from d_D: D above the diagonal, BIONJ's variance below it.
+ *                      Writes d_edge (int64, (2n - 3) x 2, (parent, child)) and d_length (float64, 2n - 3) in ape's
+ *                      numbering from 0 (leaves 0 .. n-1, root n, the node of join t 2n - 3 - t), the rows in join
+ *                      order, and *h_compactions = how often the live block was packed.  d_D is read only; it must be
+ *                      finite and symmetric (po_hdbscan_check).  Fails with PO_ERR_ARG when a join finds no pair whose
+ *                      Q is below 1e50.  Synchronises `stream`.
+ */
+int64_t po_nj_capacity(int64_t n);
+int64_t po_nj_workspace(int64_t n);
+int64_t po_nj_stage_bytes(int64_t n);
+int po_nj_run(const void* d_D, int64_t ld, int dtype, int64_t n, int method, double* d_W, void* d_stage, void* d_work,
+              int64_t* d_edge, double* d_length, int64_t* h_compactions, po_stream_t stream);
+
 /* Number of kernels this library has launched since load (for bench.py's gpu_launches). */
 int64_t po_launch_count(void);
 
 /* Average device time (ms) of the launches of one kernel family since the last
  * po_timing_reset(): CUDA events recorded on the launching stream around each
  * launch while timing is enabled.  family: 0 = profiling, 1 = distance tile, 2 = the linkage kernels'
- * cooperative launch (po_linkage_run). */
+ * cooperative launch (po_linkage_run), 3 = the launches of one po_nj_run, first to last. */
 int po_timing_enable(int on);
 int po_timing_reset(void);
 int po_timing_read(int family, double* total_ms, int64_t* launches);

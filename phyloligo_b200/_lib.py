@@ -34,6 +34,7 @@ EXPORTED = [
     "po_hdbscan_check", "po_matrix_kth", "po_hdbscan_mst_workspace", "po_hdbscan_mst_init", "po_hdbscan_mst_round", "po_hdbscan_tree",
     "po_tsne_check", "po_tsne_conditional", "po_tsne_sum", "po_tsne_workspace", "po_tsne_repulsion", "po_tsne_attraction_step",
     "po_linkage_workspace", "po_linkage_run", "po_linkage_tree",
+    "po_nj_capacity", "po_nj_workspace", "po_nj_stage_bytes", "po_nj_run",
     "po_launch_count", "po_timing_enable", "po_timing_reset", "po_timing_read", "po_microbench",
 ]
 
@@ -159,6 +160,11 @@ def load():
     lib.po_linkage_run.restype = i32
     lib.po_linkage_tree.argtypes = [i64, vp, vp, vp, vp]
     lib.po_linkage_tree.restype = i32
+    for name in ("po_nj_capacity", "po_nj_workspace", "po_nj_stage_bytes"):
+        getattr(lib, name).argtypes = [i64]
+        getattr(lib, name).restype = i64
+    lib.po_nj_run.argtypes = [vp, i64, i32, i64, i32, vp, vp, vp, vp, vp, C.POINTER(i64), vp]
+    lib.po_nj_run.restype = i32
     lib.po_launch_count.restype = i64
     lib.po_timing_enable.argtypes = [i32]
     lib.po_timing_enable.restype = i32

@@ -16,7 +16,7 @@ struct FamilyTiming {
     double total_ms = 0.0;
     long long launches = 0;
 };
-static FamilyTiming g_fam[3];
+static FamilyTiming g_fam[4];
 
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -28,7 +28,7 @@ void set_error(const char* fmt, ...) {
 void count_launch(int) { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
 LaunchTimer::LaunchTimer(int fam, cudaStream_t s) : stream(s), family(fam), active(false) {
-    if (g_timing.load(std::memory_order_relaxed) && fam >= 0 && fam < 3) {
+    if (g_timing.load(std::memory_order_relaxed) && fam >= 0 && fam < 4) {
         if (cudaEventCreate(&e0) == cudaSuccess && cudaEventCreate(&e1) == cudaSuccess) {
             cudaEventRecord(e0, stream);
             active = true;
@@ -374,7 +374,7 @@ int po_timing_reset(void) {
 }
 
 int po_timing_read(int family, double* total_ms, int64_t* launches) {
-    if (family < 0 || family >= 3) {
+    if (family < 0 || family >= 4) {
         set_error("bad timing family %d", family);
         return PO_ERR_ARG;
     }

@@ -12,10 +12,12 @@ mutual-reachability MST, condensed tree, excess-of-mass selection), with MST tie
 index.  ``TSNE`` computes what the reference gets from sklearn.manifold.TSNE(metric="precomputed") (:381-398)
 with angle=0.0, i.e. the exact gradient; ``--tsne-out`` writes its embedding.  ``linkage`` / ``HClust`` build the
 tree bin/phyloselect.R:22-35 builds with hclust, as scipy.cluster.hierarchy.linkage computes it; ``-m hclust`` cuts
-it and ``--tree-out`` writes it in Newick format.  Plotting and the interactive loop are out of scope.
+it and ``--tree-out`` writes it in Newick format.  ``nj`` builds the neighbour-joining trees the same script offers
+(ape's nj and bionj, in the operation order DESIGN.md section 4.11 fixes); ``--tree-method nj|bionj`` makes ``--tree-out`` write one.
+Plotting and the interactive loop are out of scope.
 
-There is no CPU fallback: the sums, assignments, selections, the MST, the t-SNE gradient and the linkage loop run
-in libphyloligo_b200.so.
+There is no CPU fallback: the sums, assignments, selections, the MST, the t-SNE gradient, the linkage loop and the
+neighbour joins run in libphyloligo_b200.so.
 """
 from __future__ import annotations
 
@@ -680,6 +682,111 @@ class HClust:
         return self.fit(X).labels_
 
 
+NJ_METHODS = {"nj": 0, "bionj": 1}
+
+
+def _check_nj_method(method):
+    if method not in NJ_METHODS:
+        raise ValueError("method must be one of {}, got {!r}".format(list(NJ_METHODS), method))
+
+
+def nj_bytes(n, method="nj"):
+    """Device bytes nj(D, method) allocates for n rows besides D: the float64 C x C working state (C = n plus a front
+    headroom of new-node slots, po_nj_capacity; BIONJ keeps its variance in the same array, below the diagonal), the
+    compaction's staging rows, the workspace and the edges."""
+    _check_nj_method(method)
+    lib = _lib.load()
+    c = int(lib.po_nj_capacity(n))
+    return 8 * c * c + int(lib.po_nj_stage_bytes(n)) + int(lib.po_nj_workspace(n)) + 24 * (2 * n - 3)
+
+
+def check_nj_fits(n, method, free_bytes):
+    """Refuse (PhyloligoError) a tree of n rows whose device memory (nj_bytes) exceeds free_bytes."""
+    need = nj_bytes(n, method)
+    if need > free_bytes:
+        raise PhyloligoError("nj(method={!r}) of {} rows needs {} bytes of device memory (the float64 working state of "
+                             "the matrix, the staging rows and the workspace), {} are free".format(method, n, need, free_bytes))
+
+
+def nj_raw(D, method="nj"):
+    """nj on the device matrix D: device tensors (edge int64 (2n - 3, 2), length float64 (2n - 3,)) and the number
+    of compactions of the working state (po_nj_run).  D is checked (check_matrix) and not modified."""
+    _check_nj_method(method)
+    lib = _lib.load()
+    n = int(D.shape[0])
+    if n < 3:
+        raise ValueError("nj needs at least 3 observations, got {}".format(n))
+    check_matrix(D)
+    dev = D.device
+    free, _ = torch.cuda.mem_get_info(dev)
+    free += torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+    check_nj_fits(n, method, free)
+    c = int(lib.po_nj_capacity(n))
+    W = torch.empty((c, c), dtype=torch.float64, device=dev)
+    stage = torch.empty(int(lib.po_nj_stage_bytes(n)), dtype=torch.uint8, device=dev)
+    work = torch.empty(int(lib.po_nj_workspace(n)), dtype=torch.uint8, device=dev)
+    edge = torch.empty((2 * n - 3, 2), dtype=torch.int64, device=dev)
+    length = torch.empty(2 * n - 3, dtype=torch.float64, device=dev)
+    compactions = C.c_int64()
+    rc = lib.po_nj_run(_ptr(D), int(D.stride(0)), _dt(D), n, NJ_METHODS[method], _ptr(W), _ptr(stage), _ptr(work), _ptr(edge),
+                       _ptr(length), C.byref(compactions), _stream())
+    _lib.check(rc, "po_nj_run")
+    return edge, length, compactions.value
+
+
+def nj(D, method="nj"):
+    """Neighbour joining on the device: the unrooted tree phyloselect.R builds with ape's ``nj`` (method "nj") or
+    ``bionj`` ("bionj"), in the order of float64 operations DESIGN.md section 4.11 fixes, bit for bit.  Agreement with ape itself is
+    not pinned: ape's C source has not been available to compare against, and its bionj is Gascuel's own program,
+    whose pair order and tie tolerance are not restated.  D is an ndarray, a memmap or a device tensor, float32 or
+    float64 (float32 is widened exactly), used in place and not modified; it must be square, bitwise symmetric and
+    finite.  Returns (edge int64 (2n - 3, 2) of (parent, child), length float64 (2n - 3,)) in ape's numbering from
+    0: leaves 0 .. n-1, the root n, the node of join t (t = 0, 1, ...) 2n - 3 - t.  Rows are in join order, the
+    first-listed member first, then the three root edges in list order.  A working state (8 C^2 bytes, C slightly
+    above n) that does not fit in device memory is refused before anything is allocated."""
+    _check_nj_method(method)
+    D = as_device_matrix(D)
+    edge, length, _ = nj_raw(D, method)
+    return edge.cpu().numpy(), length.cpu().numpy()
+
+
+def write_nj_newick(edge, length, names, path):
+    """Write the tree of nj (edge, length) as an unrooted Newick tree with leaves names[0 .. n), shaped as ape's
+    write.tree writes it: a trifurcating root whose children are the root edges in order, every joined node's two
+    children in join order.  Lengths are repr(float), names go through newick_name.  The walk is iterative:
+    caterpillar trees are n deep."""
+    edge = np.asarray(edge, dtype=np.int64)
+    length = np.asarray(length, dtype=np.float64)
+    n = (len(edge) + 3) // 2
+    if edge.ndim != 2 or edge.shape != (2 * n - 3, 2) or length.shape != (2 * n - 3,) or n < 3 or len(names) != n:
+        raise ValueError("a ({0}, 2) edge matrix, {0} lengths and {1} names are expected, got {2}, {3} and {4} names".format(
+            2 * n - 3, n, edge.shape, length.shape, len(names)))
+    children = {}
+    for (parent, child), ln in zip(edge.tolist(), length.tolist()):
+        children.setdefault(parent, []).append((child, ln))
+    out = []
+    stack = [(n, "")]
+    while stack:
+        item = stack.pop()
+        if isinstance(item, str):
+            out.append(item)
+            continue
+        node, tail = item
+        if node < n:
+            out.append(newick_name(names[node]) + tail)
+            continue
+        out.append("(")
+        stack.append(")" + tail)
+        kids = children[node]
+        for i in range(len(kids) - 1, -1, -1):
+            child, ln = kids[i]
+            stack.append((child, ":" + repr(float(ln))))
+            if i:
+                stack.append(",")
+    with open(path, "w") as fh:
+        fh.write("".join(out) + ";\n")
+
+
 def newick_name(name):
     """A Newick leaf label: single-quoted, with every ' doubled, when it is empty or holds a blank or one of
     ( ) [ ] ' : ; ,"""
@@ -842,8 +949,11 @@ def get_cmd(argv=None):
     parser.add_argument("--linkage", action="store", dest="linkage", default="average", choices=list(LINKAGE_METHODS),
                         help="linkage of -m hclust and --tree-out (scipy.cluster.hierarchy.linkage's method)")
     parser.add_argument("--tree-out", action="store", dest="tree_out",
-                        help="write the hierarchical tree of the matrix (--linkage) to this file in Newick format; leaves "
+                        help="write the tree of the matrix (--tree-method) to this file in Newick format; leaves "
                              "are the FASTA record ids with -f or --assembly, row indices otherwise")
+    parser.add_argument("--tree-method", action="store", dest="tree_method", default="hclust", choices=["hclust"] + list(NJ_METHODS),
+                        help="the tree --tree-out writes: the hierarchical tree (hclust, --linkage, rooted) or the "
+                             "neighbour-joining tree (nj, bionj: ape's nj / bionj as phyloselect.R offers them, unrooted)")
     parser.add_argument("-f", action="store", dest="fastafile",
                         help="Path of the original fasta file used for the computation of the distance matrix")
     parser.add_argument("--large", action="store", choices=["memmap", "h5py"], dest="large", default=False,
@@ -907,7 +1017,15 @@ def main(argv=None):
     if params.tsne_out:
         print("Store t-SNE embedding in {}".format(params.tsne_out))
         np.savetxt(params.tsne_out, TSNE(perplexity=params.perplexity, random_state=0).fit(matrix).embedding_, delimiter="\t")
-    if params.tree_out:
+    if params.tree_out and params.tree_method != "hclust":
+        print("Store the {} tree in {}".format(params.tree_method, params.tree_out))
+        edge, length = nj(matrix, params.tree_method)
+        n = (len(edge) + 3) // 2
+        names = fasta_record_ids(params.fastafile) if params.fastafile else [str(i) for i in range(n)]
+        if len(names) != n:
+            raise PhyloligoError("{} holds {} records, the matrix {} rows".format(params.fastafile, len(names), n))
+        write_nj_newick(edge, length, names, params.tree_out)
+    elif params.tree_out:
         print("Store the {} linkage tree in {}".format(params.linkage, params.tree_out))
         if Z is None:
             Z = linkage(matrix, params.linkage)
