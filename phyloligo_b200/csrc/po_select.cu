@@ -64,7 +64,8 @@ __global__ void __launch_bounds__(256) rowsums_kernel(const void* __restrict__ D
     }
 }
 
-// out[j] = index c (0 .. k-1) of the smallest D[rows[c], j]; the first one on ties, as np.argmin.
+// out[j] = index c (0 .. k-1) of the smallest D[rows[c], j] as np.argmin picks it: the first NaN when there is
+// one (whatever its sign), else the first of the smallest values (-0.0 == +0.0).
 template <typename T>
 __global__ void __launch_bounds__(256) argmin_rows_kernel(const void* __restrict__ D, int64_t ld, const int64_t* __restrict__ rows,
                                                           int k, int64_t ncols, int* __restrict__ out) {
@@ -72,9 +73,9 @@ __global__ void __launch_bounds__(256) argmin_rows_kernel(const void* __restrict
     if (j >= ncols) return;
     double best = ld_entry<T>(D, rows[0] * ld + j);
     int arg = 0;
-    for (int c = 1; c < k; ++c) {
+    for (int c = 1; c < k && best == best; ++c) {
         const double v = ld_entry<T>(D, rows[c] * ld + j);
-        if (v < best) {
+        if (v < best || v != v) {
             best = v;
             arg = c;
         }
@@ -82,13 +83,17 @@ __global__ void __launch_bounds__(256) argmin_rows_kernel(const void* __restrict
     out[j] = arg;
 }
 
-// order-preserving map of a double onto an unsigned 64-bit key
+// order-preserving map of a double onto an unsigned 64-bit key; -0.0 takes the key of +0.0 (they compare equal)
 __device__ __forceinline__ unsigned long long dkey(double v) {
-    const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+    unsigned long long b = (unsigned long long)__double_as_longlong(v);
+    if (b == 0x8000000000000000ull) b = 0ull;
     return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
+// np.argmin's order of the costs: a NaN of either sign comes first, then the values ascending
+__device__ __forceinline__ unsigned long long argmin_key(double v) { return (v != v) ? 0ull : dkey(v); }
 
-// per cluster: members, smallest cost among the members and the first member that has it
+// per cluster: members, smallest cost among the members and the first member that has it (np.argmin: the first
+// NaN cost when there is one)
 __global__ void __launch_bounds__(256) cluster_min_kernel(const double* __restrict__ cost, const int* __restrict__ labels, int64_t n,
                                                           int k, unsigned long long* __restrict__ min_key,
                                                           long long* __restrict__ count) {
@@ -96,7 +101,7 @@ __global__ void __launch_bounds__(256) cluster_min_kernel(const double* __restri
     if (i >= n) return;
     const int c = labels[i];
     if (c < 0 || c >= k) return;
-    atomicMin(&min_key[c], dkey(cost[i]));
+    atomicMin(&min_key[c], argmin_key(cost[i]));
     atomicAdd(reinterpret_cast<unsigned long long*>(&count[c]), 1ull);
 }
 __global__ void __launch_bounds__(256) cluster_argmin_kernel(const double* __restrict__ cost, const int* __restrict__ labels, int64_t n,
@@ -106,7 +111,7 @@ __global__ void __launch_bounds__(256) cluster_argmin_kernel(const double* __res
     if (i >= n) return;
     const int c = labels[i];
     if (c < 0 || c >= k) return;
-    if (dkey(cost[i]) == min_key[c]) atomicMin(&arg[c], (long long)i);
+    if (argmin_key(cost[i]) == min_key[c]) atomicMin(&arg[c], (long long)i);
 }
 __global__ void cluster_init_kernel(unsigned long long* min_key, long long* arg, long long* count, int k) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -127,7 +132,7 @@ __global__ void cluster_finish_kernel(const unsigned long long* min_key, const l
 }
 
 // k nearest neighbours of every row, the row's own column excluded: ascending distance, ties by
-// column index.  One CTA per row.
+// column index, -0.0 equal to +0.0, NaN (either sign) last.  One CTA per row.  Float32 rows:
 // Fast path (one pass over the row, HBM bound): 8192 entries of the row -- 64 evenly spaced runs of 128
 // consecutive columns, or the whole row when it is that short -- are loaded into shared memory and a radix
 // select over them gives a threshold at about twice the sample rank that corresponds to k; one pass over
@@ -139,15 +144,34 @@ __global__ void cluster_finish_kernel(const unsigned long long* min_key, const l
 // entries (four 8-bit passes, each a shared-memory histogram of the still undecided prefix class) finds
 // the key of the k-th smallest entry; everything strictly below it, then the first ties in column
 // order, are gathered and sorted in shared memory (bitonic, keys = (distance key, column)).
+// Float64 rows take the exact path only, over the entries' full-width 64-bit keys (eight histogram passes):
+// float64 distances that round to one float32 are ordered by value, not as ties.  Such matrices come from
+// text files and are small; the float32 path is what the resident matrix of the distance stage takes.
 constexpr int KNN_THREADS = 256;
 constexpr int KNN_MAX_K = 1024;
 constexpr int KNN_CAP = 4096;     // candidates the fast path can hold (32 KB of shared memory)
 constexpr int KNN_SAMPLE = 8192;  // entries of the row sampled for the fast path's threshold
 
+// order-preserving map of a float onto an unsigned 32-bit key; -0.0 takes the key of +0.0
 __device__ __forceinline__ unsigned fkey(float v) {
-    const unsigned b = __float_as_uint(v);
+    unsigned b = __float_as_uint(v);
+    if (b == 0x80000000u) b = 0u;
     return (b >> 31) ? ~b : (b | 0x80000000u);
 }
+// the keys the selections rank by: NaN (either sign) last
+__device__ __forceinline__ unsigned okey(float v) { return (v != v) ? 0xFFFFFFFFu : fkey(v); }
+__device__ __forceinline__ unsigned long long okey(double v) { return (v != v) ? ~0ull : dkey(v); }
+
+// an item of the exact path's sort, ordered by (key, column): one word for a 32-bit key, a pair for a 64-bit one
+__device__ __forceinline__ unsigned long long knn_item(unsigned key, int64_t j) { return ((unsigned long long)key << 32) | (unsigned)j; }
+__device__ __forceinline__ unsigned knn_col(unsigned long long it) { return (unsigned)(it & 0xFFFFFFFFull); }
+struct KnnItem64 {
+    unsigned long long key, col;
+};
+__device__ __forceinline__ KnnItem64 knn_item(unsigned long long key, int64_t j) { return {key, (unsigned long long)(unsigned)j}; }
+__device__ __forceinline__ unsigned knn_col(KnnItem64 it) { return (unsigned)it.col; }
+__device__ __forceinline__ bool operator>(KnnItem64 a, KnnItem64 b) { return a.key != b.key ? a.key > b.key : a.col > b.col; }
+__device__ __forceinline__ bool operator==(KnnItem64 a, KnnItem64 b) { return a.key == b.key && a.col == b.col; }
 
 // Radix select over order-preserving keys K (32 bits for float entries, 64 for double), 8 bits per pass from
 // the top, each pass a shared-memory histogram of the still undecided prefix class: the key of the
@@ -204,20 +228,16 @@ __device__ __forceinline__ K radix_select(KeyOf key_of, int64_t ncols, int64_t s
 template <typename T>
 __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict__ D, int64_t ld, int64_t ncols, int64_t self0, int k,
                                                           int kpad, int* __restrict__ out_idx, float* __restrict__ out_dist) {
-    extern __shared__ unsigned long long knn_items[];  // kpad (distance key << 32 | column)
+    extern __shared__ unsigned long long knn_items[];  // fast path: candidates (distance key << 32 | column)
     __shared__ unsigned hist[256];
     __shared__ unsigned s_prefix, s_mask, s_need, s_below, s_ties;
     const int64_t i = blockIdx.x;
     const T* row = reinterpret_cast<const T*>(D) + i * ld;
     const int64_t self = self0 + i;
     const int tid = threadIdx.x;
-    // NaN entries sort last (key 0xFFFFFFFF after the float map only for -NaN; force it)
-    auto key_of = [&](int64_t j) -> unsigned {
-        const float v = (float)row[j];
-        return (v != v) ? 0xFFFFFFFFu : fkey(v);
-    };
-    // ---------------- fast path ----------------
-    {
+    auto key_of = [&](int64_t j) { return okey(row[j]); };
+    // ---------------- fast path (float32) ----------------
+    if constexpr (sizeof(T) == 4) {
         unsigned* samp = reinterpret_cast<unsigned*>(knn_items);
         const int S = (int)min((int64_t)KNN_SAMPLE, ncols);
         const bool whole = (int64_t)S == ncols;
@@ -301,8 +321,7 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
                     bool takes[VEC], any = false;
 #pragma unroll
                     for (int c = 0; c < VEC; ++c) {
-                        const float x = (float)e[c];
-                        keys[c] = (x != x) ? 0xFFFFFFFFu : fkey(x);
+                        keys[c] = okey(e[c]);
                         takes[c] = v < nvec && keys[c] <= tau && v * VEC + c != self;
                         any |= takes[c];
                     }
@@ -358,25 +377,29 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
         __syncthreads();
     }
     // ---------------- exact path ----------------
+    using K = decltype(okey(T()));
+    using Item = decltype(knn_item(K(), 0));
+    Item* items = reinterpret_cast<Item*>(knn_items);  // kpad
+    const Item pad = knn_item(~K(0), 0xFFFFFFFFll);   // sorts after every entry, NaN included
     unsigned nties;  // how many entries equal to the k-th smallest belong to the k smallest
-    const unsigned kth = radix_select<unsigned>(key_of, ncols, self, (unsigned)k, hist, &nties);  // key of the k-th smallest
+    const K kth = radix_select<K>(key_of, ncols, self, (unsigned)k, hist, &nties);  // key of the k-th smallest
     if (tid == 0) {
         s_below = 0u;
         s_ties = 0u;
     }
-    for (int q = tid; q < kpad; q += KNN_THREADS) knn_items[q] = ~0ull;
+    for (int q = tid; q < kpad; q += KNN_THREADS) items[q] = pad;
     __syncthreads();
     // gather: entries below the threshold in any order (sorted afterwards); ties in column order, which a
     // strided sweep does not give -- so ties are taken by their rank among the ties (count of equal
     // entries at smaller columns), computed block by block of columns in order
     for (int64_t j0 = 0; j0 < ncols; j0 += KNN_THREADS) {
         const int64_t j = j0 + tid;
-        unsigned key = 0xFFFFFFFFu;
+        K key = ~K(0);
         bool valid = j < ncols && j != self;
         if (valid) key = key_of(j);
         const bool below = valid && key < kth;
         const bool tie = valid && key == kth;
-        if (below) knn_items[atomicAdd(&s_below, 1u)] = ((unsigned long long)key << 32) | (unsigned)j;
+        if (below) items[atomicAdd(&s_below, 1u)] = knn_item(key, j);
         // rank of this tie among the ties: ties in earlier blocks (s_ties) + ties at smaller columns in this block
         const unsigned tmask = __ballot_sync(0xFFFFFFFFu, tie);
         __shared__ unsigned warp_ties[KNN_THREADS / 32];
@@ -385,7 +408,7 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
         if (tie) {
             unsigned before = s_ties + __popc(tmask & ((1u << (tid & 31)) - 1u));
             for (int w = 0; w < (tid >> 5); ++w) before += warp_ties[w];
-            if (before < nties) knn_items[(unsigned)k - nties + before] = ((unsigned long long)key << 32) | (unsigned)j;
+            if (before < nties) items[(unsigned)k - nties + before] = knn_item(key, j);
         }
         __syncthreads();
         if (tid == 0) {
@@ -395,17 +418,17 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
         }
         __syncthreads();
     }
-    // bitonic sort of the kpad items (padding = ~0 sorts last); the ties already sit in column order at the end
+    // bitonic sort of the kpad items (padding sorts last); the ties already sit in column order at the end
     for (int size = 2; size <= kpad; size <<= 1) {
         for (int stride = size >> 1; stride > 0; stride >>= 1) {
             for (int q = tid; q < kpad; q += KNN_THREADS) {
                 const int partner = q ^ stride;
                 if (partner > q) {
                     const bool up = (q & size) == 0;
-                    const unsigned long long a = knn_items[q], b = knn_items[partner];
+                    const Item a = items[q], b = items[partner];
                     if ((a > b) == up) {
-                        knn_items[q] = b;
-                        knn_items[partner] = a;
+                        items[q] = b;
+                        items[partner] = a;
                     }
                 }
             }
@@ -413,10 +436,10 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
         }
     }
     for (int q = tid; q < k; q += KNN_THREADS) {
-        const unsigned long long it = knn_items[q];
-        const int col = (int)(unsigned)(it & 0xFFFFFFFFull);
-        out_idx[i * k + q] = (it == ~0ull) ? -1 : col;
-        out_dist[i * k + q] = (it == ~0ull) ? __int_as_float(0x7FC00000) : (float)row[col];
+        const Item it = items[q];
+        const int col = (int)knn_col(it);
+        out_idx[i * k + q] = (it == pad) ? -1 : col;
+        out_dist[i * k + q] = (it == pad) ? __int_as_float(0x7FC00000) : (float)row[col];
     }
 }
 
@@ -424,9 +447,7 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const void* __restrict
 // The k-th smallest entry (1-based, every column counted, the diagonal too) of every row, returned bit for
 // bit in the matrix's dtype: the exact radix select of knn_kernel over the full-width key of the entry
 // (4 passes for float, 8 for double), so that no two float64 entries that round to one float32 are
-// confused.  NaN entries sort last.  One CTA per row.
-__device__ __forceinline__ unsigned okey(float v) { return (v != v) ? 0xFFFFFFFFu : fkey(v); }
-__device__ __forceinline__ unsigned long long okey(double v) { return (v != v) ? ~0ull : dkey(v); }
+// confused.  NaN entries sort last; -0.0 equals +0.0 and comes back as +0.0.  One CTA per row.
 __device__ __forceinline__ float from_okey(unsigned k) { return __uint_as_float((k >> 31) ? (k & 0x7FFFFFFFu) : ~k); }
 __device__ __forceinline__ double from_okey(unsigned long long k) {
     return __longlong_as_double((long long)((k >> 63) ? (k & 0x7FFFFFFFFFFFFFFFull) : ~k));
@@ -449,7 +470,8 @@ extern "C" {
 
 int po_matrix_rowsums(const void* d_D, int64_t ld, int dtype, const int64_t* d_rows, int64_t n_rows, int64_t n_cols,
                       const int* d_labels, const int* d_row_labels, double* d_out, po_stream_t stream) {
-    if (!d_D || !d_out || n_rows < 0 || n_cols < 0 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64) ||
+    // a matrix without columns may have no storage: its sums are 0 and it is never read
+    if ((!d_D && n_cols > 0) || !d_out || n_rows < 0 || n_cols < 0 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64) ||
         ((d_labels == nullptr) != (d_row_labels == nullptr)) || n_rows > 0x7FFFFFFFll) {
         set_error("po_matrix_rowsums: bad arguments");
         return PO_ERR_ARG;
@@ -483,7 +505,8 @@ int po_matrix_argmin_rows(const void* d_D, int64_t ld, int dtype, const int64_t*
 
 int po_cluster_argmin(const double* d_cost, const int* d_labels, int64_t n, int k, void* d_work, int64_t* d_best_idx,
                       double* d_best_cost, int64_t* d_count, po_stream_t stream) {
-    if (!d_cost || !d_labels || !d_work || !d_best_idx || !d_best_cost || !d_count || n < 0 || k < 1) {
+    // no points (n = 0) may come with no storage: every cluster is then empty
+    if (((!d_cost || !d_labels) && n > 0) || !d_work || !d_best_idx || !d_best_cost || !d_count || n < 0 || k < 1) {
         set_error("po_cluster_argmin: bad arguments");
         return PO_ERR_ARG;
     }
@@ -516,7 +539,8 @@ int po_matrix_knn(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_
     if (n_rows == 0) return PO_OK;
     int kpad = 2;
     while (kpad < k) kpad <<= 1;
-    const size_t smem = (size_t)(kpad > KNN_CAP ? kpad : KNN_CAP) * 8;  // candidates of the fast path / items of the exact path
+    // float32: candidates of the fast path / items of the exact path; float64: the exact path's (key, column) pairs
+    const size_t smem = dtype == PO_F32 ? (size_t)(kpad > KNN_CAP ? kpad : KNN_CAP) * 8 : (size_t)kpad * sizeof(KnnItem64);
     if (dtype == PO_F32)
         knn_kernel<float><<<(unsigned)n_rows, KNN_THREADS, smem, (cudaStream_t)stream>>>(d_D, ld, n_cols, self0, k, kpad, d_idx, d_dist);
     else

@@ -470,7 +470,7 @@ int po_tsne_conditional(const void* d_D, int64_t ld, int dtype, int64_t n, const
 }
 
 int po_tsne_sum(const double* d_x, int64_t n, double* d_out, po_stream_t stream) {
-    if (!d_x || !d_out || n < 0) {
+    if ((!d_x && n > 0) || !d_out || n < 0) {  // an empty vector may have no storage
         set_error("po_tsne_sum: bad arguments");
         return PO_ERR_ARG;
     }

@@ -170,7 +170,11 @@ class KMedoids:
             rs = self.random_state if isinstance(self.random_state, np.random.RandomState) else np.random.RandomState(self.random_state)
             medoids = torch.from_numpy(np.asarray(rs.permutation(n)[:k], dtype=np.int64)).to(dev)
         else:
-            medoids = torch.argsort(row_sums(D), stable=True)[:k].contiguous()
+            # np.argsort's order: NaN sums last whatever their sign (torch's device sort puts a negative NaN first)
+            sums = row_sums(D)
+            nan = torch.isnan(sums)
+            medoids = torch.argsort(torch.where(nan, torch.inf, sums), stable=True)
+            medoids = medoids[torch.argsort(nan[medoids].to(torch.int8), stable=True)][:k].contiguous()
         cluster_ids = torch.arange(k, dtype=torch.int32, device=dev)
         old = None
         labels = None
