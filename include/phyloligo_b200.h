@@ -397,8 +397,8 @@ int po_hdbscan_tree(int64_t n, int64_t min_cluster_size, int64_t* u, int64_t* v,
  *   po_tsne_repulsion        the exact all-pairs pass over the positions d_Y (float32 [n x 2]): per row
  *                            sum_j q_ij^2 (y_i - y_j) and Z = sum_{i != j} q_ij, q_ij = 1 / (1 + |y_i - y_j|^2),
  *                            kept in d_work for the step
- *   po_tsne_attraction_step  per row the CSR walk sum_j p_ij q_ij (y_i - y_j), p_ij = float32((P_ij * mul) / div),
- *                            and the gradient 4 (attraction - repulsion / Z) of the positions the last
+ *   po_tsne_attraction_step  per row the CSR walk sum_j p_ij q_ij (y_i - y_j), p_ij = float32((P_ij * mul) * r),
+ *                            r = 1.0 / div (scipy's in-place P /= div multiplies by the reciprocal), and the gradient 4 (attraction - repulsion / Z) of the positions the last
  *                            po_tsne_repulsion saw.  d_grad (optional, float32 [n x 2]) receives it.  With d_Y_next
  *                            one _gradient_descent step: gains (+0.2 / x0.8, at least 0.01, float32), update =
  *                            momentum update - learning_rate grad gains (float64 when update64, else float32 as

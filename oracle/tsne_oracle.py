@@ -8,8 +8,10 @@ Barnes-Hut gradient is the exact gradient of the sparse-P objective, which is wh
   joint P       (C + C^T) / sum, pairs whose sum is 0 dropped (scipy's sparse addition)
   gradient      4 (sum_j p_ij q_ij (y_i - y_j) - sum_j q_ij^2 (y_i - y_j) / Z), p_ij read as float32, exact
                 over all pairs in row chunks (memory bounded)
-  optimiser     _gradient_descent as _tsne drives it: 250 iterations with P x early_exaggeration and momentum 0.5,
-                then momentum 0.8; gains +0.2 / x0.8 clipped at 0.01; a convergence check every 50 iterations
+  optimiser     _gradient_descent as _tsne drives it, with its dtypes: 250 iterations with P x early_exaggeration
+                and momentum 0.5, then momentum 0.8; gains +0.2 / x0.8 clipped at 0.01 in float32, positions
+                float32, the update float64 or float32 by the learning rate's type; a convergence check every 50
+                iterations
 """
 import numpy as np
 from scipy.sparse import csr_matrix
@@ -107,23 +109,25 @@ def random_init(n, random_state):
     return 1e-4 * rs.standard_normal(size=(n, 2)).astype(np.float32)
 
 
-def _descend(P, p, it, max_iter, momentum, lr, exaggeration, n_iter_without_progress, min_grad_norm, n_iter_check=50):
+def _descend(objective, p, it, max_iter, momentum, lr, n_iter_without_progress, min_grad_norm, n_iter_check=50):
+    """_gradient_descent with scikit-learn's dtypes: positions and gains float32 like p; the update float32 at
+    first, then float64 when lr is a numpy float64 scalar ("auto": np.maximum) and float32 when it is a Python
+    number; the gradient norm of the float32 gains x gradient.  objective(p, compute_error) -> (KL, float32 grad)."""
+    p = p.copy().ravel()
     update = np.zeros_like(p)
     gains = np.ones_like(p)
     error = best_error = np.finfo(float).max
     best_iter = i = it
     for i in range(it, max_iter):
         check = (i + 1) % n_iter_check == 0
-        grad, kl = gradient(P, p, exaggeration)
-        if check or i == max_iter - 1:
-            error = kl
+        error, grad = objective(p, check or i == max_iter - 1)
         inc = update * grad < 0.0
         gains[inc] += 0.2
         gains[~inc] *= 0.8
         np.clip(gains, 0.01, np.inf, out=gains)
         grad *= gains
         update = momentum * update - lr * grad
-        p = p + update
+        p += update
         if check:
             if error < best_error:
                 best_error, best_iter = error, i
@@ -134,14 +138,25 @@ def _descend(P, p, it, max_iter, momentum, lr, exaggeration, n_iter_without_prog
     return p, error, i
 
 
-def fit(D, perplexity=30.0, early_exaggeration=12.0, max_iter=1000, n_iter_without_progress=300, min_grad_norm=1e-7,
-        random_state=0, init=None):
-    """{"embedding", "kl_divergence", "n_iter", "learning_rate", "P"} of the whole fit."""
+def fit(D, perplexity=30.0, early_exaggeration=12.0, learning_rate="auto", max_iter=1000, n_iter_without_progress=300,
+        min_grad_norm=1e-7, random_state=0, init=None):
+    """{"embedding", "kl_divergence", "n_iter", "learning_rate", "P"} of the whole fit: TSNE._tsne's two stages,
+    each step with the exact gradient of gradient() read as float32.  As in _tsne, P is scaled in place by scipy:
+    P *= early_exaggeration for the first stage, then P /= early_exaggeration, which multiplies by
+    1.0 / early_exaggeration, so the second stage reads (P x ee) x (1 / ee), not always P's own bits."""
     n = np.asarray(D).shape[0]
     P = joint_probabilities(D, perplexity)
-    lr = np.maximum(n / early_exaggeration / 4, 50)
-    Y = (random_init(n, random_state) if init is None else np.asarray(init)).astype(np.float64)
-    Y, kl, it = _descend(P, Y, 0, 250, 0.5, lr, early_exaggeration, 250, min_grad_norm)
+    lr = np.maximum(n / early_exaggeration / 4, 50) if learning_rate == "auto" else learning_rate
+    Y = random_init(n, random_state) if init is None else np.asarray(init, dtype=np.float32)
+    Pe = P.copy()
+
+    def objective(p, compute_error):
+        g, kl = gradient(Pe, p.reshape(n, 2))
+        return (kl if compute_error else np.nan), g.astype(np.float32).ravel()
+
+    Pe *= early_exaggeration
+    Y, kl, it = _descend(objective, Y, 0, 250, 0.5, lr, 250, min_grad_norm)
+    Pe /= early_exaggeration
     if it < 250 or max_iter - 250 > 0:
-        Y, kl, it = _descend(P, Y, it + 1, max_iter, 0.8, lr, 1.0, n_iter_without_progress, min_grad_norm)
-    return {"embedding": Y, "kl_divergence": kl, "n_iter": it, "learning_rate": lr, "P": P}
+        Y, kl, it = _descend(objective, Y, it + 1, max_iter, 0.8, lr, n_iter_without_progress, min_grad_norm)
+    return {"embedding": Y.reshape(n, 2), "kl_divergence": kl, "n_iter": it, "learning_rate": lr, "P": P}

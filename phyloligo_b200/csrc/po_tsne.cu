@@ -316,8 +316,8 @@ __global__ void fold_kernel(int64_t n, int chunks, const double* __restrict__ px
 
 // ---------------------------------------------------------------------------------------------------
 // attraction + step, one warp per row: sum_j P_ij q_ij (y_i - y_j) over the row's CSR entries (P_ij read as
-// scikit-learn's float32 val_P of the float64 P scaled by mul / div: P * early_exaggeration in the first stage,
-// (P * ee) / ee in the second), the gradient 4 (attraction - repulsion / Z), optionally the row's KL terms, then
+// scikit-learn's float32 val_P of the float64 P scaled as _tsne scales it in place: P * early_exaggeration in the
+// first stage, then (P * ee) * (1 / ee) in the second, since scipy's P /= ee multiplies by the reciprocal), the gradient 4 (attraction - repulsion / Z), optionally the row's KL terms, then
 // _gradient_descent's gains / momentum / position update into the other position buffer.
 // ---------------------------------------------------------------------------------------------------
 constexpr int STEP_WARPS = 8;
@@ -326,7 +326,7 @@ struct StepArgs {
     const int64_t* indptr;
     const int* indices;
     const double* P;
-    double mul, div;
+    double mul, rdiv;  // rdiv = 1.0 / div, rounded once on the host as scipy's 1.0 / other
     const float2* Y;
     float2* Y_next;   // NULL: gradient only
     double* update;   // float64 (scikit-learn's update is float64 when the learning rate is a float64 scalar)
@@ -349,7 +349,7 @@ __global__ void __launch_bounds__(STEP_WARPS * 32) step_kernel(StepArgs a, int64
     const float tiny = 1.17549435e-38f;  // FLOAT32_TINY
     for (int64_t e = a.indptr[i] + lane; e < a.indptr[i + 1]; e += 32) {
         const int j = a.indices[e];
-        const float p = (float)((a.P[e] * a.mul) / a.div);
+        const float p = (float)((a.P[e] * a.mul) * a.rdiv);
         const float2 yj = a.Y[j];
         const float bx = __fsub_rn(yi.x, yj.x), by = __fsub_rn(yi.y, yj.y);
         const float d = __fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by));
@@ -511,7 +511,7 @@ int po_tsne_attraction_step(const int64_t* d_indptr, const int* d_indices, const
     a.indices = d_indices;
     a.P = d_P;
     a.mul = mul;
-    a.div = div;
+    a.rdiv = 1.0 / div;
     a.Y = reinterpret_cast<const float2*>(d_Y);
     a.Y_next = reinterpret_cast<float2*>(d_Y_next);
     a.update = d_update;

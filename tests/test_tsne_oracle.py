@@ -70,6 +70,45 @@ def test_full_fit_matches_scikit_learn(kind, n, seed):
     assert abs(t_sk - t_or) <= 0.005
 
 
+def sklearn_descent(monkeypatch, P, Y0, objective, **kwargs):
+    """(embedding, kl_divergence_, n_iter_) of scikit-learn's own TSNE._tsne from P (scaled in place, as fit does)
+    and Y0, with _kl_divergence_bh replaced by objective(P, params, compute_error) -> (KL, float32 grad)."""
+    sk = SkTSNE(metric="precomputed", init="random", angle=0.0, **kwargs)
+    n = Y0.shape[0]
+    sk.learning_rate_ = np.maximum(n / sk.early_exaggeration / 4, 50) if sk.learning_rate == "auto" else sk.learning_rate
+
+    def bh(params, P, dof, n_samples, n_components, compute_error=True, **_):
+        assert params.dtype == np.float32 and P.data.dtype == np.float64
+        return objective(P, params, compute_error)
+
+    monkeypatch.setattr(_t_sne, "_kl_divergence_bh", bh)
+    Y = sk._tsne(P.copy(), 1, n, X_embedded=Y0.copy())
+    return Y, sk.kl_divergence_, sk.n_iter_
+
+
+@pytest.mark.parametrize("kwargs", [{}, {"learning_rate": 200.0, "early_exaggeration": 7.0, "max_iter": 300},
+                                    {"min_grad_norm": 1e3, "max_iter": 400}, {"n_iter_without_progress": 0}],
+                         ids=["auto", "lr200-ee7", "min-grad-norm", "no-progress"])
+def test_oracle_descent_is_scikit_learns_bit_for_bit(monkeypatch, kwargs):
+    # scikit-learn's _gradient_descent, fed the oracle's gradient read as float32, against the oracle's own fit: the
+    # same float32 positions and gains, the same update dtype, the same stage-2 P and the same stopping iteration
+    D = jsd_matrix(120, 3)  # its KL stops improving in stage 2, so n_iter_without_progress=0 ends the fit early
+    Y0 = to.random_init(120, 3)
+    res = to.fit(D, perplexity=20.0, init=Y0, **kwargs)
+
+    def objective(P, params, compute_error):
+        g, kl = to.gradient(P, params.reshape(-1, 2))
+        return (kl if compute_error else np.nan), g.astype(np.float32).ravel()
+
+    Y, kl, n_iter = sklearn_descent(monkeypatch, res["P"], Y0, objective, perplexity=20.0, **kwargs)
+    assert Y.dtype == np.float32 and res["embedding"].dtype == np.float32
+    assert np.array_equal(Y, res["embedding"]) and kl == res["kl_divergence"] and n_iter == res["n_iter"]
+    if "min_grad_norm" in kwargs:
+        assert n_iter == 99  # both stages stop at their first check
+    if "n_iter_without_progress" in kwargs:
+        assert n_iter < 999
+
+
 def test_random_init_is_scikit_learns_draw():
     # TSNE(init="random") draws 1e-4 * standard_normal((n, 2)).astype(float32) from check_random_state(seed)
     from sklearn.utils import check_random_state
