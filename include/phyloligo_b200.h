@@ -56,6 +56,9 @@ enum po_dtype { PO_F32 = 0, PO_F64 = 1 };
 /* flags of po_distance_block */
 #define PO_FLAG_SKIP_LOWER 1u /* skip the kernel tiles that lie wholly below the diagonal       */
 #define PO_FLAG_MIRROR     2u /* tiles wholly above the diagonal are also written transposed  */
+#define PO_FLAG_MIRROR_ONLY 4u /* with PO_FLAG_MIRROR: store only the transposed tiles (into the mirror
+                                  buffer) and nothing into d_out -- the part of a row panel left of its
+                                  diagonal square, computed from the block rows above it */
 
 #define PO_MAX_PATTERN 32 /* longest spaced pattern (window width) */
 #define PO_MAX_K       10 /* most '1's in a pattern (4^10 bins)     */
@@ -350,18 +353,26 @@ int po_matrix_knn(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_
  * MST edges compare by the triple (mutual reachability, min(i, j), max(i, j)); the MST is then unique.
  *   po_hdbscan_check         refuses (PO_ERR_ARG) a matrix that is not square, not bitwise symmetric or holds a
  *                            NaN or an infinite entry; the message names the first offending entry in row-major
- *                            order.  d_work: 8 bytes.  Synchronises `stream`.
+ *                            order.  d_work: 8 bytes.  Synchronises `stream`.  With ld_cols = 0 (row0 = 0, d_cols
+ *                            NULL), d_D is the whole matrix.  With ld_cols > 0, d_D is the row panel [row0, row0 +
+ *                            n_rows) x [0, n_cols) of an n_cols x n_cols matrix, and entry (i, j) is compared with
+ *                            (j, i) taken from d_cols, the column strip [0, n_cols) x [row0, row0 + n_rows) with row
+ *                            pitch ld_cols; with d_cols NULL (a source symmetric by construction) only the panel's
+ *                            diagonal square is tested for symmetry.  Checked panel by panel in row order, the first
+ *                            panel that fails names the entry the whole-matrix check names.
  *   po_matrix_kth            d_out[i] = the k-th smallest (1-based) entry of row i, every column counted (the
  *                            diagonal too), bit for bit in the matrix's dtype: the core distances, k =
  *                            min_samples + 1 (contrib's np.partition(D, min_samples, axis=0)[min_samples] in
  *                            mutual_reachability)
- *   po_hdbscan_mst_workspace bytes of d_work the two entries below need for n points
+ *   po_hdbscan_mst_workspace bytes of d_work the three entries below need for n points
  *   po_hdbscan_mst_init      n singleton components in d_work
- *   po_hdbscan_mst_round     one Boruvka round over mr(i, j) = max(core_i, core_j, D[i, j]), computed on the fly
- *                            and never stored (replaces contrib's mutual_reachability and mst_linkage_core): one
- *                            pass over the matrix finds every row's lightest edge to another component, then a
- *                            per-component reduction, hooking and pointer jumping.  Appends the new edges to
- *                            d_u, d_v (int64) and d_w (the matrix's dtype), n - 1 entries each over all rounds,
+ *   po_hdbscan_mst_scan      the pass of one Boruvka round over the rows [row0, row0 + n_rows) of the matrix, held in
+ *                            d_D (row pitch ld, n columns): every row's lightest edge to another component under
+ *                            mr(i, j) = max(core_i, core_j, D[i, j]), computed on the fly and never stored
+ *                            (replaces contrib's mutual_reachability and mst_linkage_core).  A round scans every
+ *                            row once, in one call or in row panels, then merges.
+ *   po_hdbscan_mst_merge     the rest of the round: per-component reduction, hooking and pointer jumping.  Appends
+ *                            the new edges to d_u, d_v (int64) and d_w (dtype), n - 1 entries each over all rounds,
  *                            in no particular order; *h_components = components left (1 when done).  Reads two
  *                            counters to the host (synchronises `stream`).
  *   po_hdbscan_tree          host: sorts the n - 1 MST edges in place by the tie rule (u < v), then contrib's
@@ -371,12 +382,15 @@ int po_matrix_knn(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_
  *                            get_probabilities: labels (-1 = noise; clusters numbered in ascending condensed-tree
  *                            id) and probabilities.  O(N log N).
  */
-int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, void* d_work, po_stream_t stream);
+int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int64_t row0, const void* d_cols,
+                     int64_t ld_cols, void* d_work, po_stream_t stream);
 int po_matrix_kth(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int k, void* d_out, po_stream_t stream);
 int64_t po_hdbscan_mst_workspace(int64_t n);
 int po_hdbscan_mst_init(int64_t n, void* d_work, po_stream_t stream);
-int po_hdbscan_mst_round(const void* d_D, int64_t ld, int dtype, int64_t n, const void* d_core, void* d_work, int64_t* d_u,
-                         int64_t* d_v, void* d_w, int64_t* h_components, po_stream_t stream);
+int po_hdbscan_mst_scan(const void* d_D, int64_t ld, int dtype, int64_t row0, int64_t n_rows, int64_t n, const void* d_core,
+                        void* d_work, po_stream_t stream);
+int po_hdbscan_mst_merge(int64_t n, int dtype, const void* d_core, void* d_work, int64_t* d_u, int64_t* d_v, void* d_w,
+                         int64_t* h_components, po_stream_t stream);
 int po_hdbscan_tree(int64_t n, int64_t min_cluster_size, int64_t* u, int64_t* v, double* w, int64_t* sl_left, int64_t* sl_right,
                     double* sl_dist, int64_t* sl_size, int64_t* ct_parent, int64_t* ct_child, double* ct_lambda, int64_t* ct_size,
                     int64_t* ct_rows, int64_t* labels, double* probabilities);
@@ -387,7 +401,8 @@ int po_hdbscan_tree(int64_t n, int64_t min_cluster_size, int64_t* u, int64_t* v,
  * exact gradient of the sparse-P objective; these entries evaluate it exactly.  Sums run in a fixed order.
  *   po_tsne_check            refuses (PO_ERR_ARG) a matrix holding a NaN, an infinite or a negative entry
  *                            (check_array / check_non_negative); the message names the first in row-major order.
- *                            d_work: 8 bytes.  Synchronises `stream`.
+ *                            d_D holds the rows [row0, row0 + n_rows) (row0 = 0: the whole matrix); the message
+ *                            names the absolute entry.  d_work: 8 bytes.  Synchronises `stream`.
  *   po_tsne_conditional      _binary_search_perplexity over the k neighbours d_idx [n x k] (po_matrix_knn) of
  *                            every row: squared distances D[i, idx]^2 in the matrix's dtype, then float32; the
  *                            search in float64 (tolerance 1e-5 on the entropy, at most 100 steps).  d_P float64
@@ -407,7 +422,8 @@ int po_hdbscan_tree(int64_t n, int64_t min_cluster_size, int64_t* u, int64_t* v,
  *                            tiny)) and |grad gains|^2 are reduced and copied to h_kl_gradnorm2[0..1]
  *                            (synchronises `stream`).
  */
-int po_tsne_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, void* d_work, po_stream_t stream);
+int po_tsne_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int64_t row0, void* d_work,
+                  po_stream_t stream);
 int po_tsne_conditional(const void* d_D, int64_t ld, int dtype, int64_t n, const int* d_idx, int k, double perplexity, double* d_P,
                         po_stream_t stream);
 int po_tsne_sum(const double* d_x, int64_t n, double* d_out, po_stream_t stream);

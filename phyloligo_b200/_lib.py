@@ -19,7 +19,7 @@ METRICS = {"Eucl": 0, "JSD": 1, "KT": 2, "BC": 3, "SC": 4,
            # through sklearn euclidean_distances, bin/phyloligo.py:200-202, 238-246)
            "EuclGram": 5}
 PO_F32, PO_F64 = 0, 1
-FLAG_SKIP_LOWER, FLAG_MIRROR = 1, 2
+FLAG_SKIP_LOWER, FLAG_MIRROR, FLAG_MIRROR_ONLY = 1, 2, 4
 TILE = 128  # largest kernel tile edge: row panels and rank boundaries are multiples of it
 
 # every symbol include/phyloligo_b200.h declares (tests check the library exports them all)
@@ -31,7 +31,7 @@ EXPORTED = [
     "po_host_pread", "po_host_transpose_f32",
     "po_host_mirror_open", "po_host_mirror_submit", "po_host_mirror_wait", "po_host_mirror_close",
     "po_matrix_rowsums", "po_matrix_argmin_rows", "po_cluster_argmin", "po_matrix_knn",
-    "po_hdbscan_check", "po_matrix_kth", "po_hdbscan_mst_workspace", "po_hdbscan_mst_init", "po_hdbscan_mst_round", "po_hdbscan_tree",
+    "po_hdbscan_check", "po_matrix_kth", "po_hdbscan_mst_workspace", "po_hdbscan_mst_init", "po_hdbscan_mst_scan", "po_hdbscan_mst_merge", "po_hdbscan_tree",
     "po_tsne_check", "po_tsne_conditional", "po_tsne_sum", "po_tsne_workspace", "po_tsne_repulsion", "po_tsne_attraction_step",
     "po_linkage_workspace", "po_linkage_run", "po_linkage_tree",
     "po_nj_capacity", "po_nj_workspace", "po_nj_stage_bytes", "po_nj_run",
@@ -129,7 +129,7 @@ def load():
     lib.po_cluster_argmin.restype = i32
     lib.po_matrix_knn.argtypes = [vp, i64, i32, i64, i64, i64, i32, vp, vp, vp]
     lib.po_matrix_knn.restype = i32
-    lib.po_hdbscan_check.argtypes = [vp, i64, i32, i64, i64, vp, vp]
+    lib.po_hdbscan_check.argtypes = [vp, i64, i32, i64, i64, i64, vp, i64, vp, vp]
     lib.po_hdbscan_check.restype = i32
     lib.po_matrix_kth.argtypes = [vp, i64, i32, i64, i64, i32, vp, vp]
     lib.po_matrix_kth.restype = i32
@@ -137,11 +137,13 @@ def load():
     lib.po_hdbscan_mst_workspace.restype = i64
     lib.po_hdbscan_mst_init.argtypes = [i64, vp, vp]
     lib.po_hdbscan_mst_init.restype = i32
-    lib.po_hdbscan_mst_round.argtypes = [vp, i64, i32, i64, vp, vp, vp, vp, vp, C.POINTER(i64), vp]
-    lib.po_hdbscan_mst_round.restype = i32
+    lib.po_hdbscan_mst_scan.argtypes = [vp, i64, i32, i64, i64, i64, vp, vp, vp]
+    lib.po_hdbscan_mst_scan.restype = i32
+    lib.po_hdbscan_mst_merge.argtypes = [i64, i32, vp, vp, vp, vp, vp, C.POINTER(i64), vp]
+    lib.po_hdbscan_mst_merge.restype = i32
     lib.po_hdbscan_tree.argtypes = [i64, i64] + [vp] * 14
     lib.po_hdbscan_tree.restype = i32
-    lib.po_tsne_check.argtypes = [vp, i64, i32, i64, i64, vp, vp]
+    lib.po_tsne_check.argtypes = [vp, i64, i32, i64, i64, i64, vp, vp]
     lib.po_tsne_check.restype = i32
     lib.po_tsne_conditional.argtypes = [vp, i64, i32, i64, vp, i32, C.c_double, vp, vp]
     lib.po_tsne_conditional.restype = i32

@@ -135,8 +135,9 @@ struct TileParams {
     int kdim;             // number of elements to stream (== ldp)
 };
 
-// TM = tile rows; tile columns are always 64; threads = 4 * TM.
-template <int KIND, typename OUT_T, int TM>
+// TM = tile rows; tile columns are always 64; threads = 4 * TM.  MO (PO_FLAG_MIRROR_ONLY): the tile goes to the
+// mirror buffer only; the instantiations of the other flags do not contain the branch.
+template <int KIND, typename OUT_T, int TM, bool MO>
 __global__ void __launch_bounds__(4 * TM, 2) distance_tile_kernel(const TileParams p) {
     constexpr int NT = 4 * TM;          // threads
     constexpr int RS = TM / 4;          // row stride between the 4 rows a thread owns
@@ -259,10 +260,12 @@ __global__ void __launch_bounds__(4 * TM, 2) distance_tile_kernel(const TilePara
     OUT_T* out = reinterpret_cast<OUT_T*>(p.out);
     const int64_t rmax = min((int64_t)TM, p.row1 - row_base);
     const int64_t cmax = min((int64_t)TN, p.col1 - col_base);
-    for (int e = tid; e < TM * TN; e += NT) {
-        const int r = e >> 6, c = e & 63;
-        if (r < rmax && c < cmax)
-            out[(row_base + r - p.out_row0) * p.ld_out + (col_base + c - p.out_col0)] = tile[r * TP + c];
+    if (!MO) {
+        for (int e = tid; e < TM * TN; e += NT) {
+            const int r = e >> 6, c = e & 63;
+            if (r < rmax && c < cmax)
+                out[(row_base + r - p.out_row0) * p.ld_out + (col_base + c - p.out_col0)] = tile[r * TP + c];
+        }
     }
     if ((p.flags & PO_FLAG_MIRROR) && row_base + TM <= col_base) {
         OUT_T* mir = reinterpret_cast<OUT_T*>(p.mir);
@@ -283,10 +286,15 @@ static int launch_kind(const TileParams& p, int out_dtype, cudaStream_t stream) 
     }
     dim3 grid((unsigned)tc, (unsigned)tr, 1);
     LaunchTimer t(1, stream);
-    if (out_dtype == PO_F32)
-        distance_tile_kernel<KIND, float, TM><<<grid, 4 * TM, 0, stream>>>(p);
+    const bool mo = (p.flags & PO_FLAG_MIRROR_ONLY) != 0;
+    if (out_dtype == PO_F32 && !mo)
+        distance_tile_kernel<KIND, float, TM, false><<<grid, 4 * TM, 0, stream>>>(p);
+    else if (out_dtype == PO_F32)
+        distance_tile_kernel<KIND, float, TM, true><<<grid, 4 * TM, 0, stream>>>(p);
+    else if (!mo)
+        distance_tile_kernel<KIND, double, TM, false><<<grid, 4 * TM, 0, stream>>>(p);
     else
-        distance_tile_kernel<KIND, double, TM><<<grid, 4 * TM, 0, stream>>>(p);
+        distance_tile_kernel<KIND, double, TM, true><<<grid, 4 * TM, 0, stream>>>(p);
     count_launch(1);
     PO_LAUNCH_CHECK("distance_tile_kernel");
     return PO_OK;

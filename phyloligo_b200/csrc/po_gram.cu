@@ -491,7 +491,8 @@ template <> struct GramCfg<GM_SC> {
 // group itself -- and the computed values left of the diagonal are dropped, whatever the flags, so
 // that a block row computed on its own equals the rows of the symmetric run bit for bit.  Groups
 // wholly below the diagonal get the same effect from the MMA issue order (see the kernel).
-template <typename OUT_T, int MODE, bool INTERIOR, bool DIAG>
+// MO (PO_FLAG_MIRROR_ONLY): only the mirror stores; the kernel never calls a diagonal group's epilogue with it.
+template <typename OUT_T, int MODE, bool INTERIOR, bool DIAG, bool MO>
 __device__ __forceinline__ void gram_epilogue(const GramParams& p, unsigned tmem, int64_t row_base, int64_t col_base,
                                               const double* s_nb, unsigned char* gsmem) {
     constexpr int NCQ = GramCfg<MODE>::THREADS / 128;  // column slices of the group (warps per lane quarter)
@@ -604,7 +605,7 @@ __device__ __forceinline__ void gram_epilogue(const GramParams& p, unsigned tmem
             for (int j = 0; j < 16; ++j) tbuf[half * 16 + j] = val[j];
         }
         __syncwarp();
-        {
+        if (!MO) {
             const int c = cq * WCOLS + blk * 32 + lane;  // column of the group this lane stores
             const int64_t gcol = col_base + c;
             const bool col_ok = INTERIOR || (gcol >= p.col0 && gcol < p.col1);
@@ -623,7 +624,7 @@ __device__ __forceinline__ void gram_epilogue(const GramParams& p, unsigned tmem
     }
 }
 
-template <typename OUT_T, int MODE>
+template <typename OUT_T, int MODE, bool MO>
 __global__ void __launch_bounds__(GramCfg<MODE>::THREADS, GramCfg<MODE>::CTAS) gram_tile_kernel(const GramParams p) {
     using Cfg = GramCfg<MODE>;
     constexpr int NB = Cfg::NB, KS = Cfg::KS, NSTAGE = Cfg::STAGES;
@@ -841,12 +842,13 @@ __global__ void __launch_bounds__(GramCfg<MODE>::THREADS, GramCfg<MODE>::CTAS) g
         const unsigned tg = tmem + (unsigned)(g * Cfg::GROUP_COLS);
         // groups wholly inside the requested block (all but the ragged edges) skip the per-entry bounds tests
         const bool interior = row_base >= p.row0 && row_base + GT <= p.row1 && cb >= p.col0 && cb + GT <= p.col1;
-        if (!gm_is_sc(MODE) && cb == row_base)
-            gram_epilogue<OUT_T, MODE, false, true>(p, tg, row_base, cb, s_nb + g * GT, gsmem);
-        else if (interior)
-            gram_epilogue<OUT_T, MODE, true, false>(p, tg, row_base, cb, s_nb + g * GT, gsmem);
-        else
-            gram_epilogue<OUT_T, MODE, false, false>(p, tg, row_base, cb, s_nb + g * GT, gsmem);
+        if (!gm_is_sc(MODE) && cb == row_base) {
+            if (!MO) gram_epilogue<OUT_T, MODE, false, true, false>(p, tg, row_base, cb, s_nb + g * GT, gsmem);
+        } else if (interior) {
+            gram_epilogue<OUT_T, MODE, true, false, MO>(p, tg, row_base, cb, s_nb + g * GT, gsmem);
+        } else {
+            gram_epilogue<OUT_T, MODE, false, false, MO>(p, tg, row_base, cb, s_nb + g * GT, gsmem);
+        }
         if (NB > 1) __syncthreads();  // the staging buffers are reused by the next group
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -854,8 +856,8 @@ __global__ void __launch_bounds__(GramCfg<MODE>::THREADS, GramCfg<MODE>::CTAS) g
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((unsigned)Cfg::TMEM_COLS));
 }
 
-template <typename OUT_T, int MODE>
-static int launch_gram_t(GramParams p, int64_t row1, int64_t col1, cudaStream_t stream) {
+template <typename OUT_T, int MODE, bool MO>
+static int launch_gram_mo(GramParams p, int64_t row1, int64_t col1, cudaStream_t stream) {
     using Cfg = GramCfg<MODE>;
     const int64_t tile_n = (int64_t)Cfg::NB * GT;
     p.tile_col0 = p.col0 / tile_n * tile_n;
@@ -867,9 +869,15 @@ static int launch_gram_t(GramParams p, int64_t row1, int64_t col1, cudaStream_t 
     p.tiles_r = tr;
     p.tiles_c = tc;
     const size_t smem = (size_t)Cfg::STAGES * (1 + Cfg::NB) * 2 * GT * Cfg::KS * Cfg::ELEM_BYTES + 1024;
-    PO_CUDA_CHECK(cudaFuncSetAttribute(gram_tile_kernel<OUT_T, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    gram_tile_kernel<OUT_T, MODE><<<dim3((unsigned)(tr * tc), 1, 1), Cfg::THREADS, smem, stream>>>(p);
+    PO_CUDA_CHECK(cudaFuncSetAttribute(gram_tile_kernel<OUT_T, MODE, MO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    gram_tile_kernel<OUT_T, MODE, MO><<<dim3((unsigned)(tr * tc), 1, 1), Cfg::THREADS, smem, stream>>>(p);
     return PO_OK;
+}
+
+template <typename OUT_T, int MODE>
+static int launch_gram_t(GramParams p, int64_t row1, int64_t col1, cudaStream_t stream) {
+    return (p.flags & PO_FLAG_MIRROR_ONLY) ? launch_gram_mo<OUT_T, MODE, true>(p, row1, col1, stream)
+                                           : launch_gram_mo<OUT_T, MODE, false>(p, row1, col1, stream);
 }
 
 int launch_gram(int metric, const void* d_P, const double* d_aux, int64_t n, int64_t dim, int64_t row0, int64_t row1,

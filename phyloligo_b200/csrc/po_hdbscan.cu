@@ -3,8 +3,9 @@
 // default).  Replaces, in scikit-learn-contrib/hdbscan:
 //   mutual_reachability + mst_linkage_core   the float64 N x N copy and the O(N^2) Prim loop on one core
 //                                            -> po_hdbscan_check, po_matrix_kth (po_select.cu: core
-//                                               distances), po_hdbscan_mst_init / po_hdbscan_mst_round
-//                                               (Boruvka; mutual reachability computed on the fly)
+//                                               distances), po_hdbscan_mst_init / po_hdbscan_mst_scan /
+//                                               po_hdbscan_mst_merge (Boruvka; mutual reachability computed
+//                                               on the fly, the matrix read whole or in row panels)
 //   label, condense_tree, compute_stability,
 //   get_clusters, get_probabilities          -> po_hdbscan_tree (host, O(N log N))
 //
@@ -64,6 +65,46 @@ __global__ void __launch_bounds__(256) check_kernel(const void* __restrict__ D, 
     if ((threadIdx.x & 31) == 0 && bad != ~0ull) atomicMin(first_bad, bad);
 }
 
+// The same test on the row panel [row0, row0 + rows) x [0, n): entry (i, j) against (j, i), read from the column
+// strip S ([0, n) x [row0, row0 + rows), pitch lds) or, without a strip, from the panel itself when j lies in the
+// panel's rows (a source symmetric by construction is tested on its diagonal square only).  Keys are absolute.
+template <typename T>
+__global__ void __launch_bounds__(256) panel_check_kernel(const void* __restrict__ D, int64_t ld, int64_t rows, int64_t n,
+                                                          int64_t row0, const void* __restrict__ S, int64_t lds,
+                                                          unsigned long long* __restrict__ first_bad) {
+    using B = typename Bits<T>::type;
+    const int64_t bi = blockIdx.y, bj = blockIdx.x;
+    __shared__ B a[CHK][CHK + 1], b[CHK][CHK + 1];
+    __shared__ bool has[CHK][CHK + 1];
+    const B* M = reinterpret_cast<const B*>(D);
+    const B* ST = reinterpret_cast<const B*>(S);
+    const int c = threadIdx.x & 31;
+    unsigned long long bad = ~0ull;
+    for (int r = threadIdx.x >> 5; r < CHK; r += 8) {
+        const int64_t li = bi * CHK + r, j = bj * CHK + c;     // entry (row0 + li, j)
+        const int64_t tj = bj * CHK + r, tli = bi * CHK + c;   // entry (tj, row0 + tli)
+        a[r][c] = (li < rows && j < n) ? M[li * ld + j] : (B)0;
+        bool h = tj < n && tli < rows;
+        B v = (B)0;
+        if (h && S) v = ST[tj * lds + tli];
+        else if (h && tj >= row0 && tj < row0 + rows) v = M[(tj - row0) * ld + row0 + tli];
+        else h = false;
+        b[r][c] = v;
+        has[r][c] = h;
+    }
+    __syncthreads();
+    for (int r = threadIdx.x >> 5; r < CHK; r += 8) {
+        const int64_t li = bi * CHK + r, j = bj * CHK + c, i = row0 + li;
+        if (li < rows && j < n) {
+            if (!isfinite(reinterpret_cast<const T&>(a[r][c]))) bad = min(bad, (unsigned long long)(i * n + j));
+            if (has[c][r] && a[r][c] != b[c][r]) bad = min(bad, (unsigned long long)(min(i, j) * n + max(i, j)));
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) bad = min(bad, __shfl_xor_sync(0xFFFFFFFFu, bad, o));
+    if ((threadIdx.x & 31) == 0 && bad != ~0ull) atomicMin(first_bad, bad);
+}
+
 // ---------------------------------------------------------------------------------------------------
 // Boruvka over the mutual-reachability graph
 // ---------------------------------------------------------------------------------------------------
@@ -77,11 +118,13 @@ __device__ __forceinline__ T mr(T core_i, T core_j, T d) {
     return c > d ? c : d;
 }
 
-// workspace (all n entries): comp, P, P2 int32; row_j int32; row_key, comp_key, comp_edge uint64; then
-// two int32 counters (edges found so far, components)
+// workspace (all n entries): row_key, comp_key, comp_edge uint64; row_d float64 (D[i, row_j[i]], so that the
+// merge needs no access to the matrix); comp, P, P2, row_j int32; then two int32 counters (edges found so far,
+// components)
 struct Work {
     int *comp, *P, *P2, *row_j;
     unsigned long long *row_key, *comp_key, *comp_edge;
+    double* row_d;
     int* counters;
 };
 Work carve(void* d_work, int64_t n) {
@@ -90,7 +133,8 @@ Work carve(void* d_work, int64_t n) {
     w.row_key = reinterpret_cast<unsigned long long*>(p);
     w.comp_key = w.row_key + n;
     w.comp_edge = w.comp_key + n;
-    int* q = reinterpret_cast<int*>(w.comp_edge + n);
+    w.row_d = reinterpret_cast<double*>(w.comp_edge + n);
+    int* q = reinterpret_cast<int*>(w.row_d + n);
     w.comp = q;
     w.P = q + n;
     w.P2 = q + 2 * n;
@@ -103,25 +147,29 @@ constexpr int RM_THREADS = 256;
 constexpr int RM_ROWS = 8;    // rows per CTA: the column's core distance and component are loaded once for all of them
 constexpr int RM_UNROLL = 4;  // columns per thread per step: RM_ROWS x RM_UNROLL loads in flight
 
-// For every row i, its lightest edge (mr(i, j), j) to a column of another component.  For a fixed row the tie
-// rule's (min(i, j), max(i, j)) orders the columns as j does, so the per-row minimum is taken over (mr, j).
+// For every row i of the panel [row0, row0 + n_rows) (D points at its first row), its lightest edge (mr(i, j), j)
+// to a column of another component.  For a fixed row the tie rule's (min(i, j), max(i, j)) orders the columns as
+// j does, so the per-row minimum is taken over (mr, j).
 template <typename T>
-__global__ void __launch_bounds__(RM_THREADS) rowmin_kernel(const void* __restrict__ D, int64_t ld, int n, const T* __restrict__ core,
-                                                            const int* __restrict__ comp, unsigned long long* __restrict__ row_key,
-                                                            int* __restrict__ row_j) {
-    const int r0 = blockIdx.x * RM_ROWS;
-    const T* base = reinterpret_cast<const T*>(D) + (int64_t)r0 * ld;
-    T ci[RM_ROWS], bw[RM_ROWS];
+__global__ void __launch_bounds__(RM_THREADS) rowmin_kernel(const void* __restrict__ D, int64_t ld, int row0, int n_rows, int n,
+                                                            const T* __restrict__ core, const int* __restrict__ comp,
+                                                            unsigned long long* __restrict__ row_key, int* __restrict__ row_j,
+                                                            double* __restrict__ row_d) {
+    const int l0 = blockIdx.x * RM_ROWS;  // first panel row of this CTA
+    const int r0 = row0 + l0;             // its matrix row
+    const T* base = reinterpret_cast<const T*>(D) + (int64_t)l0 * ld;
+    T ci[RM_ROWS], bw[RM_ROWS], bd[RM_ROWS];
     int cc[RM_ROWS], bj[RM_ROWS];
 #pragma unroll
     for (int r = 0; r < RM_ROWS; ++r) {
-        const bool ok = r0 + r < n;
+        const bool ok = l0 + r < n_rows;
         ci[r] = ok ? core[r0 + r] : (T)0;
         cc[r] = ok ? comp[r0 + r] : -1;
         bw[r] = (T)__longlong_as_double(0x7FF0000000000000ll);  // +inf
+        bd[r] = (T)0;
         bj[r] = -1;
     }
-    const int rows = min(RM_ROWS, n - r0);
+    const int rows = min(RM_ROWS, n_rows - l0);
     // rows past the end re-read the last row (never written back): no branch between the loads, so all
     // RM_ROWS x RM_UNROLL of them are in flight together
     int64_t roff[RM_ROWS];
@@ -146,6 +194,7 @@ __global__ void __launch_bounds__(RM_THREADS) rowmin_kernel(const void* __restri
                 // columns are visited in increasing order by each thread: strict < keeps the first on ties
                 if (gj[u] >= 0 && gj[u] != cc[r] && w < bw[r]) {
                     bw[r] = w;
+                    bd[r] = d[r][u];
                     bj[r] = j0 + u * RM_THREADS;
                 }
             }
@@ -153,23 +202,28 @@ __global__ void __launch_bounds__(RM_THREADS) rowmin_kernel(const void* __restri
     }
     __shared__ unsigned long long s_key[RM_THREADS / 32][RM_ROWS];
     __shared__ int s_j[RM_THREADS / 32][RM_ROWS];
+    __shared__ double s_d[RM_THREADS / 32][RM_ROWS];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
     for (int r = 0; r < RM_ROWS; ++r) {
         unsigned long long k = bj[r] >= 0 ? wkey((double)bw[r]) : ~0ull;
         int j = bj[r] >= 0 ? bj[r] : 0x7FFFFFFF;
+        double dv = (double)bd[r];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
             const unsigned long long k2 = __shfl_xor_sync(0xFFFFFFFFu, k, o);
             const int j2 = __shfl_xor_sync(0xFFFFFFFFu, j, o);
+            const double d2 = __shfl_xor_sync(0xFFFFFFFFu, dv, o);
             if (k2 < k || (k2 == k && j2 < j)) {
                 k = k2;
                 j = j2;
+                dv = d2;
             }
         }
         if (lane == 0) {
             s_key[warp][r] = k;
             s_j[warp][r] = j;
+            s_d[warp][r] = dv;
         }
     }
     __syncthreads();
@@ -177,14 +231,17 @@ __global__ void __launch_bounds__(RM_THREADS) rowmin_kernel(const void* __restri
         const int r = threadIdx.x;
         unsigned long long k = s_key[0][r];
         int j = s_j[0][r];
+        double dv = s_d[0][r];
         for (int w = 1; w < RM_THREADS / 32; ++w) {
             if (s_key[w][r] < k || (s_key[w][r] == k && s_j[w][r] < j)) {
                 k = s_key[w][r];
                 j = s_j[w][r];
+                dv = s_d[w][r];
             }
         }
         row_key[r0 + r] = k;
         row_j[r0 + r] = (k == ~0ull) ? -1 : j;
+        row_d[r0 + r] = dv;
     }
 }
 
@@ -206,11 +263,13 @@ __global__ void comp_edge_kernel(int n, const int* __restrict__ comp, const unsi
 
 // hooking: every component (root c, comp[c] == c) points at the component across its lightest edge.  Two
 // components that chose the same edge point at each other; the smaller id stays a root and the edge is
-// emitted once, by the other.  Non-roots keep pointing at their root.
+// emitted once, by the other.  Non-roots keep pointing at their root.  The edge (u, v) came from row u or row v,
+// whose scan kept D[u, v] or D[v, u]: the same bits, the matrix having passed the symmetry check.
 template <typename T>
-__global__ void hook_kernel(const void* __restrict__ D, int64_t ld, int n, const T* __restrict__ core, const int* __restrict__ comp,
-                            const unsigned long long* __restrict__ comp_edge, int* __restrict__ P, int* __restrict__ counters,
-                            int64_t* __restrict__ out_u, int64_t* __restrict__ out_v, T* __restrict__ out_w) {
+__global__ void hook_kernel(int n, const T* __restrict__ core, const int* __restrict__ comp, const int* __restrict__ row_j,
+                            const double* __restrict__ row_d, const unsigned long long* __restrict__ comp_edge, int* __restrict__ P,
+                            int* __restrict__ counters, int64_t* __restrict__ out_u, int64_t* __restrict__ out_v,
+                            T* __restrict__ out_w) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n) return;
     if (comp[c] != c || comp_edge[c] == ~0ull) {
@@ -229,7 +288,7 @@ __global__ void hook_kernel(const void* __restrict__ D, int64_t ld, int n, const
     if (pos < n - 1) {
         out_u[pos] = u;
         out_v[pos] = v;
-        out_w[pos] = mr(core[u], core[v], reinterpret_cast<const T*>(D)[(int64_t)u * ld + v]);
+        out_w[pos] = mr(core[u], core[v], (T)(row_j[u] == v ? row_d[u] : row_d[v]));
     }
 }
 
@@ -284,30 +343,41 @@ using namespace po;
 
 extern "C" {
 
-int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, void* d_work, po_stream_t stream) {
-    if (!d_D || !d_work || n_rows < 0 || n_cols < 0 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64)) {
+int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int64_t row0, const void* d_cols,
+                     int64_t ld_cols, void* d_work, po_stream_t stream) {
+    if (!d_D || !d_work || n_rows < 0 || n_cols < 0 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64) || row0 < 0 ||
+        ld_cols < 0 || (d_cols && ld_cols < n_rows) || (ld_cols == 0 && (d_cols || row0 != 0))) {
         set_error("po_hdbscan_check: bad arguments");
         return PO_ERR_ARG;
     }
-    if (n_rows != n_cols) {
-        set_error("po_hdbscan_check: the matrix is not square (%lld x %lld)", (long long)n_rows, (long long)n_cols);
+    const bool whole = ld_cols == 0;
+    if (whole ? n_rows != n_cols : row0 + n_rows > n_cols) {
+        set_error("po_hdbscan_check: the matrix is not square (%lld x %lld)", (long long)(row0 + n_rows), (long long)n_cols);
         return PO_ERR_ARG;
     }
-    const int64_t n = n_rows;
-    if (n == 0) return PO_OK;
-    const int64_t nb = (n + CHK - 1) / CHK;
-    if (nb > 65535) {
-        set_error("po_hdbscan_check: %lld rows is more than this check supports", (long long)n);
+    const int64_t n = n_cols;
+    if (n_rows == 0) return PO_OK;
+    const int64_t nb = (n + CHK - 1) / CHK, rb = (n_rows + CHK - 1) / CHK;
+    if (rb > 65535 || (whole && nb > 65535)) {
+        set_error("po_hdbscan_check: %lld rows is more than this check supports", (long long)n_rows);
         return PO_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long* first = reinterpret_cast<unsigned long long*>(d_work);
     PO_CUDA_CHECK(cudaMemsetAsync(first, 0xFF, sizeof(unsigned long long), st));
-    const dim3 grid((unsigned)nb, (unsigned)nb);
-    if (dtype == PO_F32)
-        check_kernel<float><<<grid, 256, 0, st>>>(d_D, ld, n, first);
-    else
-        check_kernel<double><<<grid, 256, 0, st>>>(d_D, ld, n, first);
+    if (whole) {
+        const dim3 grid((unsigned)nb, (unsigned)nb);
+        if (dtype == PO_F32)
+            check_kernel<float><<<grid, 256, 0, st>>>(d_D, ld, n, first);
+        else
+            check_kernel<double><<<grid, 256, 0, st>>>(d_D, ld, n, first);
+    } else {
+        const dim3 grid((unsigned)nb, (unsigned)rb);
+        if (dtype == PO_F32)
+            panel_check_kernel<float><<<grid, 256, 0, st>>>(d_D, ld, n_rows, n, row0, d_cols, ld_cols, first);
+        else
+            panel_check_kernel<double><<<grid, 256, 0, st>>>(d_D, ld, n_rows, n, row0, d_cols, ld_cols, first);
+    }
     count_launch(2);
     PO_LAUNCH_CHECK("check_kernel");
     unsigned long long bad = 0;
@@ -319,8 +389,17 @@ int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int
     double x[2];
     for (int q = 0; q < 2; ++q) {
         const int64_t r = q ? j : i, c = q ? i : j;
+        // entry (r, c): in the panel when r is one of its rows, else in the column strip.  Without a strip the source
+        // is symmetric and a pair outside the diagonal square can only be named for a non-finite (i, j)
+        if (q && !whole && !d_cols && !(r >= row0 && r < row0 + n_rows)) {
+            x[1] = x[0];
+            continue;
+        }
+        const char* src = (r >= row0 && r < row0 + n_rows)
+                              ? reinterpret_cast<const char*>(d_D) + ((r - row0) * ld + c) * (int64_t)es
+                              : reinterpret_cast<const char*>(d_cols) + (r * ld_cols + (c - row0)) * (int64_t)es;
         unsigned char raw[8];
-        PO_CUDA_CHECK(cudaMemcpy(raw, reinterpret_cast<const char*>(d_D) + (r * ld + c) * (int64_t)es, es, cudaMemcpyDeviceToHost));
+        PO_CUDA_CHECK(cudaMemcpy(raw, src, es, cudaMemcpyDeviceToHost));
         if (dtype == PO_F32) {
             float f;
             memcpy(&f, raw, 4);
@@ -339,7 +418,7 @@ int po_hdbscan_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int
     return PO_ERR_ARG;
 }
 
-int64_t po_hdbscan_mst_workspace(int64_t n) { return n < 0 ? -1 : n * 3 * 8 + n * 4 * 4 + 2 * 4; }
+int64_t po_hdbscan_mst_workspace(int64_t n) { return n < 0 ? -1 : n * 4 * 8 + n * 4 * 4 + 2 * 4; }
 
 int po_hdbscan_mst_init(int64_t n, void* d_work, po_stream_t stream) {
     if (!d_work || n < 1 || n > 0x7FFFFFFFll) {
@@ -353,11 +432,33 @@ int po_hdbscan_mst_init(int64_t n, void* d_work, po_stream_t stream) {
     return PO_OK;
 }
 
-int po_hdbscan_mst_round(const void* d_D, int64_t ld, int dtype, int64_t n, const void* d_core, void* d_work, int64_t* d_u,
-                         int64_t* d_v, void* d_w, int64_t* h_components, po_stream_t stream) {
-    if (!d_D || !d_core || !d_work || !d_u || !d_v || !d_w || !h_components || n < 1 || n > 0x7FFFFFFFll || ld < n ||
+int po_hdbscan_mst_scan(const void* d_D, int64_t ld, int dtype, int64_t row0, int64_t n_rows, int64_t n, const void* d_core,
+                        void* d_work, po_stream_t stream) {
+    if (!d_D || !d_core || !d_work || n < 1 || n > 0x7FFFFFFFll || row0 < 0 || n_rows < 0 || row0 + n_rows > n || ld < n ||
         (dtype != PO_F32 && dtype != PO_F64)) {
-        set_error("po_hdbscan_mst_round: bad arguments");
+        set_error("po_hdbscan_mst_scan: bad arguments");
+        return PO_ERR_ARG;
+    }
+    if (n_rows == 0) return PO_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    Work w = carve(d_work, n);
+    const unsigned grows = (unsigned)((n_rows + RM_ROWS - 1) / RM_ROWS);
+    if (dtype == PO_F32)
+        rowmin_kernel<float><<<grows, RM_THREADS, 0, st>>>(d_D, ld, (int)row0, (int)n_rows, (int)n, (const float*)d_core, w.comp,
+                                                          w.row_key, w.row_j, w.row_d);
+    else
+        rowmin_kernel<double><<<grows, RM_THREADS, 0, st>>>(d_D, ld, (int)row0, (int)n_rows, (int)n, (const double*)d_core, w.comp,
+                                                           w.row_key, w.row_j, w.row_d);
+    count_launch(2);
+    PO_LAUNCH_CHECK("rowmin_kernel");
+    return PO_OK;
+}
+
+int po_hdbscan_mst_merge(int64_t n, int dtype, const void* d_core, void* d_work, int64_t* d_u, int64_t* d_v, void* d_w,
+                         int64_t* h_components, po_stream_t stream) {
+    if (!d_core || !d_work || !d_u || !d_v || !d_w || !h_components || n < 1 || n > 0x7FFFFFFFll ||
+        (dtype != PO_F32 && dtype != PO_F64)) {
+        set_error("po_hdbscan_mst_merge: bad arguments");
         return PO_ERR_ARG;
     }
     cudaStream_t st = (cudaStream_t)stream;
@@ -372,20 +473,15 @@ int po_hdbscan_mst_round(const void* d_D, int64_t ld, int dtype, int64_t n, cons
         return PO_OK;
     }
     const unsigned g = (unsigned)((n + 255) / 256);
-    const unsigned grows = (unsigned)((n + RM_ROWS - 1) / RM_ROWS);
-    if (dtype == PO_F32)
-        rowmin_kernel<float><<<grows, RM_THREADS, 0, st>>>(d_D, ld, ni, (const float*)d_core, w.comp, w.row_key, w.row_j);
-    else
-        rowmin_kernel<double><<<grows, RM_THREADS, 0, st>>>(d_D, ld, ni, (const double*)d_core, w.comp, w.row_key, w.row_j);
     PO_CUDA_CHECK(cudaMemsetAsync(w.comp_key, 0xFF, 2 * n * sizeof(unsigned long long), st));
     comp_key_kernel<<<g, 256, 0, st>>>(ni, w.comp, w.row_key, w.comp_key);
     comp_edge_kernel<<<g, 256, 0, st>>>(ni, w.comp, w.row_key, w.row_j, w.comp_key, w.comp_edge);
     if (dtype == PO_F32)
-        hook_kernel<float><<<g, 256, 0, st>>>(d_D, ld, ni, (const float*)d_core, w.comp, w.comp_edge, w.P, w.counters, d_u, d_v,
-                                              (float*)d_w);
+        hook_kernel<float><<<g, 256, 0, st>>>(ni, (const float*)d_core, w.comp, w.row_j, w.row_d, w.comp_edge, w.P, w.counters, d_u,
+                                              d_v, (float*)d_w);
     else
-        hook_kernel<double><<<g, 256, 0, st>>>(d_D, ld, ni, (const double*)d_core, w.comp, w.comp_edge, w.P, w.counters, d_u, d_v,
-                                               (double*)d_w);
+        hook_kernel<double><<<g, 256, 0, st>>>(ni, (const double*)d_core, w.comp, w.row_j, w.row_d, w.comp_edge, w.P, w.counters,
+                                               d_u, d_v, (double*)d_w);
     // the hook forest is at most `before` deep: ceil(log2(before)) + 1 jumps reach every root
     int jumps = 1;
     while ((1 << (jumps - 1)) < before) ++jumps;
@@ -397,14 +493,15 @@ int po_hdbscan_mst_round(const void* d_D, int64_t ld, int dtype, int64_t n, cons
     }
     PO_CUDA_CHECK(cudaMemsetAsync(w.counters + 1, 0, sizeof(int), st));
     relabel_kernel<<<g, 256, 0, st>>>(ni, src, w.comp, w.counters);
-    for (int q = 0; q < 5 + jumps; ++q) count_launch(2);  // rowmin, comp_key, comp_edge, hook, the jumps, relabel
-    PO_LAUNCH_CHECK("Boruvka round kernels");
+    for (int q = 0; q < 4 + jumps; ++q) count_launch(2);  // comp_key, comp_edge, hook, the jumps, relabel
+    PO_LAUNCH_CHECK("Boruvka merge kernels");
     PO_CUDA_CHECK(cudaMemcpyAsync(counters, w.counters, sizeof(counters), cudaMemcpyDeviceToHost, st));
     PO_CUDA_CHECK(cudaStreamSynchronize(st));
     // a forest over n vertices: edges + components == n, and every component lost at least half
     if (counters[0] + counters[1] != ni || counters[1] > before / 2 || counters[0] <= edges_before) {
-        set_error("po_hdbscan_mst_round: inconsistent round (%d components before, %d after, %d edges); is the matrix "
-                  "symmetric and free of NaN?", before, counters[1], counters[0]);
+        set_error("po_hdbscan_mst_merge: inconsistent round (%d components before, %d after, %d edges); is the matrix "
+                  "symmetric and free of NaN, and was every row scanned once since the last merge?", before, counters[1],
+                  counters[0]);
         return PO_ERR_CUDA;
     }
     *h_components = counters[1];

@@ -321,7 +321,9 @@ __device__ __forceinline__ void jsd_chunk(const float4* __restrict__ sA, const u
     }
 }
 
-template <typename OUT_T>
+// MO (PO_FLAG_MIRROR_ONLY): the tile goes to the mirror buffer only; the instantiations of the other flags do not
+// contain the branch.
+template <typename OUT_T, bool MO>
 __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdParams p) {
     extern __shared__ __align__(128) unsigned char jsmem[];
     __shared__ __align__(8) unsigned long long bars[JSTAGES];
@@ -449,10 +451,12 @@ __global__ void __launch_bounds__(JTHREADS, JSD_CTAS) jsd_tile_kernel(const JsdP
     OUT_T* out = reinterpret_cast<OUT_T*>(p.out);
     const int r_lo = (int)max((int64_t)0, p.row0 - row_base), r_hi = (int)min((int64_t)JT_M, p.row1 - row_base);
     const int c_lo = (int)max((int64_t)0, p.col0 - col_base), c_hi = (int)min((int64_t)JT_N, p.col1 - col_base);
-    for (int e = tid; e < JT_M * JT_N; e += JTHREADS) {
-        const int r = e >> 6, c = e & 63;
-        if (r >= r_lo && r < r_hi && c >= c_lo && c < c_hi)
-            out[(row_base + r - p.out_row0) * p.ld_out + (col_base + c - p.out_col0)] = tile[r * TP + c];
+    if (!MO) {
+        for (int e = tid; e < JT_M * JT_N; e += JTHREADS) {
+            const int r = e >> 6, c = e & 63;
+            if (r >= r_lo && r < r_hi && c >= c_lo && c < c_hi)
+                out[(row_base + r - p.out_row0) * p.ld_out + (col_base + c - p.out_col0)] = tile[r * TP + c];
+        }
     }
     if ((p.flags & PO_FLAG_MIRROR) && row_base + JT_M <= col_base) {
         OUT_T* mir = reinterpret_cast<OUT_T*>(p.mir);
@@ -493,12 +497,19 @@ int launch_jsd(const void* d_P, int64_t n, int64_t dim, int64_t row0, int64_t ro
     dim3 grid((unsigned)(tr * tc), 1, 1);
     LaunchTimer tm(1, stream);
     // the opt-in is per device: set it on every launch (a process may drive several GPUs)
-    if (out_dtype == PO_F32) {
-        PO_CUDA_CHECK(cudaFuncSetAttribute(jsd_tile_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        jsd_tile_kernel<float><<<grid, JTHREADS, smem, stream>>>(p);
+    const bool mo = (flags & PO_FLAG_MIRROR_ONLY) != 0;
+    if (out_dtype == PO_F32 && !mo) {
+        PO_CUDA_CHECK(cudaFuncSetAttribute(jsd_tile_kernel<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        jsd_tile_kernel<float, false><<<grid, JTHREADS, smem, stream>>>(p);
+    } else if (out_dtype == PO_F32) {
+        PO_CUDA_CHECK(cudaFuncSetAttribute(jsd_tile_kernel<float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        jsd_tile_kernel<float, true><<<grid, JTHREADS, smem, stream>>>(p);
+    } else if (!mo) {
+        PO_CUDA_CHECK(cudaFuncSetAttribute(jsd_tile_kernel<double, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        jsd_tile_kernel<double, false><<<grid, JTHREADS, smem, stream>>>(p);
     } else {
-        PO_CUDA_CHECK(cudaFuncSetAttribute(jsd_tile_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        jsd_tile_kernel<double><<<grid, JTHREADS, smem, stream>>>(p);
+        PO_CUDA_CHECK(cudaFuncSetAttribute(jsd_tile_kernel<double, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        jsd_tile_kernel<double, true><<<grid, JTHREADS, smem, stream>>>(p);
     }
     count_launch(1);
     PO_LAUNCH_CHECK("jsd_tile_kernel");

@@ -408,8 +408,10 @@ using namespace po;
 
 extern "C" {
 
-int po_tsne_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, void* d_work, po_stream_t stream) {
-    if (!d_D || !d_work || n_rows < 0 || n_cols < 0 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64) || n_rows > 0x7FFFFFFFll) {
+int po_tsne_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_t n_cols, int64_t row0, void* d_work,
+                  po_stream_t stream) {
+    if (!d_D || !d_work || n_rows < 0 || n_cols < 0 || row0 < 0 || ld < n_cols || (dtype != PO_F32 && dtype != PO_F64) ||
+        n_rows > 0x7FFFFFFFll) {
         set_error("po_tsne_check: bad arguments");
         return PO_ERR_ARG;
     }
@@ -440,11 +442,11 @@ int po_tsne_check(const void* d_D, int64_t ld, int dtype, int64_t n_rows, int64_
         memcpy(&x, raw, 8);
     }
     if (std::isnan(x))
-        set_error("po_tsne_check: entry (%lld, %lld) is NaN", (long long)i, (long long)j);
+        set_error("po_tsne_check: entry (%lld, %lld) is NaN", (long long)(row0 + i), (long long)j);
     else if (std::isinf(x))
-        set_error("po_tsne_check: entry (%lld, %lld) is infinite (%g)", (long long)i, (long long)j, x);
+        set_error("po_tsne_check: entry (%lld, %lld) is infinite (%g)", (long long)(row0 + i), (long long)j, x);
     else
-        set_error("po_tsne_check: entry (%lld, %lld) is negative (%.17g); t-SNE needs non-negative distances", (long long)i,
+        set_error("po_tsne_check: entry (%lld, %lld) is negative (%.17g); t-SNE needs non-negative distances", (long long)(row0 + i),
                   (long long)j, x);
     return PO_ERR_ARG;
 }

@@ -30,7 +30,7 @@ import warnings
 import numpy as np
 import torch
 
-from . import _lib, engine, io_formats
+from . import _lib, engine, io_formats, panels
 from ._lib import PhyloligoError, PO_F32, PO_F64
 
 
@@ -66,6 +66,17 @@ def as_device_matrix(D):
         t = t.contiguous()
     _dt(t)
     return t
+
+
+def _source(X, metric):
+    """The row-panel source (panels.py) a fit reads: X itself when it is one; for "precomputed" the matrix X
+    (resident, or read in panels from a matrix file that does not fit on the device); otherwise the matrix of the
+    profiles X for `metric`, resident when it fits in device memory and recomputed panel by panel when not."""
+    if isinstance(X, panels.SOURCES):
+        return X
+    if metric == "precomputed":
+        return panels.as_source(X)
+    return panels.profile_source(X, metric)
 
 
 def row_sums(D, rows=None, labels=None, row_labels=None):
@@ -105,18 +116,31 @@ def cluster_argmin(cost, labels, k):
     return best_idx, best_cost, count
 
 
+def _knn_rows(P, self0, k, idx, dist):
+    """po_matrix_knn of the rows of the device view P (row i is matrix row self0 + i) into idx / dist."""
+    rc = _lib.load().po_matrix_knn(_ptr(P), int(P.stride(0)), _dt(P), int(P.shape[0]), int(P.shape[1]), int(self0), int(k),
+                                   _ptr(idx), _ptr(dist), _stream())
+    _lib.check(rc, "po_matrix_knn")
+
+
 def knn_graph(D, k, row0=0, as_sparse=False):
     """The k nearest neighbours of every row of the device matrix D (a block row when row0 > 0: row i is
-    profile row0 + i and that column is excluded), ascending, ties by column (po_matrix_knn).
+    profile row0 + i and that column is excluded), ascending, ties by column (po_matrix_knn).  D may also be a
+    row-panel source (panels.py): one pass over its panels.
     Returns (indices int32 [n, k], distances float32 [n, k]) device tensors, or with `as_sparse` the
     scipy CSR matrix that sklearn's TSNE(metric="precomputed") / kneighbors_graph(mode="distance") use."""
-    lib = _lib.load()
-    D = D if isinstance(D, torch.Tensor) and D.is_cuda else as_device_matrix(D)
-    n_rows, n_cols = int(D.shape[0]), int(D.shape[1])
-    idx = torch.empty((n_rows, k), dtype=torch.int32, device=D.device)
-    dist = torch.empty((n_rows, k), dtype=torch.float32, device=D.device)
-    rc = lib.po_matrix_knn(_ptr(D), int(D.stride(0)), _dt(D), n_rows, n_cols, int(row0), int(k), _ptr(idx), _ptr(dist), _stream())
-    _lib.check(rc, "po_matrix_knn")
+    if isinstance(D, panels.SOURCES):
+        parts = ((r0, r1, P) for r0, r1, P in D.panels())
+        n_rows, n_cols, dev = D.n, D.n, D.device
+    else:
+        D = D if isinstance(D, torch.Tensor) and D.is_cuda else as_device_matrix(D)
+        n_rows, n_cols, dev = int(D.shape[0]), int(D.shape[1]), D.device
+        parts = [(0, n_rows, D)]
+        row0 = int(row0)
+    idx = torch.empty((n_rows, k), dtype=torch.int32, device=dev)
+    dist = torch.empty((n_rows, k), dtype=torch.float32, device=dev)
+    for r0, r1, P in parts:
+        _knn_rows(P, r0 if isinstance(D, panels.SOURCES) else row0, k, idx[r0:r1], dist[r0:r1])
     if not as_sparse:
         return idx, dist
     from scipy.sparse import csr_matrix
@@ -156,22 +180,18 @@ class KMedoids:
 
     def fit(self, X, y=None):
         self._check_init_args()
-        if self.distance_metric == "precomputed":
-            D = as_device_matrix(X)
-        else:
-            Xd = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(X)))
-            D = engine.distance_matrix_device(Xd.to(engine.require_cuda()), self.distance_metric, torch.float32, symmetric=True)
-        n, k = int(D.shape[0]), self.n_clusters
+        src = _source(X, self.distance_metric)
+        n, k = src.n, self.n_clusters
         if k > n:
             raise ValueError("The number of medoids ({}) must be larger than the number of samples ({})".format(k, n))
-        dev = D.device
+        dev = src.device
         # initial medoids (:291-309)
         if self.init == "random":
             rs = self.random_state if isinstance(self.random_state, np.random.RandomState) else np.random.RandomState(self.random_state)
             medoids = torch.from_numpy(np.asarray(rs.permutation(n)[:k], dtype=np.int64)).to(dev)
         else:
             # np.argsort's order: NaN sums last whatever their sign (torch's device sort puts a negative NaN first)
-            sums = row_sums(D)
+            sums = torch.cat([row_sums(P) for _, _, P in src.panels()])
             nan = torch.isnan(sums)
             medoids = torch.argsort(torch.where(nan, torch.inf, sums), stable=True)
             medoids = medoids[torch.argsort(nan[medoids].to(torch.int8), stable=True)][:k].contiguous()
@@ -182,9 +202,11 @@ class KMedoids:
         while (old is None or not torch.equal(old, medoids)) and self.n_iter_ < self.max_iter:
             self.n_iter_ += 1
             old = medoids.clone()
-            labels = assign_to_medoids(D, medoids)                                   # :187-195
-            cost = row_sums(D, labels=labels, row_labels=labels)                     # every point's cost inside its own cluster
-            curr = row_sums(D, rows=medoids, labels=labels, row_labels=cluster_ids)  # the current medoids' costs (:207-211)
+            M = src.rows(medoids)                                                    # the medoids' rows, k x n
+            labels = assign_to_medoids(M, cluster_ids.to(torch.int64))               # :187-195
+            # every point's cost inside its own cluster
+            cost = torch.cat([row_sums(P, labels=labels, row_labels=labels[r0:r1]) for r0, r1, P in src.panels()])
+            curr = row_sums(M, labels=labels, row_labels=cluster_ids)               # the current medoids' costs (:207-211)
             best_idx, best_cost, count = cluster_argmin(cost, labels, k)             # :213-227
             empty = torch.nonzero(count == 0).flatten().tolist()
             for c in empty:
@@ -193,19 +215,30 @@ class KMedoids:
             medoids = torch.where(better, best_idx, medoids)
         self.medoid_indices_ = medoids.cpu().numpy()
         self.labels_ = labels.cpu().numpy().astype(np.int64) if labels is not None else np.zeros(n, dtype=np.int64)
-        if isinstance(X, torch.Tensor):
+        if isinstance(X, panels.SOURCES):
+            self.cluster_centers_ = X.rows(medoids).cpu().numpy()
+        elif isinstance(X, torch.Tensor):
             self.cluster_centers_ = X[medoids.to(X.device)].cpu().numpy()
         else:
             self.cluster_centers_ = np.asarray(X).take(self.medoid_indices_, axis=0)
         return self
 
 
-def check_matrix(D):
+def check_matrix(D, row0=None, cols=None):
     """Refuse (PhyloligoError) a device matrix that is not square, not bitwise symmetric or holds a NaN or an
-    infinite entry; the message names the first offending entry (po_hdbscan_check)."""
+    infinite entry; the message names the first offending entry (po_hdbscan_check).  With row0, D is the row
+    panel [row0, row0 + rows) of a square matrix of D.shape[1] rows, and `cols` its column strip (the
+    transposed entries), or None for a source symmetric by construction (only the diagonal square is tested
+    for symmetry); checked panel by panel in row order, the first failure names the entry the whole-matrix
+    check names."""
     lib = _lib.load()
     work = torch.empty(1, dtype=torch.int64, device=D.device)
-    rc = lib.po_hdbscan_check(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), _ptr(work), _stream())
+    if row0 is None:
+        r0, cptr, cld = 0, None, 0
+    else:
+        r0, cptr, cld = int(row0), _ptr(cols), (int(cols.stride(0)) if cols is not None else max(1, int(D.shape[0])))
+    rc = lib.po_hdbscan_check(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), r0, cptr, cld, _ptr(work),
+                              _stream())
     _lib.check(rc, "po_hdbscan_check")
 
 
@@ -220,23 +253,26 @@ def kth_smallest(D, k):
 
 
 def mutual_reachability_mst(D, core, on_round=None):
-    """The minimum spanning tree of mr(i, j) = max(core[i], core[j], D[i, j]) by Boruvka rounds on the device
-    (po_hdbscan_mst_round), edges compared by (mr, min(i, j), max(i, j)).  Returns device tensors
-    (u int64, v int64, w in D's dtype), n - 1 edges in no particular order.  `on_round(components)` is
-    called after every round."""
+    """The minimum spanning tree of mr(i, j) = max(core[i], core[j], D[i, j]) by Boruvka rounds on the device,
+    edges compared by (mr, min(i, j), max(i, j)): every round scans the rows (po_hdbscan_mst_scan, one call per
+    panel when D is a row-panel source) and then merges (po_hdbscan_mst_merge).  D must be bitwise symmetric
+    (check_matrix).  Returns device tensors (u int64, v int64, w in D's dtype), n - 1 edges in no particular
+    order.  `on_round(components)` is called after every round."""
     lib = _lib.load()
-    n = int(D.shape[0])
-    dev = D.device
+    src = D if isinstance(D, panels.SOURCES) else panels.ResidentSource(D)
+    n, dev, dt = src.n, src.device, _dt(torch.empty(0, dtype=src.dtype))
     work = torch.empty(int(lib.po_hdbscan_mst_workspace(n)), dtype=torch.uint8, device=dev)
     u = torch.empty(max(n - 1, 1), dtype=torch.int64, device=dev)
     v = torch.empty_like(u)
-    w = torch.empty(max(n - 1, 1), dtype=D.dtype, device=dev)
+    w = torch.empty(max(n - 1, 1), dtype=src.dtype, device=dev)
     _lib.check(lib.po_hdbscan_mst_init(n, _ptr(work), _stream()), "po_hdbscan_mst_init")
     comps = C.c_int64(n)
     while comps.value > 1:
-        rc = lib.po_hdbscan_mst_round(_ptr(D), int(D.stride(0)), _dt(D), n, _ptr(core), _ptr(work), _ptr(u), _ptr(v), _ptr(w),
-                                      C.byref(comps), _stream())
-        _lib.check(rc, "po_hdbscan_mst_round")
+        for r0, r1, P in src.panels():
+            rc = lib.po_hdbscan_mst_scan(_ptr(P), int(P.stride(0)), dt, r0, r1 - r0, n, _ptr(core), _ptr(work), _stream())
+            _lib.check(rc, "po_hdbscan_mst_scan")
+        rc = lib.po_hdbscan_mst_merge(n, dt, _ptr(core), _ptr(work), _ptr(u), _ptr(v), _ptr(w), C.byref(comps), _stream())
+        _lib.check(rc, "po_hdbscan_mst_merge")
         if on_round is not None:
             on_round(comps.value)
     return u[:n - 1], v[:n - 1], w[:n - 1]
@@ -310,18 +346,19 @@ class HDBSCAN:
         self.metric = metric
 
     def fit(self, X, y=None):
-        if self.metric == "precomputed":
-            D = as_device_matrix(X)
-        else:
-            Xd = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(X)))
-            D = engine.distance_matrix_device(Xd.to(engine.require_cuda()), self.metric, torch.float32, symmetric=True)
-        n = int(D.shape[0])
+        src = _source(X, self.metric)
+        n = src.n
         if n < 2:
             raise ValueError("HDBSCAN needs at least 2 samples, got {}".format(n))
-        check_matrix(D)
         ms = min(self.min_cluster_size if self.min_samples is None else self.min_samples, n - 1)
-        core = kth_smallest(D, ms + 1)
-        u, v, w = mutual_reachability_mst(D, core)
+        core = torch.empty(n, dtype=src.dtype, device=src.device)
+        for r0, r1, P in src.panels():  # the check and the core distances: one pass
+            if src.resident:
+                check_matrix(P)
+            else:
+                check_matrix(P, r0, None if src.symmetric else src.column_strip(r0, r1))
+            core[r0:r1] = kth_smallest(P, ms + 1)
+        u, v, w = mutual_reachability_mst(src, core)
         (self.labels_, self.probabilities_, self.condensed_tree_, self.single_linkage_tree_,
          self.minimum_spanning_tree_) = hdbscan_tree(u.cpu().numpy(), v.cpu().numpy(), w.cpu().numpy(), n, self.min_cluster_size)
         return self
@@ -333,12 +370,14 @@ class HDBSCAN:
 TSNE_MAX_K = 1024  # po_matrix_knn's largest k
 
 
-def check_tsne_matrix(D):
+def check_tsne_matrix(D, row0=0):
     """Refuse (PhyloligoError) a device matrix holding a NaN, an infinite or a negative entry, as scikit-learn's
-    TSNE(metric="precomputed") does; the message names the first one in row-major order (po_tsne_check)."""
+    TSNE(metric="precomputed") does; the message names the first one in row-major order (po_tsne_check).  With
+    row0, D holds the rows [row0, row0 + rows) of the matrix and the message names the absolute entry."""
     lib = _lib.load()
     work = torch.empty(1, dtype=torch.int64, device=D.device)
-    rc = lib.po_tsne_check(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), _ptr(work), _stream())
+    rc = lib.po_tsne_check(_ptr(D), int(D.stride(0)), _dt(D), int(D.shape[0]), int(D.shape[1]), int(row0), _ptr(work),
+                           _stream())
     _lib.check(rc, "po_tsne_check")
 
 
@@ -358,23 +397,39 @@ def tsne_affinities(D, perplexity, as_sparse=False):
     `as_sparse` the scipy CSR matrix.  The transpose and the merge of the two halves are torch sort and gather
     plumbing; each merged value is one addition of two terms, and the total is a fixed-order sum, so the result
     is deterministic."""
+    src = D if isinstance(D, panels.SOURCES) else panels.ResidentSource(
+        D if isinstance(D, torch.Tensor) and D.is_cuda else as_device_matrix(D))
+    return _affinities(src, perplexity, as_sparse=as_sparse)
+
+
+def _affinities(src, perplexity, as_sparse=False, check=False):
+    """tsne_affinities over the panels of a source, with `check` the input check of every panel first
+    (check_tsne_matrix; the first panel with an offending entry stops the pass)."""
     lib = _lib.load()
-    D = D if isinstance(D, torch.Tensor) and D.is_cuda else as_device_matrix(D)
-    n = int(D.shape[0])
+    n = src.n
+    dev = src.device
     k = min(n - 1, int(3.0 * perplexity + 1))
-    if k > TSNE_MAX_K:
-        raise ValueError("perplexity {} needs {} neighbours per point; at most {} are supported (perplexity <= 341)"
-                         .format(perplexity, k, TSNE_MAX_K))
-    idx, _ = knn_graph(D, k)
-    cond = torch.empty((n, k), dtype=torch.float64, device=D.device)
-    rc = lib.po_tsne_conditional(_ptr(D), int(D.stride(0)), _dt(D), n, _ptr(idx), k, float(perplexity), _ptr(cond), _stream())
-    _lib.check(rc, "po_tsne_conditional")
-    rows = torch.arange(n, dtype=torch.int64, device=D.device).repeat_interleave(k)
+    for r0, r1, P in src.panels():
+        if check:
+            check_tsne_matrix(P, r0)
+        if r0 == 0:  # after the first panel's check, as the whole-matrix check came first
+            if k > TSNE_MAX_K:
+                raise ValueError("perplexity {} needs {} neighbours per point; at most {} are supported (perplexity <= 341)"
+                                 .format(perplexity, k, TSNE_MAX_K))
+            idx = torch.empty((n, k), dtype=torch.int32, device=dev)
+            dist = torch.empty((n, k), dtype=torch.float32, device=dev)
+            cond = torch.empty((n, k), dtype=torch.float64, device=dev)
+        _knn_rows(P, r0, k, idx[r0:r1], dist[r0:r1])
+        # po_tsne_conditional takes n as the row count: row i of P is matrix row r0 + i
+        rc = lib.po_tsne_conditional(_ptr(P), int(P.stride(0)), _dt(P), r1 - r0, _ptr(idx[r0:r1]), k, float(perplexity),
+                                     _ptr(cond[r0:r1]), _stream())
+        _lib.check(rc, "po_tsne_conditional")
+    rows = torch.arange(n, dtype=torch.int64, device=dev).repeat_interleave(k)
     cols = idx.reshape(-1).to(torch.int64)
     keys, order = torch.sort(torch.cat([rows * n + cols, cols * n + rows]), stable=True)
     vals = torch.cat([cond.reshape(-1), cond.reshape(-1)])[order]
     m = int(keys.numel())
-    first = torch.ones(m, dtype=torch.bool, device=D.device)
+    first = torch.ones(m, dtype=torch.bool, device=dev)
     first[1:] = keys[1:] != keys[:-1]
     starts = torch.nonzero(first).flatten()
     nxt = torch.clamp(starts + 1, max=m - 1)
@@ -383,7 +438,7 @@ def tsne_affinities(D, perplexity, as_sparse=False):
     keep = merged != 0
     ukeys, data = keys[starts][keep], merged[keep]
     indices = (ukeys % n).to(torch.int32)
-    indptr = torch.zeros(n + 1, dtype=torch.int64, device=D.device)
+    indptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
     indptr[1:] = torch.cumsum(torch.bincount(ukeys // n, minlength=n), 0)
     total = max(float(_fixed_sum(data).item()), float(np.finfo(np.float64).eps))
     data = data / total
@@ -531,15 +586,9 @@ class TSNE:
         self.angle = angle
         self.n_jobs = n_jobs
 
-    def _matrix(self, X):
-        if self.metric == "precomputed":
-            return as_device_matrix(X)
-        Xd = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(X)))
-        return engine.distance_matrix_device(Xd.to(engine.require_cuda()), self.metric, torch.float32, symmetric=True)
-
     def fit_transform(self, X, y=None):
-        D = self._matrix(X)
-        n = int(D.shape[0])
+        src = _source(X, self.metric)
+        n = src.n
         if n < 2:
             raise ValueError("TSNE needs at least 2 samples, got {}".format(n))
         if self.perplexity >= n:
@@ -548,14 +597,13 @@ class TSNE:
             self.learning_rate_ = np.maximum(n / self.early_exaggeration / 4, 50)
         else:
             self.learning_rate_ = self.learning_rate
-        check_tsne_matrix(D)
+        P = _affinities(src, self.perplexity, check=True)  # one pass: check, neighbours, conditional P
         if isinstance(self.init, np.ndarray):
             if self.init.shape != (n, 2):
                 raise ValueError("init has shape {}; ({}, 2) is expected".format(self.init.shape, n))
             Y0 = self.init
         else:
             Y0 = 1e-4 * _random_state(self.random_state).standard_normal(size=(n, self.n_components)).astype(np.float32)
-        P = tsne_affinities(D, self.perplexity)
         st = _Descent(P, Y0)
         # scikit-learn's update is float64 when the learning rate is a float64 scalar ("auto": np.maximum), float32
         # for a Python float
@@ -855,6 +903,49 @@ def read_matrix(path, large=False):
     return read_distmat(path)
 
 
+def read_source(path, large=False):
+    """The matrix of `path` for the clustering methods: resident on the device when it fits with their working
+    state (panels.fits), else, for a --large memmap / h5py file, a panels.FileSource that reads it panel by panel
+    (never the whole file into host memory).  A text matrix that does not fit is refused with its byte count."""
+    if large:
+        if large == "memmap":
+            size = os.path.getsize(path) // 4
+            n = int(round(np.sqrt(size)))
+            if n * n != size:
+                print("Error, weird shape for matrix {}".format(path), file=sys.stderr)
+                sys.exit(1)
+            offset, dtype = 0, np.float32
+        else:
+            shape, dtype, offset = io_formats.dataset_location(path, "distances")
+            if len(shape) != 2 or shape[0] != shape[1]:
+                raise PhyloligoError("a square distance matrix is expected, got shape %s" % (tuple(shape),))
+            n = int(shape[0])
+        if panels.fits(n, np.dtype(dtype).itemsize):
+            return panels.ResidentSource(as_device_matrix(read_matrix(path, large)))
+        return panels.FileSource(path, n, offset=offset, dtype=dtype)
+    matrix = read_matrix(path, large)
+    n = int(matrix.shape[0]) if matrix.ndim == 2 else 0
+    budget = panels.device_budget()
+    if not panels.fits(n, 8, budget):
+        raise PhyloligoError("a text matrix of {} rows needs {} bytes of device memory (float64, with the working state), "
+                             "{} are free; write it with phyloligo.py --large memmap or h5py to cluster it in row panels"
+                             .format(n, 8 * n * n + panels.state_bytes(n), budget))
+    return panels.ResidentSource(as_device_matrix(matrix))
+
+
+def check_resident_methods(params, n, element_size):
+    """Refuse (PhyloligoError), before any pass, what needs the matrix resident: -m hclust and --tree-out keep an
+    O(n^2) float64 working state besides it."""
+    wants = (["-m hclust"] if params.method == "hclust" else []) + (["--tree-out"] if params.tree_out else [])
+    if not wants:
+        return
+    budget = panels.device_budget()
+    work = nj_bytes(n, params.tree_method) if params.tree_out and params.tree_method != "hclust" else linkage_bytes(n, params.linkage)
+    need = int(n) * int(n) * int(element_size) + work
+    raise PhyloligoError("{} of {} rows needs {} bytes of device memory (the matrix and the tree's float64 working state), "
+                         "{} are free".format(" and ".join(wants), n, need, budget))
+
+
 def find_clusters(data, method, kwargs, return_model=False):
     """reference :403-428; with `return_model` the fitted estimator (its ``labels_`` are what is returned
     otherwise; HClust's also holds the tree, ``linkage_``)"""
@@ -1001,12 +1092,18 @@ def main(argv=None):
         if res is None:
             print("Error, no FASTA record in {}".format(params.assembly), file=sys.stderr)
             sys.exit(1)
-        matrix = engine.distance_matrix_device(res["freq32"], phyloligo._large_metric(params.dist), torch.float32, symmetric=True)
+        source = panels.profile_source(res["freq32"], phyloligo._large_metric(params.dist))
         if params.fastafile is None:
             params.fastafile = params.assembly
     else:
         print("Read matrix")
-        matrix = read_matrix(params.distmat, params.large)
+        source = read_source(params.distmat, params.large)
+    if source.resident:
+        matrix = source.D
+    else:
+        check_resident_methods(params, source.n, torch.empty(0, dtype=source.dtype).element_size())
+        matrix = source
+        print("The matrix does not fit on the device: {} rows in panels of {}".format(source.n, source.panel_rows))
     print("Clusterize")
     model = clusterize(matrix, params.method, min_cluster_size=params.min_cluster_size, min_samples=params.min_samples,
                        nbk=params.nbk, linkage_method=params.linkage, return_model=True)

@@ -17,7 +17,7 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-KERNEL = "_ZN2po15jsd_tile_kernelIfEEvNS_9JsdParamsE"
+KERNEL = "_ZN2po15jsd_tile_kernelIfLb0EEEvNS_9JsdParamsE"  # jsd_tile_kernel<float, false>: the stores of the resident matrix
 UNROLL = 2
 
 LINE = re.compile(r"/\*([0-9a-f]{4,})\*/\s+(.*?)\s*;")
